@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # reference impl_c on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last timed step's results as DIR/<name>.npy
 
 Metric (BASELINE.json): frames x iterations per second of Baum-Welch EM.  Workload (config.workload): "c3" =
 10-state dalton-style Gaussian HMM, 1024 trajectories x 1e5 frames PER GPU (weak scaling), synthetic data drawn
@@ -12,9 +13,15 @@ all-reduce of the packed statistics across ranks, host M-step.
 
 One JSON line on stdout (rank 0).  `value` is measured with the observations resident in HBM; `e2e` repeats the
 measurement through the public API with the observations in pinned HOST memory, copied to the device inside the
-timed region every step, and the statistics read back.  `roofline` is for the dominant kernel, timed live with CUDA
-events on the launching stream.  `cpu_baseline` times the reference's own C implementation (oracle/_ref, built from
-/root/reference) on the host cores on a bounded sample of the same workload.
+timed region every step, and the statistics read back.  `--steps` sets the timed EM steps of `value` and the timed
+Gibbs sweeps; the end-to-end fit is a workload of its own with `--e2e-iters` iterations (default 20), whatever `--steps`.  `roofline` is for the dominant kernel, timed live with CUDA
+events on the launching stream.  `cpu_baseline` times the reference's own C implementation (oracle/_ref, built by
+build() from a checkout of the reference package; the oracle's C restatement where there is none) on the host cores on
+a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step returned (the EM leg's updated model and
+log-likelihood; for c5 the forward-backward statistics) as float64 .npy files.  The inputs are drawn from fixed
+seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -237,8 +244,8 @@ def cpu_model():
 
 
 def reference_kind():
+    """The CPU libraries are built by build(); the benchmark compiles nothing into the (possibly read-only) tree."""
     from oracle import oracle as orc
-    orc.build(ref=os.path.isdir('/root/reference'))
     return 'reference' if orc.have_reference_lib() else 'port'
 
 
@@ -334,6 +341,21 @@ def hbm_peak():
     if os.path.exists(peaks_path):
         return float(json.load(open(peaks_path))['hbm_gbs']), 'measured (MEASURED_PEAKS.json hbm_gbs)'
     return 6650.0, 'fallback (B200_PROFILING.md)'
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: one float64 DIR/<name>.npy per array the last timed step returned (all of it: every workload's
+    step returns a model or statistics of at most a few MB)."""
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError('--dump-outputs: %d bytes exceed the %d-byte limit' % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 FP64_DFMA_TFLOPS = 34.2     # vector DFMA, measured on this pool's B200 with tools/micro/fp64_peak.cu (DESIGN.md 5.4)
@@ -451,6 +473,8 @@ def run_gaussian_em(args, torch, td, dev, world, rank, local):
     ms = tm.stop()
     launches = _lib.lib.bhmm_b200_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'A': model[0], 'pi': model[1], 'means': model[2], 'sigmas': model[3], 'loglik': [ll]})
     value = world * rows * args.steps / (ms * 1e-3)
     info = batch.info()
     phase0 = {'estep_call_ms': 1e3 * PHASE['estep'] / args.steps, 'allreduce_mstep_readback_ms': 1e3 * PHASE['reduce_mstep_readback'] / args.steps}
@@ -470,7 +494,7 @@ def run_gaussian_em(args, torch, td, dev, world, rank, local):
     from bhmm_b200.hmm import HMM
     from bhmm_b200.output_models import GaussianOutputModel
     A_, pi_, m_, s_ = model
-    gsteps = max(1, min(args.steps, 10))
+    gsteps = args.steps
     np.random.seed(11)
     smp_init = HMM(pi_, A_, GaussianOutputModel(N, means=m_, sigmas=s_))
     # the sampler runs on the resident batch (batch=: no second upload of the observations)
@@ -625,6 +649,8 @@ def run_c4(args, torch, td, dev, world, rank, local):
     ms = tm.stop()
     launches = _lib.lib.bhmm_b200_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'A': model[0], 'pi': model[1], 'B': model[2], 'loglik': [ll]})
     value = world * rows * args.steps / (ms * 1e-3)
     A_, pi_, B_ = model
     batch.viterbi_discrete(A_, pi_, B_)
@@ -715,6 +741,8 @@ def run_c5(args, torch, td, dev, world, rank, local):
     launches = _lib.lib.bhmm_b200_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     st = unpack_stats(stats.cpu().numpy(), N)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(st, loglik=[st['loglik']]))
     info = batch.info()
     # ---- Viterbi path of the WHOLE trajectory across the shards (engine.TimeShardedTrajectories.viterbi): chain-parallel
     # back-pointer maps per shard, certified borders, paths resolved from the last shard to the first.  The forward-variable
@@ -811,10 +839,18 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--scaling', default='weak', choices=['weak', 'strong'],
                     help='weak: the workload\'s trajectories PER GPU; strong: in total (BASELINE config 3: 1024 over 8 GPUs)')
-    ap.add_argument('--e2e-iters', type=int, default=20, help='EM iterations of the end-to-end fit (SURVEY 8d: 20 for C3)')
+    ap.add_argument('--e2e-iters', type=int, default=20,
+                    help='EM iterations of the timed end-to-end fit (SURVEY 8d: 20 for C3); independent of --steps, which '
+                         'sets the timed EM steps and Gibbs sweeps')
     ap.add_argument('--frames', type=float, default=0, help='c5: frames of the trajectory')
     ap.add_argument('--budget-gb', type=float, default=140.0, help='c4: workspace budget per GPU')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned as DIR/<name>.npy (float64)')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs applies to --impl ours (the reference arm only times its steps)')
     if args.impl == 'reference':
         run_reference_arm(args)
     else:

@@ -114,11 +114,12 @@ def test_glibc_stream_restatement_in_the_library():
 def test_reference_install_hook_dispatches_to_cuda():
     """bhmm_b200.install() registers 'cuda' in an importable reference package (scratch build under baseline/_ref,
     tools/build_reference_scratch.py).  Without a device the dispatch must end in CudaUnavailableError -- never in CPU code;
-    with a device tests/test_reference_on_cuda.py runs the reference's estimators on it."""
+    with a device tests/test_reference_on_cuda.py runs the reference's estimators on it.  The reference package is not part
+    of this repository: without that scratch build this test skips and the install hook is not exercised."""
     import sys
     ref = os.path.join(ROOT, 'baseline', '_ref')
     if not os.path.isdir(os.path.join(ref, 'bhmm')) or have_device():
-        pytest.skip('no importable reference build (or a GPU is present)')
+        pytest.skip('no importable reference build under baseline/_ref (or a GPU is present): install hook NOT exercised')
     sys.path.insert(0, os.path.join(ROOT, 'tests', 'golden'))
     import msmtools_stub
     msmtools_stub.install()

@@ -4,7 +4,8 @@
 * against tests/golden/*.npz, which tests/golden/make_golden.py produced by running the
   reference package itself (bhmm.hidden with kernel 'c', MaximumLikelihoodEstimator.fit),
 * bit-for-bit against oracle/_ref/libbhmm_ref.so (the reference's own C sources compiled in place)
-  on fresh seeded inputs, whenever that library is present,
+  on fresh seeded inputs, whenever that library is present, and always against the outputs on those
+  inputs stored in tests/golden/oracle_bitwise.npz (provenance in tests/golden/make_oracle_bitwise.py),
 * and the glibc rand() restatement against the C library of the machine running the test.
 """
 import ctypes
@@ -77,15 +78,61 @@ def test_emission_fixtures(oracle_port, golden):
     assert np.array_equal(oracle_port.discrete_p_obs(g['obs'], g['B']), g['pobs'])
 
 
-def test_port_bitwise_equals_reference_library(oracle_port, oracle_ref):
+BITWISE_SHAPES = [(2, 50), (3, 700), (7, 400), (10, 900), (32, 300), (100, 60)]
+BITWISE_SEEDS = (0, 1, 31337)
+
+
+def bitwise_cases():
+    """The seeded inputs of the bit-for-bit comparison with the reference library, one tuple per (N, T)."""
     rng = np.random.default_rng(2024)
-    for N, T in [(2, 50), (3, 700), (7, 400), (10, 900), (32, 300), (100, 60)]:
+    for N, T in BITWISE_SHAPES:
         X = rng.random((N, N)) + 0.05
         A = X / X.sum(axis=1)[:, None]
         pi = rng.random(N)
         pi /= pi.sum()
         means, sigmas = np.linspace(-3, 3, N), np.linspace(0.4, 1.5, N)
         obs = rng.normal(size=T) * 2.0
+        w = rng.random((T, N))
+        sym = rng.integers(0, 13, size=T).astype(np.int32)
+        yield A, pi, means, sigmas, obs, w, sym
+
+
+def bitwise_outputs(oracle, case, k):
+    """Everything the comparison checks, computed by one library, keyed as in tests/golden/oracle_bitwise.npz."""
+    A, pi, means, sigmas, obs, w, sym = case
+    N = A.shape[0]
+    pobs = oracle.gaussian_p_obs(obs, means, sigmas)
+    logprob, alpha = oracle.forward(A, pobs, pi)
+    beta = oracle.backward(A, pobs)
+    out = {'obs': obs, 'pobs': pobs, 'logprob': np.float64(logprob), 'alpha': alpha, 'beta': beta,
+           'C': oracle.transition_counts(alpha, beta, A, pobs), 'viterbi': oracle.viterbi(A, pobs, pi),
+           'pout': oracle.update_pout(sym, w, np.zeros((N, 13)))}
+    for seed in BITWISE_SEEDS:
+        out['sample_path_seed%d' % seed] = oracle.sample_path(alpha, A, seed=seed)
+    return {'%s_%d' % (name, k): v for name, v in out.items()}
+
+
+def _assert_equals_stored(oracle, golden):
+    g = golden('oracle_bitwise')
+    for k, case in enumerate(bitwise_cases()):
+        for name, v in bitwise_outputs(oracle, case, k).items():
+            assert np.asarray(v).dtype == g[name].dtype and np.array_equal(v, g[name]), name
+
+
+def test_port_bitwise_equals_stored_reference_outputs(oracle_port, golden):
+    """test_port_bitwise_equals_reference_library without the library: the same inputs, every output compared bit for bit
+    with tests/golden/oracle_bitwise.npz (provenance in tests/golden/make_oracle_bitwise.py)."""
+    _assert_equals_stored(oracle_port, golden)
+
+
+def test_reference_library_reproduces_stored_outputs(oracle_ref, golden):
+    """Wherever the reference library is built, the stored outputs are checked against it."""
+    _assert_equals_stored(oracle_ref, golden)
+
+
+def test_port_bitwise_equals_reference_library(oracle_port, oracle_ref):
+    for A, pi, means, sigmas, obs, w, sym in bitwise_cases():
+        N = A.shape[0]
         pa = oracle_port.gaussian_p_obs(obs, means, sigmas)
         pb = oracle_ref.gaussian_p_obs(obs, means, sigmas)
         assert np.array_equal(pa, pb)
@@ -96,11 +143,9 @@ def test_port_bitwise_equals_reference_library(oracle_port, oracle_ref):
         assert np.array_equal(ba, bb)
         assert np.array_equal(oracle_port.transition_counts(aa, ba, A, pa), oracle_ref.transition_counts(aa, ba, A, pa))
         assert np.array_equal(oracle_port.viterbi(A, pa, pi), oracle_ref.viterbi(A, pa, pi))
-        for seed in (0, 1, 31337):
+        for seed in BITWISE_SEEDS:
             # reference: set_seed(seed) + libc rand(); port: restated generator + explicit uniforms
             assert np.array_equal(oracle_port.sample_path(aa, A, seed=seed), oracle_ref.sample_path(aa, A, seed=seed))
-        w = rng.random((T, N))
-        sym = rng.integers(0, 13, size=T).astype(np.int32)
         assert np.array_equal(oracle_port.update_pout(sym, w, np.zeros((N, 13))),
                               oracle_ref.update_pout(sym, w, np.zeros((N, 13))))
 

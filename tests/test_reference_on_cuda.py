@@ -4,6 +4,10 @@ exists; it travels to the GPU box) is imported, `bhmm_b200.install(bhmm)` regist
 the reference's own estimators -- maximum_likelihood.py:354-446, bayesian_sampling.py:206-373, not a line of them changed
 -- are compared with fixtures that the same classes produced with `config.kernel = 'c'` (tests/golden/make_golden.py).
 
+The reference package is not part of this repository.  Without the scratch build under baseline/_ref both tests skip, and
+then nothing here has checked that the reference's estimators run unchanged on 'cuda'.  Their expected values do not need
+it: test_engine_cuda.py compares this package's own engine with the same fixtures in every run.
+
 `msmtools` (absent, un-pinned) is replaced by tests/golden/msmtools_stub.py exactly as it was when the fixtures were made.
 Run in a child process: importing the reference package and the stub must not leak into the other tests.
 """
@@ -109,7 +113,8 @@ print('all ok')
 
 def _run(cache):
     if not os.path.isdir(os.path.join(REF, 'bhmm')):
-        pytest.skip('no scratch build of the reference under baseline/_ref (tools/build_reference_scratch.py)')
+        pytest.skip('no scratch build of the reference under baseline/_ref (tools/build_reference_scratch.py): the '
+                    'reference estimators were NOT run on cuda')
     r = subprocess.run(['timeout', '600', sys.executable, '-c', CHILD, ROOT, REF, '1' if cache else '0'],
                        stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     print(r.stdout)
