@@ -112,6 +112,12 @@ _proto('bhmm_b200_transfer_config', C.c_int, C.c_int, C.c_int)
 _proto('bhmm_b200_prefault', C.c_int, _vp, C.c_longlong, C.c_int)
 _proto('bhmm_b200_download_ragged', C.c_int, C.POINTER(C.c_void_p), _vp, _llp, C.c_int, C.c_int, _vp)
 _proto('bhmm_b200_path_symbol_histogram', C.c_int, _vp, _vp, C.c_longlong, C.c_int, C.c_int, _vp, _vp)
+# synthetic trajectories
+_proto('bhmm_b200_generate_workspace_bytes', C.c_size_t, _llp, C.c_int, C.c_int, C.c_int)
+_proto('bhmm_b200_generate_states', C.c_int, _vp, _llp, C.c_int, C.c_int, _dp, _dp, _ip, C.c_ulonglong, C.c_int, _vp,
+       C.c_size_t, _vp)
+_proto('bhmm_b200_emit_gaussian', C.c_int, _vp, _vp, C.c_longlong, C.c_int, _dp, _dp, C.c_ulonglong, _vp)
+_proto('bhmm_b200_emit_discrete', C.c_int, _vp, _vp, C.c_longlong, C.c_int, C.c_int, _dp, C.c_ulonglong, _vp)
 
 if os.environ.get('BHMM_B200_REPAIR_TOL'):      # A/B measurements: 0 = repair every hand-over above the certification tolerance
     lib.bhmm_b200_set_repair_tolerance(float(os.environ['BHMM_B200_REPAIR_TOL']))

@@ -986,3 +986,215 @@ extern "C" int bhmm_b200_mstep_discrete_dev(const double* d_Bnum, int N, int M, 
     CUDA_TRY(cudaGetLastError());
     return BHMM_OK;
 }
+
+// ------------------------------------------------------------------------------------------------
+// Synthetic trajectories (generate_synthetic_*, bhmm/hmm/generic_hmm.py:433-589): hidden states by exact time-parallel
+// forward simulation (sample_kernels.cu:k_gen_*), observations frame-parallel from the states.
+// ------------------------------------------------------------------------------------------------
+static int gen_fail(int code, const char* msg)
+{
+    bhmm_set_error(code, msg);
+    return code;
+}
+
+// Cumulative table of one distribution: sequential float64 sums (what np.cumsum computes), every entry from the last
+// positive probability on set to exactly 1.0.  False when p is not a probability vector.
+static bool cumulative_row(const double* p, int n, double* cum)
+{
+    double c = 0.0;
+    int last = -1;
+    for (int i = 0; i < n; ++i) {
+        if (!(p[i] >= 0.0) || !std::isfinite(p[i])) return false;
+        c += p[i];
+        cum[i] = c;
+        if (p[i] > 0.0) last = i;
+    }
+    if (last < 0 || std::fabs(c - 1.0) > 1e-6) return false;
+    for (int i = last; i < n; ++i) cum[i] = 1.0;
+    return true;
+}
+
+static int gen_check(const long long* offsets, int K, int N, int segment)
+{
+    if (!offsets || K < 1 || N < 1 || segment < 0) return gen_fail(BHMM_ERR_INVALID, "generate: bad offsets, K, N or segment");
+    if (N > 256) return gen_fail(BHMM_ERR_UNSUPPORTED, "generate: at most 256 hidden states (uint8 segment maps)");
+    if (offsets[0] != 0) return gen_fail(BHMM_ERR_INVALID, "generate: offsets[0] must be 0");
+    for (int k = 0; k < K; ++k) {
+        const long long T = offsets[k + 1] - offsets[k];
+        if (T < 1) return gen_fail(BHMM_ERR_INVALID, "generate: every trajectory needs at least one frame");
+        if (T > 2147483647LL) return gen_fail(BHMM_ERR_INVALID, "generate: trajectories must be shorter than 2^31 frames");
+    }
+    return BHMM_OK;
+}
+
+// Segment length of a call.  Trajectories that fill the GPU on their own (at least two warps per SM for every warp of
+// map work a segment would need) run as one segment each: replay alone, the serial generator.  Otherwise segments are cut
+// so that there are about as many as the SMs hold 1024 threads, i.e. a few waves of map warps and replay threads.
+static int gen_segment_len(const long long* offsets, int K, int N, int segment, bool* whole, long long* nseg)
+{
+    long long maxT = 0;
+    for (int k = 0; k < K; ++k) maxT = std::max(maxT, offsets[k + 1] - offsets[k]);
+    long long L = segment;
+    if (L <= 0) {
+        int sms = 148, dev = 0;
+        if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+            { cudaGetLastError(); sms = 148; }
+        const int W = (N + 31) / 32;
+        if ((long long)K * W >= 64LL * sms) L = maxT;
+        else L = std::max<long long>(32, (offsets[K] + 1024LL * sms - 1) / (1024LL * sms));
+    }
+    L = std::min(L, maxT);
+    *whole = (L >= maxT);
+    long long n = 0;
+    for (int k = 0; k < K; ++k) n += (offsets[k + 1] - offsets[k] + L - 1) / L;
+    *nseg = n;
+    return (int)L;
+}
+
+struct GenLayout {
+    size_t row0, len, t0, T, start, map, enter, cum, bytes;
+};
+
+static GenLayout gen_layout(long long nseg, int N, bool whole)
+{
+    GenLayout g;
+    Carver cv;
+    g.row0 = cv.add<long long>(nseg);
+    g.len = cv.add<int>(nseg);
+    g.t0 = cv.add<int>(nseg);
+    g.T = cv.add<int>(nseg);
+    g.start = cv.add<int>(nseg);
+    g.map = cv.add<unsigned char>(whole ? 0 : (size_t)nseg * N);
+    g.enter = cv.add<int>(whole ? 0 : nseg);
+    g.cum = cv.add<double>((size_t)N + (size_t)N * N);
+    g.bytes = cv.off + 256;                  // the base is aligned up to 256 bytes
+    return g;
+}
+
+extern "C" size_t bhmm_b200_generate_workspace_bytes(const long long* offsets, int K, int N, int segment)
+{
+    if (gen_check(offsets, K, N, segment) != BHMM_OK) return 0;
+    bool whole;
+    long long nseg;
+    gen_segment_len(offsets, K, N, segment, &whole, &nseg);
+    if (nseg > 2147483647LL) return 0;
+    return gen_layout(nseg, N, whole).bytes;
+}
+
+extern "C" int bhmm_b200_generate_states(int* d_states, const long long* offsets, int K, int N, const double* A,
+                                         const double* p0, const int* start, unsigned long long seed, int segment,
+                                         void* d_workspace, size_t bytes, void* stream)
+{
+    clear_error();
+    RC_TRY(gen_check(offsets, K, N, segment));
+    if (!d_states || !A || (!p0 && !start)) return gen_fail(BHMM_ERR_INVALID, "generate: null states, A or initial distribution");
+    std::vector<double> cum((size_t)N + (size_t)N * N, 1.0);
+    if (!start && !cumulative_row(p0, N, cum.data()))
+        return gen_fail(BHMM_ERR_INVALID, "generate: the initial distribution is not a probability vector");
+    for (int i = 0; i < N; ++i)
+        if (!cumulative_row(A + (size_t)i * N, N, cum.data() + N + (size_t)i * N))
+            return gen_fail(BHMM_ERR_INVALID, "generate: the transition matrix is not row-stochastic");
+    if (start)
+        for (int k = 0; k < K; ++k)
+            if (start[k] < 0 || start[k] >= N) return gen_fail(BHMM_ERR_INVALID, "generate: start state out of range");
+    bool whole;
+    long long nseg;
+    const int L = gen_segment_len(offsets, K, N, segment, &whole, &nseg);
+    if (nseg > 2147483647LL) return gen_fail(BHMM_ERR_INVALID, "generate: too many segments (use a longer segment)");
+    const GenLayout g = gen_layout(nseg, N, whole);
+    if (!d_workspace || bytes < g.bytes) return gen_fail(BHMM_ERR_INVALID, "generate: workspace smaller than bhmm_b200_generate_workspace_bytes");
+    RC_TRY(require_device());
+    // segments of every trajectory in reversed time order, t0 counted from the trajectory's end (sample_kernels.cu:k_gen_map)
+    HostPlan p;
+    build_plan(offsets, K, L, p);
+    std::vector<long long> row0(p.n);
+    std::vector<int> len(p.n), t0r(p.n), T(p.n), sst(p.n, -1);
+    int c = 0;
+    for (int k = 0; k < K; ++k)
+        for (int q = p.last_chain[k]; q >= p.first_chain[k]; --q, ++c) {
+            row0[c] = p.row0[q];
+            len[c] = p.len[q];
+            T[c] = p.T[q];
+            t0r[c] = p.T[q] - p.t0[q] - p.len[q];
+            if (start && p.t0[q] == 0) sst[c] = start[k];
+        }
+    char* base = (char*)(((uintptr_t)d_workspace + 255) & ~(uintptr_t)255);
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemcpyAsync(base + g.row0, row0.data(), sizeof(long long) * p.n, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(base + g.len, len.data(), sizeof(int) * p.n, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(base + g.t0, t0r.data(), sizeof(int) * p.n, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(base + g.T, T.data(), sizeof(int) * p.n, cudaMemcpyHostToDevice, st));
+    if (start) CUDA_TRY(cudaMemcpyAsync(base + g.start, sst.data(), sizeof(int) * p.n, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(base + g.cum, cum.data(), sizeof(double) * cum.size(), cudaMemcpyHostToDevice, st));
+    Chains seg{};
+    seg.row0 = (const long long*)(base + g.row0);
+    seg.len = (const int*)(base + g.len);
+    seg.t0 = (const int*)(base + g.t0);
+    seg.T = (const int*)(base + g.T);
+    seg.n = p.n;
+    const double* d_cum = (const double*)(base + g.cum);
+    RC_TRY(launch_generate_states(seg, N, d_cum, d_cum + N, start ? (const int*)(base + g.start) : nullptr, seed, whole,
+                                  (unsigned char*)(base + g.map), (int*)(base + g.enter), d_states, st));
+    LAUNCHED(whole ? 1 : 3);
+    return finish(st);
+}
+
+// small host parameters of an emission call go to the literal API's arena; a state outside [0, N) is reported, not read
+static int emit_run(const std::vector<double>& params, cudaStream_t st,
+                    const std::function<int(const double* d_params, int* d_err)>& launch)
+{
+    std::lock_guard<std::mutex> lk(g_lit_mutex);
+    Carver cv;
+    const size_t o_p = cv.add<double>(params.size());
+    const size_t o_err = cv.add<int>(1);
+    RC_TRY(g_lit_arena.ensure(cv.off + 256));
+    char* base = g_lit_arena.base;
+    CUDA_TRY(cudaMemcpyAsync(base + o_p, params.data(), sizeof(double) * params.size(), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(base + o_err, 0, sizeof(int), st));
+    RC_TRY(launch((const double*)(base + o_p), (int*)(base + o_err)));
+    LAUNCHED(1);
+    int err = 0;
+    CUDA_TRY(cudaMemcpyAsync(&err, base + o_err, sizeof(int), cudaMemcpyDeviceToHost, st));
+    RC_TRY(finish(st));
+    if (err) return gen_fail(BHMM_ERR_INVALID, "emit: a state is out of range [0, N)");
+    return BHMM_OK;
+}
+
+extern "C" int bhmm_b200_emit_gaussian(double* d_obs, const int* d_states, long long rows, int N, const double* means,
+                                       const double* sigmas, unsigned long long seed, void* stream)
+{
+    clear_error();
+    if (rows < 0 || N < 1 || !means || !sigmas || (rows > 0 && (!d_obs || !d_states)))
+        return gen_fail(BHMM_ERR_INVALID, "emit_gaussian: bad arguments");
+    std::vector<double> params(2 * (size_t)N);
+    for (int i = 0; i < N; ++i) {
+        if (!std::isfinite(means[i]) || !std::isfinite(sigmas[i]) || !(sigmas[i] >= 0.0))
+            return gen_fail(BHMM_ERR_INVALID, "emit_gaussian: means must be finite, sigmas finite and >= 0");
+        params[i] = means[i];
+        params[N + i] = sigmas[i];
+    }
+    RC_TRY(require_device());
+    if (rows == 0) return BHMM_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    return emit_run(params, st, [&](const double* d_p, int* d_err) {
+        return launch_emit_gaussian(d_states, rows, N, d_p, d_p + N, seed, d_obs, d_err, st);
+    });
+}
+
+extern "C" int bhmm_b200_emit_discrete(int* d_obs, const int* d_states, long long rows, int N, int M, const double* B,
+                                       unsigned long long seed, void* stream)
+{
+    clear_error();
+    if (rows < 0 || N < 1 || M < 1 || !B || (rows > 0 && (!d_obs || !d_states)))
+        return gen_fail(BHMM_ERR_INVALID, "emit_discrete: bad arguments");
+    std::vector<double> cumB((size_t)N * M);
+    for (int i = 0; i < N; ++i)
+        if (!cumulative_row(B + (size_t)i * M, M, cumB.data() + (size_t)i * M))
+            return gen_fail(BHMM_ERR_INVALID, "emit_discrete: the output matrix is not row-stochastic");
+    RC_TRY(require_device());
+    if (rows == 0) return BHMM_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    return emit_run(cumB, st, [&](const double* d_cumB, int* d_err) {
+        return launch_emit_discrete(d_states, rows, N, M, d_cumB, seed, d_obs, d_err, st);
+    });
+}

@@ -193,3 +193,14 @@ int launch_path_stats(const int* path, const double* obs, const long long* offse
                       long long* Cint, long long* n0, long long* cnt, double* so, double* soo, cudaStream_t st);
 int launch_symbol_histogram(const int* path, const int* sym, long long rows, int N, int M, long long* hist,
                             cudaStream_t st);
+// ---- synthetic trajectories (sample_kernels.cu).  `seg` is the segment table in REVERSED time order (t0 counted from the
+// trajectory's end, see k_gen_map); cum0 (N) and cumA (N,N) are the cumulative tables; seg_start[c] >= 0 fixes the first
+// state of segment c (NULL: drawn from cum0).  whole: every segment is a whole trajectory, the map and link steps are skipped.
+int launch_generate_states(const Chains& seg, int N, const double* cum0, const double* cumA, const int* seg_start,
+                           unsigned long long seed, bool whole, unsigned char* seg_map, int* seg_enter, int* states,
+                           cudaStream_t st);
+// one observation per frame from its state; a state outside [0, N) sets *err = BHMM_ERR_INVALID
+int launch_emit_gaussian(const int* states, long long rows, int N, const double* mu, const double* sigma,
+                         unsigned long long seed, double* obs, int* err, cudaStream_t st);
+int launch_emit_discrete(const int* states, long long rows, int N, int M, const double* cumB, unsigned long long seed,
+                         int* obs, int* err, cudaStream_t st);

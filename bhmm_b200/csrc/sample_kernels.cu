@@ -12,7 +12,8 @@
 //        k_chase_link  per trajectory, walks its segments from the last to the first,
 //        k_chase_path  per segment, follows the maps from the now-known entering state and writes the path.
 // Device Philox4x32-10 supplies the uniforms in production; an explicit uniform array reproduces the
-// reference's glibc stream for parity.
+// reference's glibc stream for parity.  The same Philox stream and link step also drive the forward simulation of
+// synthetic trajectories (k_gen_*, k_emit_*: the generate_synthetic_* API).
 #include <cstdlib>
 
 #include "common.cuh"
@@ -29,11 +30,12 @@ __device__ __forceinline__ void philox_round(uint32_t& c0, uint32_t& c1, uint32_
     c0 = n0; c1 = n1; c2 = n2; c3 = n3;
 }
 
-// uniform in [0,1) from Philox4x32-10 keyed by `seed`, counter (ctr, row)
-__device__ __forceinline__ double philox_uniform(unsigned long long seed, unsigned long long ctr, long long row)
+// Philox4x32-10 block keyed by `seed`, counter (row, ctr): c = {row lo, row hi, ctr lo, ctr hi} on entry
+__device__ __forceinline__ void philox_block(unsigned long long seed, unsigned long long ctr, long long row, uint32_t& c0,
+                                             uint32_t& c1, uint32_t& c2, uint32_t& c3)
 {
-    uint32_t c0 = (uint32_t)row, c1 = (uint32_t)((unsigned long long)row >> 32);
-    uint32_t c2 = (uint32_t)ctr, c3 = (uint32_t)(ctr >> 32);
+    c0 = (uint32_t)row; c1 = (uint32_t)((unsigned long long)row >> 32);
+    c2 = (uint32_t)ctr; c3 = (uint32_t)(ctr >> 32);
     uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
 #pragma unroll
     for (int r = 0; r < 10; ++r) {
@@ -41,6 +43,13 @@ __device__ __forceinline__ double philox_uniform(unsigned long long seed, unsign
         k0 += 0x9E3779B9u;
         k1 += 0xBB67AE85u;
     }
+}
+
+// uniform in [0,1) from Philox4x32-10 keyed by `seed`, counter (ctr, row)
+__device__ __forceinline__ double philox_uniform(unsigned long long seed, unsigned long long ctr, long long row)
+{
+    uint32_t c0, c1, c2, c3;
+    philox_block(seed, ctr, row, c0, c1, c2, c3);
     const unsigned long long bits = ((unsigned long long)c0 << 32) | c1;
     return (double)(bits >> 11) * (1.0 / 9007199254740992.0);
 }
@@ -228,6 +237,130 @@ __global__ void k_symbol_histogram(const int* __restrict__ path, const int* __re
     atomicAdd(hist + (long long)path[r] * M + sym[r], 1ULL);
 }
 
+// ---- synthetic trajectories: forward simulation of the hidden chain, parallel in time and exact
+// Given the frame's uniform u_t = U(seed, 0, row), the state is a fixed function of the previous one,
+//   s_t = G_t(s_{t-1}) = draw(cumA[s_{t-1}], u_t),   s_0 = draw(cum0, u_0) or the caller's start,
+// so the chase above applies with time running forwards:
+//   k_gen_map     per (segment, entering state) -> state at the segment's last frame, G_t evaluated on the fly;
+//   link_segments per trajectory, on a segment table in REVERSED time order (t0 counted from the trajectory's end), so
+//                 that its walk from the "last" segment down to the one with t0 == 0 goes from the first in time to the last;
+//   k_gen_replay  per segment, from the now-known entering state, writes the states.
+// Only comparisons of Philox uniforms with host-built cumulative tables are involved: every segmentation, and a single
+// serial thread, give the same states bit for bit.
+
+// smallest i with u < cum[i] (cum non-decreasing, cum[n-1] = 1 > u): never a zero-probability entry, even at u = 0
+__device__ __forceinline__ int draw_cum(const double* cum, int n, double u)
+{
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (u < cum[mid]) hi = mid; else lo = mid + 1;
+    }
+    return lo;
+}
+
+// state at frame t of a trajectory from the previous state and the frame's uniform (start < 0: draw from cum0)
+__device__ __forceinline__ int gen_step(const double* cum0, const double* cumA, int N, int t, int start, int prev, double u)
+{
+    if (t > 0) return draw_cum(cumA + prev * N, N, u);
+    return start >= 0 ? start : draw_cum(cum0, N, u);
+}
+
+// first frame, within its trajectory, of segment sidx of the reversed table
+__device__ __forceinline__ int gen_t0(const Chains& seg, int sidx) { return seg.T[sidx] - seg.t0[sidx] - seg.len[sidx]; }
+
+// One warp per segment for N <= 32 (4 segments per block), a block of ceil(N/32) warps per segment above.  Lane j carries
+// entering state j through the segment; lane l computes the uniform of the l-th frame of every 32 and the warp shares it.
+template <bool SMEM>
+__global__ void k_gen_map(Chains seg, int N, const double* __restrict__ cum0g, const double* __restrict__ cumAg,
+                          const int* __restrict__ seg_start, unsigned long long seed, unsigned char* __restrict__ map)
+{
+    extern __shared__ double gen_sh[];
+    const double* cum0 = cum0g;
+    const double* cumA = cumAg;
+    if (SMEM) {
+        for (int k = threadIdx.x; k < N + N * N; k += blockDim.x) gen_sh[k] = k < N ? cum0g[k] : cumAg[k - N];
+        __syncthreads();
+        cum0 = gen_sh;
+        cumA = gen_sh + N;
+    }
+    const int W = (N + 31) >> 5;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int sidx = blockIdx.x * ((blockDim.x >> 5) / W) + warp / W;
+    if (sidx >= seg.n) return;                                // whole warps leave together
+    const int j = (warp % W) * 32 + lane;
+    const long long r0 = seg.row0[sidx];
+    const int len = seg.len[sidx], t0 = gen_t0(seg, sidx);
+    const int start = seg_start ? seg_start[sidx] : -1;
+    int s = j < N ? j : 0;                                    // the first segment of a trajectory ignores it (t == 0)
+    for (int b = 0; b < len; b += 32) {
+        const int nb = min(32, len - b);
+        const double u = lane < nb ? philox_uniform(seed, 0ULL, r0 + b + lane) : 0.0;
+        for (int i = 0; i < nb; ++i) s = gen_step(cum0, cumA, N, t0 + b + i, start, s, __shfl_sync(0xffffffffu, u, i));
+    }
+    if (j < N) map[(long long)sidx * N + j] = (unsigned char)s;
+}
+
+// one thread per segment; enter == NULL: every segment starts its trajectory (one segment per trajectory)
+template <bool SMEM>
+__global__ void k_gen_replay(Chains seg, int N, const double* __restrict__ cum0g, const double* __restrict__ cumAg,
+                             const int* __restrict__ seg_start, unsigned long long seed, const int* __restrict__ enter,
+                             int* __restrict__ states)
+{
+    extern __shared__ double gen_sh[];
+    const double* cum0 = cum0g;
+    const double* cumA = cumAg;
+    if (SMEM) {
+        for (int k = threadIdx.x; k < N + N * N; k += blockDim.x) gen_sh[k] = k < N ? cum0g[k] : cumAg[k - N];
+        __syncthreads();
+        cum0 = gen_sh;
+        cumA = gen_sh + N;
+    }
+    const int sidx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (sidx >= seg.n) return;
+    int s = enter ? enter[sidx] : 0;
+    const long long r0 = seg.row0[sidx];
+    const int len = seg.len[sidx], t0 = gen_t0(seg, sidx);
+    const int start = seg_start ? seg_start[sidx] : -1;
+    for (int i = 0; i < len; ++i) {
+        s = gen_step(cum0, cumA, N, t0 + i, start, s, philox_uniform(seed, 0ULL, r0 + i));
+        states[r0 + i] = s;
+    }
+}
+
+#ifdef PANEL_HOST_EMU
+// the CPU emulation (tests/emu) has no cospi; its Gaussian draws are compared with a tolerance
+inline double cospi(double x) { return cos(3.14159265358979323846 * x); }
+#endif
+
+// Box-Muller on one Philox block (seed, 1, row): u1 in (0,1], u2 in [0,1); o = mu + sigma z without contraction
+__global__ void k_emit_gaussian(const int* __restrict__ states, long long rows, int N, const double* __restrict__ mu,
+                                const double* __restrict__ sigma, unsigned long long seed, double* __restrict__ obs,
+                                int* __restrict__ err)
+{
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= rows) return;
+    const int s = states[r];
+    if (s < 0 || s >= N) { obs[r] = NAN; atomicExch(err, BHMM_ERR_INVALID); return; }
+    uint32_t c0, c1, c2, c3;
+    philox_block(seed, 1ULL, r, c0, c1, c2, c3);
+    const double u1 = (double)(((((unsigned long long)c0 << 32) | c1) >> 11) + 1) * (1.0 / 9007199254740992.0);
+    const double u2 = (double)((((unsigned long long)c2 << 32) | c3) >> 11) * (1.0 / 9007199254740992.0);
+    const double z = __dmul_rn(sqrt(-2.0 * log(u1)), cospi(2.0 * u2));
+    obs[r] = __dadd_rn(mu[s], __dmul_rn(sigma[s], z));
+}
+
+__global__ void k_emit_discrete(const int* __restrict__ states, long long rows, int N, int M,
+                                const double* __restrict__ cumB, unsigned long long seed, int* __restrict__ obs,
+                                int* __restrict__ err)
+{
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= rows) return;
+    const int s = states[r];
+    if (s < 0 || s >= N) { obs[r] = -1; atomicExch(err, BHMM_ERR_INVALID); return; }
+    obs[r] = draw_cum(cumB + (long long)s * M, M, philox_uniform(seed, 1ULL, r));
+}
+
 inline unsigned nblk(long long n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 
 }  // namespace
@@ -307,5 +440,51 @@ int launch_symbol_histogram(const int* path, const int* sym, long long rows, int
     (void)N;
     if (rows <= 0) return BHMM_OK;
     k_symbol_histogram<<<nblk(rows, 256), 256, 0, st>>>(path, sym, rows, M, reinterpret_cast<unsigned long long*>(hist));
+    return BHMM_OK;
+}
+
+// cum0 + cumA in shared memory up to 100 KB (N <= 112), read through L1 above
+static size_t gen_smem_bytes(int N)
+{
+    const size_t b = sizeof(double) * ((size_t)N * N + N);
+    return b <= 100 * 1024 ? b : 0;
+}
+
+int launch_generate_states(const Chains& seg, int N, const double* cum0, const double* cumA, const int* seg_start,
+                           unsigned long long seed, bool whole, unsigned char* seg_map, int* seg_enter, int* states,
+                           cudaStream_t st)
+{
+    if (N > 256) return BHMM_ERR_UNSUPPORTED;
+    if (seg.n <= 0) return BHMM_OK;
+    const size_t smem = gen_smem_bytes(N);
+    if (smem > 48 * 1024) {
+        cudaFuncSetAttribute(k_gen_map<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(k_gen_replay<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    }
+    if (!whole) {
+        const int W = (N + 31) / 32, spb = (W == 1) ? 4 : 1;    // segments per block
+        if (smem) k_gen_map<true><<<nblk(seg.n, spb), 32 * W * spb, smem, st>>>(seg, N, cum0, cumA, seg_start, seed, seg_map);
+        else k_gen_map<false><<<nblk(seg.n, spb), 32 * W * spb, 0, st>>>(seg, N, cum0, cumA, seg_start, seed, seg_map);
+        link_segments(seg, N, seg_map, seg_enter, st);
+    }
+    const int* enter = whole ? nullptr : seg_enter;
+    if (smem) k_gen_replay<true><<<nblk(seg.n, 128), 128, smem, st>>>(seg, N, cum0, cumA, seg_start, seed, enter, states);
+    else k_gen_replay<false><<<nblk(seg.n, 128), 128, 0, st>>>(seg, N, cum0, cumA, seg_start, seed, enter, states);
+    return BHMM_OK;
+}
+
+int launch_emit_gaussian(const int* states, long long rows, int N, const double* mu, const double* sigma,
+                         unsigned long long seed, double* obs, int* err, cudaStream_t st)
+{
+    if (rows <= 0) return BHMM_OK;
+    k_emit_gaussian<<<nblk(rows, 256), 256, 0, st>>>(states, rows, N, mu, sigma, seed, obs, err);
+    return BHMM_OK;
+}
+
+int launch_emit_discrete(const int* states, long long rows, int N, int M, const double* cumB, unsigned long long seed,
+                         int* obs, int* err, cudaStream_t st)
+{
+    if (rows <= 0) return BHMM_OK;
+    k_emit_discrete<<<nblk(rows, 256), 256, 0, st>>>(states, rows, N, M, cumB, seed, obs, err);
     return BHMM_OK;
 }

@@ -722,6 +722,99 @@ def make_batch(observations, nstates, device=None, chunk=0, warm=0, max_workspac
     return SubBatchedTrajectories(observations, nstates, int(max_workspace_bytes), device=device, chunk=chunk, warm=warm)
 
 
+# ------------------------------------------------------------------------------------------------ synthetic trajectories
+def resolve_seed(seed):
+    """The 64-bit Philox key of a generator call; ``None`` takes a 63-bit key from ``np.random``, so that
+    ``np.random.seed(x)`` makes a run reproducible, as it does for the reference."""
+    if seed is None:
+        return int(np.random.randint(0, 2 ** 63 - 1, dtype=np.int64))
+    return int(seed) & 0xFFFFFFFFFFFFFFFF
+
+
+def _stochastic(P, what):
+    P = f64(P)
+    if P.ndim != 2 or not np.all(np.isfinite(P)) or np.any(P < 0) or not np.allclose(P.sum(axis=1), 1.0, rtol=0, atol=1e-6):
+        raise ValueError('%s is not row-stochastic' % what)
+    return P
+
+
+def emit_observations(states, seed, means=None, sigmas=None, B=None):
+    """One observation per frame of the device int32 tensor ``states`` (bhmm_b200_emit_gaussian / _discrete): float64
+    draws from N(means[s], sigmas[s]) or int32 symbols from the rows of B.  Frame r uses the Philox stream at row r, so the
+    result is a function of (states, seed) alone.  Returns a device tensor."""
+    torch = _torch()
+    rows = int(states.numel())
+    with torch.cuda.device(states.device):
+        stream = C.c_void_p(torch.cuda.current_stream(states.device).cuda_stream)
+        if B is not None:
+            B = _stochastic(B, 'the output probability matrix')
+            obs = torch.empty(rows, dtype=torch.int32, device=states.device)
+            check(lib.bhmm_b200_emit_discrete(C.c_void_p(obs.data_ptr()), C.c_void_p(states.data_ptr()), rows, B.shape[0],
+                                              B.shape[1], dptr(B), int(seed), stream))
+        else:
+            means, sigmas = f64(means), f64(sigmas)
+            obs = torch.empty(rows, dtype=torch.float64, device=states.device)
+            check(lib.bhmm_b200_emit_gaussian(C.c_void_p(obs.data_ptr()), C.c_void_p(states.data_ptr()), rows, len(means),
+                                              dptr(means), dptr(sigmas), int(seed), stream))
+    return obs
+
+
+def generate_trajectories(A, pi, lengths, seed, means=None, sigmas=None, B=None, start=None, states_only=False, segment=0,
+                          device=None):
+    """Synthetic trajectories of a hidden Markov model, drawn on the GPU in one call (include/bhmm_b200.h:
+    bhmm_b200_generate_states, bhmm_b200_emit_*).
+
+    The hidden states are drawn by exact time-parallel forward simulation: the result is the same for every ``segment``
+    (frames per time-parallel segment, 0 = automatic) and equal to what one serial thread would draw from the same Philox
+    stream.  ``start``: optional first state of every trajectory (``pi`` is then not used).  The output model is Gaussian
+    (``means``, ``sigmas``) or discrete (``B``); ``states_only`` skips the observations.  ``seed=None`` takes a key from
+    ``np.random``.
+
+    Returns ``(observations, states, offsets)``: the concatenated observations (float64 or int32; None with
+    ``states_only``) and int32 states as device tensors, and the int64 row offsets (K + 1) of the trajectories, also on
+    the device.  ``TrajectoryBatch.from_concatenated(observations, lengths, N)`` takes the observations as they are."""
+    A = _stochastic(A, 'the transition matrix')
+    N = A.shape[0]
+    if A.shape != (N, N):
+        raise ValueError('the transition matrix must be square')
+    if N > 256:
+        raise NotImplementedError('synthetic trajectories support at most 256 hidden states')
+    lengths = np.asarray(lengths, dtype=np.int64).ravel()
+    if len(lengths) == 0 or np.any(lengths < 1) or np.any(lengths >= 2 ** 31):
+        raise ValueError('every trajectory needs between 1 and 2^31 - 1 frames')
+    K = len(lengths)
+    st = None
+    if start is not None:
+        st = np.ascontiguousarray(np.broadcast_to(np.asarray(start), (K,)), dtype=np.int32)
+        if np.any(st < 0) or np.any(st >= N):
+            raise ValueError('start state out of range [0, %d)' % N)
+        p0 = None
+    else:
+        p0 = _stochastic(np.reshape(pi, (1, -1)), 'the initial distribution')[0]
+        if p0.shape != (N,):
+            raise ValueError('the initial distribution must have %d entries' % N)
+    if not states_only and B is None and (means is None or sigmas is None):
+        raise ValueError('observations need means and sigmas (Gaussian) or B (discrete)')
+    seed = resolve_seed(seed)
+    torch = _torch()
+    dev = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
+    offsets = np.zeros(K + 1, dtype=np.int64)
+    np.cumsum(lengths, out=offsets[1:])
+    llp = offsets.ctypes.data_as(C.POINTER(C.c_longlong))
+    with torch.cuda.device(dev):
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        states = torch.empty(int(offsets[-1]), dtype=torch.int32, device=dev)
+        nbytes = int(lib.bhmm_b200_generate_workspace_bytes(llp, K, N, int(segment)))
+        ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+        check(lib.bhmm_b200_generate_states(C.c_void_p(states.data_ptr()), llp, K, N, dptr(A),
+                                            dptr(p0) if p0 is not None else None,
+                                            st.ctypes.data_as(C.POINTER(C.c_int)) if st is not None else None,
+                                            seed, int(segment), C.c_void_p(ws.data_ptr()), nbytes, stream))
+        del ws
+        obs = None if states_only else emit_observations(states, seed, means=means, sigmas=sigmas, B=B)
+        return obs, states, torch.as_tensor(offsets, device=dev)
+
+
 def _rel_mismatch(a, b):
     """Largest component-wise relative difference of two hand-over vectors; NaN counts as a full mismatch
     (csrc/common.cuh:rel_mismatch)."""

@@ -90,3 +90,53 @@ class HMM(object):
         parts = [np.asarray(o)[np.where(np.asarray(s) == state_index)[0]]
                  for s, o in zip(self.hidden_state_trajectories, observations)]
         return np.concatenate(parts) if parts else np.array([])
+
+    # ---- synthetic data (generic_hmm.py:433-589), drawn on the GPU (engine.generate_trajectories)
+    def generate_synthetic_state_trajectory(self, nsteps, initial_Pi=None, start=None, stop=None, dtype=np.int32,
+                                            seed=None):
+        """A hidden state trajectory of ``nsteps`` frames (generic_hmm.py:433-479).  ``start``: the first state (exclusive
+        with ``initial_Pi``, the distribution of the first state; default: this model's initial distribution).  ``stop``: a
+        state or a set of states; the trajectory ends at the first frame in one of them, that frame included.  ``seed``:
+        the key of the Philox stream (None: drawn from ``np.random``)."""
+        if initial_Pi is not None and start is not None:
+            raise ValueError('Arguments initial_Pi and start are exclusive. Only set one of them.')
+        p0 = None
+        if start is None:
+            p0 = self._Pi if initial_Pi is None else initial_Pi
+        s_t = _generate_states(self, int(nsteps), p0, start, seed)
+        if stop is not None:
+            hit = np.flatnonzero(np.isin(s_t, np.atleast_1d(stop)))
+            if len(hit):
+                s_t = s_t[:hit[0] + 1]
+        return s_t.astype(dtype)
+
+    def generate_synthetic_observation_trajectory(self, length, initial_Pi=None, seed=None):
+        """``[o_t, s_t]``: observations and hidden states of one synthetic trajectory (generic_hmm.py:481-522)."""
+        O, S = self._generate_observations([int(length)], initial_Pi, seed)
+        return [O[0], S[0]]
+
+    def generate_synthetic_observation_trajectories(self, ntrajectories, length, initial_Pi=None, seed=None):
+        """``(O, S)``: lists of observation and hidden state trajectories (generic_hmm.py:524-589), all drawn in one call and
+        returned as views of one host array each."""
+        return self._generate_observations([int(length)] * int(ntrajectories), initial_Pi, seed)
+
+    def _generate_observations(self, lengths, initial_Pi, seed):
+        from .. import engine
+        om = self.output_model
+        p0 = self._Pi if initial_Pi is None else initial_Pi
+        if om.model_type == 'gaussian':
+            kw = dict(means=om.means, sigmas=om.sigmas)
+        else:
+            kw = dict(B=om.output_probabilities)
+        obs, states, _ = engine.generate_trajectories(self._Tij, p0, lengths, seed, **kw)
+        splits = np.cumsum(lengths)[:-1]
+        return np.split(engine.download_array(obs), splits), np.split(engine.download_array(states), splits)
+
+
+def _generate_states(hmm, nsteps, p0, start, seed):
+    """Host int32 hidden states of one trajectory (the GPU generator)."""
+    from .. import engine
+    _, states, _ = engine.generate_trajectories(hmm.transition_matrix, p0, [nsteps], seed,
+                                                start=None if start is None else [int(np.ravel(start)[0])],
+                                                states_only=True)
+    return engine.download_array(states)

@@ -34,6 +34,11 @@ class DiscreteOutputModel(OutputModel):
     def nsymbols(self):
         return self._nsymbols
 
+    _observation_dtype = np.int32
+
+    def _emission_parameters(self):
+        return dict(B=self._output_probabilities)
+
     def sub_output_model(self, states):
         return DiscreteOutputModel(self._output_probabilities[states])
 

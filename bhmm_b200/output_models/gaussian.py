@@ -41,6 +41,11 @@ class GaussianOutputModel(OutputModel):
     def sigmas(self):
         return self._sigmas
 
+    _observation_dtype = np.float64
+
+    def _emission_parameters(self):
+        return dict(means=self._means, sigmas=self._sigmas)
+
     def sub_output_model(self, states):
         return GaussianOutputModel(len(states), means=self._means[states], sigmas=self._sigmas[states],
                                    ignore_outliers=self.ignore_outliers)

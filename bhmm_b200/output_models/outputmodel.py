@@ -41,3 +41,28 @@ class OutputModel(object):
         self.p_obs(obs, out=out)
         np.log(out, out=out)
         return out
+
+    # ---- synthetic observations (gaussian.py:322-390, discrete.py:253-318), drawn on the GPU (engine.emit_observations)
+    def generate_observation_trajectory(self, s_t, seed=None):
+        """One observation for every hidden state of the trajectory ``s_t``.  ``seed``: the key of the Philox stream
+        (None: drawn from ``np.random``); observation t depends only on (s_t[t], seed, t)."""
+        s = np.asarray(s_t)
+        if s.ndim != 1:
+            raise ValueError('s_t must be a 1-D array of hidden states')
+        if s.size and (not np.issubdtype(s.dtype, np.integer) or s.min() < 0 or s.max() >= self.nstates):
+            raise ValueError('hidden states must be integers in [0, %d)' % self.nstates)
+        from .. import engine
+        seed = engine.resolve_seed(seed)
+        if s.size == 0:
+            return np.empty(0, dtype=self._observation_dtype)
+        torch = engine._torch()
+        d_s = torch.from_numpy(np.ascontiguousarray(s, dtype=np.int32)).cuda()
+        return engine.download_array(engine.emit_observations(d_s, seed, **self._emission_parameters()))
+
+    def generate_observations_from_state(self, state_index, nobs, seed=None):
+        """``nobs`` observations of hidden state ``state_index``."""
+        return self.generate_observation_trajectory(np.full(int(nobs), state_index, dtype=np.int64), seed=seed)
+
+    def generate_observation_from_state(self, state_index, seed=None):
+        """One observation of hidden state ``state_index``."""
+        return self.generate_observations_from_state(state_index, 1, seed=seed)[0]

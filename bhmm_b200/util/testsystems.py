@@ -113,3 +113,37 @@ def perturbed_initial_model(A_true, means_true, nstates):
     A0 = A0 * tilt
     A0 /= A0.sum(axis=1)[:, None]
     return np.ones(N) / N, A0, np.asarray(means_true) + 0.5, np.ones(N)
+
+
+def dalton_model(nstates=3, omin=-5, omax=5, sigma_min=0.5, sigma_max=2.0, lifetime_max=100, lifetime_min=10,
+                 reversible=True, output='gaussian', seed=None):
+    """The dalton test model as an ``HMM`` (testsystems.py:105-188): parameters from ``dalton_parameters``; a discrete
+    output model emits nstates symbols with B = 0.6 on the diagonal and 0.4 / (nstates - 1) elsewhere.  ``seed=None``
+    draws the generator's seed from ``np.random``."""
+    from ..hmm.generic_hmm import HMM
+    from ..output_models import DiscreteOutputModel, GaussianOutputModel
+    rng = np.random.default_rng(np.random.randint(0, 2 ** 63 - 1, dtype=np.int64) if seed is None else seed)
+    pi, A, means, sigmas = dalton_parameters(nstates, omin=omin, omax=omax, sigma_min=sigma_min, sigma_max=sigma_max,
+                                             lifetime_max=lifetime_max, lifetime_min=lifetime_min, reversible=reversible,
+                                             rng=rng)
+    if output == 'gaussian':
+        output_model = GaussianOutputModel(nstates, means=means, sigmas=sigmas)
+    elif output == 'discrete':
+        B = np.full((nstates, nstates), 0.4 / (nstates - 1) if nstates > 1 else 0.0)
+        np.fill_diagonal(B, 0.6 if nstates > 1 else 1.0)
+        output_model = DiscreteOutputModel(B)
+    else:
+        raise Exception("output_model_type = '%s' unknown" % output)
+    return HMM(pi, A, output_model)
+
+
+def generate_synthetic_observations(nstates=3, ntrajectories=10, length=10000, omin=-5, omax=5, sigma_min=0.5,
+                                    sigma_max=2.0, lifetime_max=100, lifetime_min=10, output='gaussian', reversible=True,
+                                    seed=None):
+    """``[model, O, S]``: a dalton model and ntrajectories synthetic trajectories drawn from it on the GPU
+    (testsystems.py:191-250).  ``seed`` fixes both the model and the trajectories (None: both from ``np.random``)."""
+    model = dalton_model(nstates=nstates, omin=omin, omax=omax, sigma_min=sigma_min, sigma_max=sigma_max,
+                         lifetime_max=lifetime_max, lifetime_min=lifetime_min, reversible=reversible, output=output,
+                         seed=seed)
+    O, S = model.generate_synthetic_observation_trajectories(ntrajectories=ntrajectories, length=length, seed=seed)
+    return [model, O, S]

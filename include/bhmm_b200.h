@@ -242,6 +242,29 @@ int bhmm_b200_mstep_dev(const double* d_stats, const double* d_means_old, int N,
  * receives the transposed table. */
 int bhmm_b200_mstep_discrete_dev(const double* d_Bnum, int N, int M, double* d_B, double* d_Bt, void* stream);
 
+/* ---- synthetic trajectories (HMM.generate_synthetic_*, bhmm/hmm/generic_hmm.py:433-589) --------------------------
+ * Hidden states of K trajectories (host offsets as in bhmm_b200_batch_create) drawn by exact time-parallel forward
+ * simulation of the chain, then one observation per frame.  The stream: with row the frame's index in the call and
+ * U(seed, c, row) the 53-bit uniform of Philox4x32-10 (key = seed, counter = (row, c)),
+ *   s_0 = start[k], or the smallest i with U(seed, 0, row) < cum0[i];   s_t = smallest i with U(seed, 0, row) < cumA[s_{t-1}][i]
+ * where the cumulative tables are sequential float64 sums of the rows of p0 / A, set to exactly 1.0 from the last
+ * positive entry on.  Only comparisons are involved, so the states do not depend on the device or on `segment` (frames
+ * per time-parallel segment, 0 = automatic).  A and p0 are HOST arrays (p0 may be NULL when start is given); d_states
+ * (device, rows int32) receives the states; the workspace (device) holds bhmm_b200_generate_workspace_bytes bytes
+ * (0: invalid arguments).  N <= 256; every trajectory has 1 to 2^31 - 1 frames. */
+size_t bhmm_b200_generate_workspace_bytes(const long long* offsets, int K, int N, int segment);
+int bhmm_b200_generate_states(int* d_states, const long long* offsets, int K, int N, const double* A, const double* p0,
+                              const int* start, unsigned long long seed, int segment, void* d_workspace, size_t bytes,
+                              void* stream);
+/* Observations of d_states (device, rows int32; a state outside [0, N) fails with BHMM_B200_ERR_INVALID).
+ * Gaussian: Box-Muller on the Philox block (seed, counter (row, 1)): u1 = ((bits of words 0,1 >> 11) + 1) 2^-53,
+ * u2 = (bits of words 2,3 >> 11) 2^-53, o = means[s] + sigmas[s] sqrt(-2 log u1) cospi(2 u2); d_obs device float64.
+ * Discrete: o = smallest m with U(seed, 1, row) < cumB[s][m]; B host (N, M); d_obs device int32. */
+int bhmm_b200_emit_gaussian(double* d_obs, const int* d_states, long long rows, int N, const double* means,
+                            const double* sigmas, unsigned long long seed, void* stream);
+int bhmm_b200_emit_discrete(int* d_obs, const int* d_states, long long rows, int N, int M, const double* B,
+                            unsigned long long seed, void* stream);
+
 /* ---- (4) the estimators' one-off transfers -------------------------------------------------------- */
 /* The reference estimators take a LIST of host arrays (maximum_likelihood.py:60-144, bayesian_sampling.py:60-150) and return
  * one hidden-state path per trajectory (maximum_likelihood.py:332-352).  upload_ragged concatenates K pageable host arrays
