@@ -90,6 +90,11 @@ _proto('bhmm_b200_batch_set_family', C.c_int, _vp, C.c_int)
 _proto('bhmm_b200_batch_set_viterbi_phase', C.c_int, _vp, C.c_int)
 _proto('bhmm_b200_batch_set_viterbi_end_state', C.c_int, _vp, C.c_int, C.c_int)
 _proto('bhmm_b200_batch_set_viterbi_only', C.c_int, _vp, C.c_int)
+_proto('bhmm_b200_batch_set_gibbs_phase', C.c_int, _vp, C.c_int)
+_proto('bhmm_b200_batch_set_philox_rows', C.c_int, _vp, _llp)
+_proto('bhmm_b200_batch_set_gibbs_borders', C.c_int, _vp, _ip)
+_proto('bhmm_b200_batch_set_gibbs_enter_state', C.c_int, _vp, C.c_int, C.c_int)
+_proto('bhmm_b200_batch_gibbs_shard_map', C.c_int, _vp, C.c_int, _vp)
 _proto('bhmm_b200_batch_workspace_bytes', C.c_size_t, _vp)
 _proto('bhmm_b200_batch_attach_workspace', C.c_int, _vp, _vp, C.c_size_t)
 _proto('bhmm_b200_batch_info', None, _vp, _dp)

@@ -23,6 +23,19 @@ struct bhmm_b200_batch {
     int vit_phase = 0;
     bool vit_map_chunked = false;
     std::vector<int> vit_end;
+    // Gibbs sweep on a time shard (gibbs_shard): phase 1 = forward, table and whole-shard maps, 2 = link, replay and
+    // statistics; the segment table then covers the owned frames only (gibbs_seg)
+    int gibbs_phase = 0;
+    bool gibbs_seg = false, gibbs_mapped = false, gsh_ready = false;
+    std::vector<long long> philox_base;      // per trajectory: Philox row of local frame 0 (empty: the batch row)
+    std::vector<int> gibbs_flags, gibbs_enter;
+    std::vector<unsigned char> shard_map;   // (K, N) whole-shard maps of the last phase 1
+    std::vector<int> lev_n;                 // map composition: groups per level ...
+    std::vector<size_t> lev_off;            // ... and where each level's (beg, len) table starts
+    Arena gsh;                              // device: own ranges, Philox bases, flags, entering states, level tables, maps
+    long long *d_own_lo = nullptr, *d_own_hi = nullptr, *d_base = nullptr, *d_beg = nullptr;
+    int *d_flags = nullptr, *d_enter = nullptr, *d_len = nullptr;
+    unsigned char* d_lev[2] = {nullptr, nullptr};
     bool lane = false;          // small-N fast path (lane_kernels.cuh) instead of the team family
     bool no_alpha = false;      // Viterbi-only batch: no (rows, N) forward variables in the workspace
     double* d_g0buf = nullptr;
@@ -185,8 +198,21 @@ void batch_plan(bhmm_b200_batch* b, int chunk, int warm)
     b->warm_min = warm > 0 ? warm : 32;       // an explicit warm-up length is a floor for the adaptation
     build_plan(b->offsets.data(), b->K, b->chunk, b->plan, b->own_lo.empty() ? nullptr : b->own_lo.data(),
                b->own_hi.empty() ? nullptr : b->own_hi.data());
-    build_plan(b->offsets.data(), b->K, SEG_FRAMES, b->segplan);
+    if (b->gibbs_seg) {
+        // segments over the owned frames, with t0 and T counted from own_lo: the link kernels then see a trajectory that
+        // starts at the first owned frame and ends at the last
+        build_plan(b->offsets.data(), b->K, SEG_FRAMES, b->segplan, b->own_lo.data(), b->own_hi.data());
+        for (int k = 0; k < b->K; ++k)
+            for (int q = b->segplan.first_chain[k]; q >= 0 && q <= b->segplan.last_chain[k]; ++q) {
+                b->segplan.t0[q] -= (int)b->own_lo[k];
+                b->segplan.T[q] = (int)(b->own_hi[k] - b->own_lo[k]);
+            }
+    } else {
+        build_plan(b->offsets.data(), b->K, SEG_FRAMES, b->segplan);
+    }
     b->carved = false;
+    b->gsh_ready = false;
+    b->gibbs_mapped = false;
 }
 
 int upload_small(double* dst, const double* src, size_t n, cudaStream_t st)
@@ -474,6 +500,152 @@ int gibbs_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, 
     return BHMM_OK;
 }
 
+constexpr int COMPOSE_FAN_IN = 32;   // segment maps composed by one thread per level of the whole-shard map reduction
+
+// Device tables of the sharded sweep: the level tables of the map composition are planned from the segment table once per
+// plan.  Level 0 composes each trajectory's segment maps in groups of COMPOSE_FAN_IN, every further level the previous
+// level's outputs, until one map per trajectory is left (a trajectory without segments gets the identity at level 0).
+int gibbs_shard_setup(bhmm_b200_batch* b, cudaStream_t st)
+{
+    if (b->gsh_ready) return BHMM_OK;
+    const int K = b->K, N = b->N;
+    const HostPlan& sp = b->segplan;
+    std::vector<long long> start(K), beg;
+    std::vector<int> cnt(K), len;
+    for (int k = 0; k < K; ++k) {
+        start[k] = std::max(sp.first_chain[k], 0);
+        cnt[k] = sp.first_chain[k] < 0 ? 0 : sp.last_chain[k] - sp.first_chain[k] + 1;
+    }
+    b->lev_n.clear(); b->lev_off.clear();
+    size_t maxn = 1;
+    for (;;) {
+        b->lev_off.push_back(beg.size());
+        long long o = 0;
+        for (int k = 0; k < K; ++k) {
+            const int ng = cnt[k] == 0 ? 1 : (cnt[k] + COMPOSE_FAN_IN - 1) / COMPOSE_FAN_IN;
+            for (int g = 0; g < ng; ++g) {
+                beg.push_back(start[k] + (long long)g * COMPOSE_FAN_IN);
+                len.push_back(std::min(COMPOSE_FAN_IN, cnt[k] - g * COMPOSE_FAN_IN));
+            }
+            start[k] = o; cnt[k] = ng; o += ng;
+        }
+        b->lev_n.push_back((int)o);
+        maxn = std::max(maxn, (size_t)o);
+        if (o == K) break;                   // one map per trajectory
+    }
+    Carver cv;
+    const size_t o_lo = cv.add<long long>(K), o_hi = cv.add<long long>(K), o_base = cv.add<long long>(K);
+    const size_t o_fl = cv.add<int>(K), o_en = cv.add<int>(K);
+    const size_t o_beg = cv.add<long long>(beg.size()), o_len = cv.add<int>(len.size());
+    const size_t o_l0 = cv.add<unsigned char>(maxn * N), o_l1 = cv.add<unsigned char>(maxn * N);
+    RC_TRY(b->gsh.ensure(cv.off + 256));
+    char* base = b->gsh.base;
+    b->d_own_lo = (long long*)(base + o_lo); b->d_own_hi = (long long*)(base + o_hi); b->d_base = (long long*)(base + o_base);
+    b->d_flags = (int*)(base + o_fl); b->d_enter = (int*)(base + o_en);
+    b->d_beg = (long long*)(base + o_beg); b->d_len = (int*)(base + o_len);
+    b->d_lev[0] = (unsigned char*)(base + o_l0); b->d_lev[1] = (unsigned char*)(base + o_l1);
+    CUDA_TRY(cudaMemcpyAsync(b->d_own_lo, b->own_lo.data(), sizeof(long long) * K, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b->d_own_hi, b->own_hi.data(), sizeof(long long) * K, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b->d_beg, beg.data(), sizeof(long long) * beg.size(), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b->d_len, len.data(), sizeof(int) * len.size(), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaStreamSynchronize(st));     // the host tables go out of scope
+    b->gsh_ready = true;
+    return BHMM_OK;
+}
+
+ShardRows shard_rows(const bhmm_b200_batch* b)
+{
+    ShardRows sh{};
+    sh.offsets = b->d_offsets; sh.K = b->K;
+    sh.own_lo = b->d_own_lo; sh.own_hi = b->d_own_hi;
+    sh.base = b->philox_base.empty() ? nullptr : b->d_base;
+    sh.flags = b->d_flags; sh.enter = b->d_enter;
+    return sh;
+}
+
+// Gibbs sweep over the owned frames of a time shard, in two phases with an exchange between them (bhmm_b200.h).
+// Phase 1: forward on the team / panel family (warm-up on the halo before the owned range), the table of the owned rows and,
+// per trajectory, the map from the state at the frame after the local end to the state at the first owned frame.
+// Phase 2: from the handed-in states, link and replay the segments and count the statistics of the owned frames.
+int gibbs_shard(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, const double* pi, const double* d_u,
+                unsigned long long seed, unsigned long long sweep, int* d_path, long long* d_counts, double* d_sums,
+                double* loglik_host, cudaStream_t st)
+{
+    const int N = b->N, K = b->K;
+    if (b->no_alpha) { bhmm_set_error(BHMM_ERR_UNSUPPORTED, "Viterbi-only batch: no forward variables"); return BHMM_ERR_UNSUPPORTED; }
+    if (N > 256) { bhmm_set_error(BHMM_ERR_UNSUPPORTED, "sampling supports N <= 256"); return BHMM_ERR_UNSUPPORTED; }
+    if (b->lane) { bhmm_set_error(BHMM_ERR_UNSUPPORTED, "sampling on a time shard runs the team family (bhmm_b200_batch_set_family(b, 0))"); return BHMM_ERR_UNSUPPORTED; }
+    for (int k = 0; k < K; ++k)
+        if (b->own_lo[k] < b->own_hi[k] && b->own_hi[k] != b->offsets[k + 1] - b->offsets[k]) {
+            bhmm_set_error(BHMM_ERR_INVALID, "sampling on a time shard: the local trajectory must end with its owned range");
+            return BHMM_ERR_INVALID;
+        }
+    RC_TRY(gibbs_shard_setup(b, st));
+    if (b->gibbs_flags.empty()) b->gibbs_flags.assign(K, SHARD_STARTS);
+    if (b->gibbs_enter.empty()) b->gibbs_enter.assign(K, -1);
+    CUDA_TRY(cudaMemcpyAsync(b->d_flags, b->gibbs_flags.data(), sizeof(int) * K, cudaMemcpyHostToDevice, st));
+    if (!b->philox_base.empty())
+        CUDA_TRY(cudaMemcpyAsync(b->d_base, b->philox_base.data(), sizeof(long long) * K, cudaMemcpyHostToDevice, st));
+    const ShardRows sh0 = shard_rows(b);
+    if (b->gibbs_phase == 1) {
+        b->gibbs_mapped = false;
+        RC_TRY(upload_small(b->d_A, A, (size_t)N * N, st));
+        RC_TRY(upload_small(b->d_pi, pi, N, st));
+        b->w.ch.warm = b->warm_f;
+        ScanGuard scan_guard(b, em, emkind);
+        if (b->profile) cudaEventRecord(b->ev[0], st);
+        RC_TRY(run_forward(b->w, em, emkind, N, b->d_A, b->d_pi, b->d_alpha, b->info, st));
+        if (b->profile) cudaEventRecord(b->ev[1], st);
+        if (b->w.chunked) b->warm_f = adapt_warm(b->warm_f, b->w.need_f, b->info.worst_f, b->info.fix_f > 0, b->warm_min, b->plan.maxT, b->edge_f);
+        CUDA_TRY(cudaMemsetAsync(b->d_err, 0, sizeof(int), st));
+        if (b->profile) cudaEventRecord(b->ev[2], st);
+        RC_TRY(launch_sample_table_shard(b->d_alpha, b->d_A, d_u, seed, sweep, b->d_offsets, K, N, b->rows, b->d_F, b->d_err, sh0, st));
+        RC_TRY(launch_chase_maps(b->d_F, b->seg, N, b->seg_map, st));
+        const unsigned char* src = b->seg_map;
+        for (size_t L = 0; L < b->lev_n.size(); ++L) {
+            RC_TRY(launch_compose_maps(src, b->d_beg + b->lev_off[L], b->d_len + b->lev_off[L], b->lev_n[L], N, b->d_lev[L & 1], st));
+            src = b->d_lev[L & 1];
+        }
+        if (b->profile) cudaEventRecord(b->ev[3], st);
+        LAUNCHED(2 + b->lev_n.size());
+        b->shard_map.assign((size_t)K * N, 0);
+        int err = 0;
+        CUDA_TRY(cudaMemcpyAsync(b->shard_map.data(), src, (size_t)K * N, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(&err, b->d_err, sizeof(int), cudaMemcpyDeviceToHost, st));
+        RC_TRY(finish_stream(st));
+        if (err) { bhmm_set_error(err, "sample_path: no state could be drawn"); return err; }
+        collect_times(b);
+        b->gibbs_mapped = true;
+        return BHMM_OK;
+    }
+    if (!b->gibbs_mapped) { bhmm_set_error(BHMM_ERR_INVALID, "Gibbs phase 2 on a time shard needs phase 1 first"); return BHMM_ERR_INVALID; }
+    for (int k = 0; k < K; ++k) {
+        const bool cont = (b->gibbs_flags[k] & SHARD_CONTINUES) && b->own_lo[k] < b->own_hi[k];
+        if (cont && (b->gibbs_enter[k] < 0 || b->gibbs_enter[k] >= N)) {
+            bhmm_set_error(BHMM_ERR_INVALID, "Gibbs on a time shard: a trajectory that continues needs its entering state in [0, N)");
+            return BHMM_ERR_INVALID;
+        }
+    }
+    CUDA_TRY(cudaMemcpyAsync(b->d_enter, b->gibbs_enter.data(), sizeof(int) * K, cudaMemcpyHostToDevice, st));
+    if (b->profile) cudaEventRecord(b->ev[0], st);
+    RC_TRY(launch_chase_resolve_shard(b->d_F, b->seg, N, b->seg_map, b->seg_enter, d_path, sh0, st));
+    CUDA_TRY(cudaMemsetAsync(d_counts, 0, sizeof(long long) * ((size_t)N * N + 2 * N), st));
+    if (d_sums) CUDA_TRY(cudaMemsetAsync(d_sums, 0, sizeof(double) * 2 * N, st));
+    RC_TRY(launch_path_stats_shard(d_path, d_sums ? em.obs : nullptr, b->d_offsets, K, N, b->rows, d_counts,
+                                   d_counts + (size_t)N * N, d_counts + (size_t)N * N + N, d_sums, d_sums ? d_sums + N : nullptr,
+                                   sh0, st));
+    if (b->profile) { cudaEventRecord(b->ev[1], st); cudaEventRecord(b->ev[2], st); cudaEventRecord(b->ev[3], st); }
+    LAUNCHED(3);
+    std::vector<double> ll(b->w.n_total);
+    CUDA_TRY(cudaMemcpyAsync(ll.data(), b->w.chain_ll, sizeof(double) * b->w.n_total, cudaMemcpyDeviceToHost, st));
+    RC_TRY(finish_stream(st));
+    collect_times(b);
+    double s = 0.0;
+    for (double v : ll) s += v;
+    if (loglik_host) *loglik_host = s;
+    return BHMM_OK;
+}
+
 }  // namespace
 
 extern "C" int bhmm_b200_stats_len_gaussian(int N) { return 1 + N + N * N + 3 * N; }
@@ -527,6 +699,7 @@ extern "C" void bhmm_b200_batch_destroy(bhmm_b200_batch* b)
     b->arena.release();
     b->disc.release();
     b->scan.release();
+    b->gsh.release();
     for (int k = 0; k < 4; ++k) if (b->ev[k]) cudaEventDestroy(b->ev[k]);
     delete b;
 }
@@ -782,6 +955,52 @@ extern "C" int bhmm_b200_batch_set_viterbi_end_state(bhmm_b200_batch* b, int k, 
     return BHMM_OK;
 }
 
+extern "C" int bhmm_b200_batch_set_gibbs_phase(bhmm_b200_batch* b, int phase)
+{
+    if (!b || phase < 0 || phase > 2) { bhmm_set_error(BHMM_ERR_INVALID, "Gibbs phase must be 0, 1 or 2"); return BHMM_ERR_INVALID; }
+    if (phase != 0 && b->own_lo.empty()) { bhmm_set_error(BHMM_ERR_INVALID, "Gibbs phases are for time shards (batches with owned ranges)"); return BHMM_ERR_INVALID; }
+    b->gibbs_phase = phase;
+    const bool seg = phase != 0;
+    if (seg != b->gibbs_seg) {                  // the segment table changes: re-plan, the workspace is laid out again
+        b->gibbs_seg = seg;
+        batch_plan(b, b->req_chunk, b->req_warm);
+    }
+    return BHMM_OK;
+}
+
+extern "C" int bhmm_b200_batch_set_philox_rows(bhmm_b200_batch* b, const long long* base)
+{
+    if (!b) return BHMM_ERR_INVALID;
+    if (base) b->philox_base.assign(base, base + b->K);
+    else b->philox_base.clear();
+    return BHMM_OK;
+}
+
+extern "C" int bhmm_b200_batch_set_gibbs_borders(bhmm_b200_batch* b, const int* flags)
+{
+    if (!b) return BHMM_ERR_INVALID;
+    if (!flags) { b->gibbs_flags.clear(); return BHMM_OK; }
+    for (int k = 0; k < b->K; ++k)
+        if (flags[k] & ~(SHARD_CONTINUES | SHARD_STARTS)) { bhmm_set_error(BHMM_ERR_INVALID, "unknown Gibbs border flag"); return BHMM_ERR_INVALID; }
+    b->gibbs_flags.assign(flags, flags + b->K);
+    return BHMM_OK;
+}
+
+extern "C" int bhmm_b200_batch_set_gibbs_enter_state(bhmm_b200_batch* b, int k, int state)
+{
+    if (!b || k < 0 || k >= b->K || state < -1 || state >= b->N) { bhmm_set_error(BHMM_ERR_INVALID, "Gibbs entering state: bad trajectory or state"); return BHMM_ERR_INVALID; }
+    if ((int)b->gibbs_enter.size() != b->K) b->gibbs_enter.assign(b->K, -1);
+    b->gibbs_enter[k] = state;
+    return BHMM_OK;
+}
+
+extern "C" int bhmm_b200_batch_gibbs_shard_map(const bhmm_b200_batch* b, int k, unsigned char* out)
+{
+    if (!b || !out || k < 0 || k >= b->K || !b->gibbs_mapped) { bhmm_set_error(BHMM_ERR_INVALID, "gibbs_shard_map: bad arguments or no phase 1 yet"); return BHMM_ERR_INVALID; }
+    std::memcpy(out, b->shard_map.data() + (size_t)k * b->N, (size_t)b->N);
+    return BHMM_OK;
+}
+
 extern "C" int bhmm_b200_viterbi_gaussian(bhmm_b200_batch* b, const double* d_obs, const double* A, const double* pi,
                                           const double* means, const double* sigmas, int ignore_outliers,
                                           int* d_path, void* stream)
@@ -824,6 +1043,7 @@ extern "C" int bhmm_b200_gibbs_gaussian(bhmm_b200_batch* b, const double* d_obs,
     RC_TRY(upload_small(b->d_sigma, sigmas, b->N, st));
     Emission em{};
     em.obs = d_obs; em.mu = b->d_mu; em.sigma = b->d_sigma; em.ignore_outliers = ignore_outliers;
+    if (b->gibbs_phase) return gibbs_shard(b, em, EM_GAUSS, A, pi, d_u, seed, sweep, d_path, d_counts, d_sums, loglik_host, st);
     return gibbs_common(b, em, EM_GAUSS, A, pi, means, sigmas, d_u, seed, sweep, d_path, d_counts, d_sums, loglik_host, st);
 }
 
@@ -839,6 +1059,7 @@ extern "C" int bhmm_b200_gibbs_discrete(bhmm_b200_batch* b, const int* d_obs, co
     Emission em{};
     em.sym = d_obs; em.ignore_outliers = ignore_outliers;
     RC_TRY(prepare_discrete(b, B, M, em, st));
+    if (b->gibbs_phase) return gibbs_shard(b, em, EM_DISC, A, pi, d_u, seed, sweep, d_path, d_counts, nullptr, loglik_host, st);
     return gibbs_common(b, em, EM_DISC, A, pi, nullptr, nullptr, d_u, seed, sweep, d_path, d_counts, nullptr, loglik_host, st);
 }
 

@@ -177,6 +177,19 @@ int launch_finalize_stats(const double* partials, int grid, const double* chain_
                           int N, double* stats, cudaStream_t st);
 
 // ---- forward-filter / backward-sample and path statistics (sample_kernels.cu)
+// A sampling batch of a time shard (engine.cu: gibbs_shard): local trajectory k owns the frames [own_lo[k], own_hi[k]) and
+// ends with them (no right halo).  All arrays are device memory with one entry per local trajectory.
+enum { SHARD_CONTINUES = 1,   // the trajectory goes on after the local end: the last owned row is an ordinary row
+       SHARD_STARTS = 2 };    // local frame 0 is the trajectory's frame 0 (n0 is counted)
+struct ShardRows {
+    const long long* offsets;   // (K+1) local row offsets
+    int K;
+    const long long* own_lo;
+    const long long* own_hi;
+    const long long* base;      // Philox row of local frame 0 (NULL: the batch row)
+    const int* flags;
+    const int* enter;           // state at the frame after the local end (-1: none)
+};
 // choice table F[row][s'] = state drawn at `row` given the next frame's state s' and the frame's uniform.
 int launch_sample_table(const double* alpha, const double* A, const double* u, const long long* offsets, int K,
                         int N, long long rows, unsigned char* F, int* err, cudaStream_t st);
@@ -192,6 +205,19 @@ int launch_chase_link(const Chains& seg, int N, const unsigned char* seg_map, in
 int launch_path_stats(const int* path, const double* obs, const long long* offsets, int K, int N, long long rows,
                       long long* Cint, long long* n0, long long* cnt, double* so, double* soo, cudaStream_t st);
 int launch_symbol_histogram(const int* path, const int* sym, long long rows, int N, int M, long long* hist,
+                            cudaStream_t st);
+// time shards: the table of the owned rows (u == NULL: Philox), the segment maps alone, one level of their per-trajectory
+// composition, the link from the handed-in states + replay, and the statistics of the owned frames
+int launch_sample_table_shard(const double* alpha, const double* A, const double* u, unsigned long long seed,
+                              unsigned long long ctr, const long long* offsets, int K, int N, long long rows,
+                              unsigned char* F, int* err, const ShardRows& sh, cudaStream_t st);
+int launch_chase_maps(const unsigned char* F, const Chains& seg, int N, unsigned char* seg_map, cudaStream_t st);
+int launch_compose_maps(const unsigned char* src, const long long* beg, const int* len, int n, int N, unsigned char* dst,
+                        cudaStream_t st);
+int launch_chase_resolve_shard(const unsigned char* F, const Chains& seg, int N, const unsigned char* seg_map, int* seg_enter,
+                               int* path, const ShardRows& sh, cudaStream_t st);
+int launch_path_stats_shard(const int* path, const double* obs, const long long* offsets, int K, int N, long long rows,
+                            long long* Cint, long long* n0, long long* cnt, double* so, double* soo, const ShardRows& sh,
                             cudaStream_t st);
 // ---- synthetic trajectories (sample_kernels.cu).  `seg` is the segment table in REVERSED time order (t0 counted from the
 // trajectory's end, see k_gen_map); cum0 (N) and cumA (N,N) are the cumulative tables; seg_start[c] >= 0 fixes the first

@@ -64,19 +64,34 @@ __device__ __forceinline__ int traj_of_row(const long long* __restrict__ offsets
     return lo;
 }
 
-template <bool PHILOX>
+// frame t of local trajectory k of a time shard: the owned range, the Philox row and whether the next frame exists
+__device__ __forceinline__ bool shard_owned(const ShardRows& sh, int tr, long long t)
+{
+    return t >= sh.own_lo[tr] && t < sh.own_hi[tr];
+}
+
+// SHARD: a sampling batch of a time shard (ShardRows): only owned rows get a table, frame t of trajectory k draws the Philox
+// row base[k] + t, and the last local row of a trajectory that continues past the shard is an ordinary row
+template <bool PHILOX, bool SHARD>
 __global__ void k_sample_table(const double* __restrict__ alpha, const double* __restrict__ A,
                                const double* __restrict__ u, unsigned long long seed, unsigned long long ctr,
                                const long long* __restrict__ offsets, int K, int N, long long rows,
-                               unsigned char* __restrict__ F, int* __restrict__ err)
+                               unsigned char* __restrict__ F, int* __restrict__ err, ShardRows sh)
 {
     const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= rows * N) return;
     const long long row = k / N;
     const int sp = (int)(k - row * N);          // hypothetical state of the next frame
     const int tr = traj_of_row(offsets, K, row);
-    const bool last = (row + 1 == offsets[tr + 1]);
-    const double r = PHILOX ? philox_uniform(seed, ctr, row) : u[row];
+    bool last = (row + 1 == offsets[tr + 1]);
+    long long prow = row;
+    if (SHARD) {
+        const long long t = row - offsets[tr];
+        if (!shard_owned(sh, tr, t)) return;
+        if (sh.flags[tr] & SHARD_CONTINUES) last = false;
+        if (sh.base) prow = sh.base[tr] + t;
+    }
+    const double r = PHILOX ? philox_uniform(seed, ctr, prow) : u[row];
     const double* a = alpha + row * N;
     double s = 0.0;
     for (int i = 0; i < N; ++i) {
@@ -106,12 +121,20 @@ __global__ void k_chase_map(const unsigned char* __restrict__ F, Chains seg, int
     map[k] = (unsigned char)s;
 }
 
-__global__ void k_chase_link(Chains seg, int N, const unsigned char* __restrict__ map, int* __restrict__ enter)
+// ENTER: the walk starts from the state handed in for the trajectory (time shards, ShardRows.enter; -1 = none) instead of 0
+__device__ __forceinline__ int link_start(const ShardRows& sh, const Chains& seg, int sidx)
+{
+    const int e = sh.enter[traj_of_row(sh.offsets, sh.K, seg.row0[sidx])];
+    return e >= 0 ? e : 0;
+}
+
+template <bool ENTER>
+__global__ void k_chase_link(Chains seg, int N, const unsigned char* __restrict__ map, int* __restrict__ enter, ShardRows sh)
 {
     const int sidx = blockIdx.x * blockDim.x + threadIdx.x;
     if (sidx >= seg.n) return;
     if (seg.t0[sidx] + seg.len[sidx] < seg.T[sidx]) return;   // only the last segment of a trajectory walks
-    int s = 0;                                                // F at the last frame ignores the entering state
+    int s = ENTER ? link_start(sh, seg, sidx) : 0;            // F at the last frame ignores the entering state
     int cur = sidx;
     for (;;) {
         enter[cur] = s;
@@ -126,7 +149,9 @@ __global__ void k_chase_link(Chains seg, int N, const unsigned char* __restrict_
 // segments are contiguous, the warp copies them into shared memory with coalesced loads whose addresses do not depend on
 // the walk, lane 0 walks the 32 rows there (one shared-memory round trip per segment), the lanes store the 32 entering
 // states.  Chosen by the launchers when the batch has at least chase_tiled_threshold() segments.
-__global__ void k_chase_link_tiled(Chains seg, int N, const unsigned char* __restrict__ map, int* __restrict__ enter)
+template <bool ENTER>
+__global__ void k_chase_link_tiled(Chains seg, int N, const unsigned char* __restrict__ map, int* __restrict__ enter,
+                                   ShardRows sh)
 {
     __shared__ unsigned char tile[32 * 256];
     __shared__ int states[32];
@@ -138,7 +163,7 @@ __global__ void k_chase_link_tiled(Chains seg, int N, const unsigned char* __res
         const int l0 = __ffs(todo) - 1;
         todo &= todo - 1;
         int cur = blockIdx.x * 32 + l0;                       // the last segment of one trajectory
-        int s = 0;                                            // F at the last frame ignores the entering state
+        int s = ENTER ? link_start(sh, seg, cur) : 0;         // F at the last frame ignores the entering state
         for (;;) {
             const int lo = max(cur - 31, 0);
             const int nrows = cur - lo + 1;
@@ -179,14 +204,32 @@ __global__ void k_chase_path(const unsigned char* __restrict__ F, Chains seg, in
     }
 }
 
+// One level of the whole-shard map reduction: output map g is the composition of the source maps [beg[g], beg[g] + len[g])
+// -- consecutive segments of one trajectory in time order, so the state entering from the right goes through the last one
+// first -- and len 0 is the identity (a trajectory with no owned frames passes the state through).
+__global__ void k_compose_maps(const unsigned char* __restrict__ src, const long long* __restrict__ beg,
+                               const int* __restrict__ len, int n, int N, unsigned char* __restrict__ dst)
+{
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= (long long)n * N) return;
+    const int g = (int)(k / N);
+    int s = (int)(k - (long long)g * N);
+    const long long b = beg[g];
+    for (int j = len[g] - 1; j >= 0; --j) s = src[(b + j) * N + s];
+    dst[k] = (unsigned char)s;
+}
+
 // Gibbs path statistics (HMM.count_matrix / count_init / collect_observations_in_state,
 // bhmm/hmm/generic_hmm.py:297-334,398-431): integer lag-1 transition counts, first-state histogram, frames per
 // state, and sum(o), sum(o^2) per state.  Block-private shared-memory counters, then one global atomic each.
+// SHARD: owned frames only; the first frame counts in n0 only where the local trajectory starts the global one
+// (SHARD_STARTS), and the last owned frame of a trajectory that continues counts its transition into the handed-in state.
+template <bool SHARD>
 __global__ void k_path_stats(const int* __restrict__ path, const double* __restrict__ obs,
                              const long long* __restrict__ offsets, int K, int N, long long rows,
                              unsigned long long* __restrict__ Cint, unsigned long long* __restrict__ n0,
                              unsigned long long* __restrict__ cnt, double* __restrict__ so, double* __restrict__ soo,
-                             int use_smem)
+                             int use_smem, ShardRows shr)
 {
     extern __shared__ unsigned long long sh[];
     unsigned long long* sC = sh;                    // N*N
@@ -201,20 +244,26 @@ __global__ void k_path_stats(const int* __restrict__ path, const double* __restr
     }
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += stride) {
-        const int s = path[r];
         const int tr = traj_of_row(offsets, K, r);
-        const bool first = (r == offsets[tr]);
-        const bool last = (r + 1 == offsets[tr + 1]);
+        bool first = (r == offsets[tr]);
+        bool last = (r + 1 == offsets[tr + 1]);
+        int next = -1;                                   // SHARD: the handed-in state after the last local frame
+        if (SHARD) {
+            if (!shard_owned(shr, tr, r - offsets[tr])) continue;
+            first = first && (shr.flags[tr] & SHARD_STARTS);
+            if (last && (shr.flags[tr] & SHARD_CONTINUES)) { last = false; next = shr.enter[tr]; }
+        }
+        const int s = path[r];
         const double o = obs ? obs[r] : 0.0;
         if (use_smem) {
             atomicAdd(sc + s, 1ULL);
             if (first) atomicAdd(s0 + s, 1ULL);
-            if (!last) atomicAdd(sC + s * N + path[r + 1], 1ULL);
+            if (!last) atomicAdd(sC + s * N + (next >= 0 ? next : path[r + 1]), 1ULL);
             if (obs) { atomicAdd(sso + s, o); atomicAdd(ssoo + s, o * o); }
         } else {
             atomicAdd(cnt + s, 1ULL);
             if (first) atomicAdd(n0 + s, 1ULL);
-            if (!last) atomicAdd(Cint + (long long)s * N + path[r + 1], 1ULL);
+            if (!last) atomicAdd(Cint + (long long)s * N + (next >= 0 ? next : path[r + 1]), 1ULL);
             if (obs) { atomicAdd(so + s, o); atomicAdd(soo + s, o * o); }
         }
     }
@@ -370,7 +419,8 @@ int launch_sample_table(const double* alpha, const double* A, const double* u, c
 {
     if (N > 256) return BHMM_ERR_UNSUPPORTED;
     if (rows <= 0) return BHMM_OK;
-    k_sample_table<false><<<nblk(rows * N, 256), 256, 0, st>>>(alpha, A, u, 0ULL, 0ULL, offsets, K, N, rows, F, err);
+    k_sample_table<false, false><<<nblk(rows * N, 256), 256, 0, st>>>(alpha, A, u, 0ULL, 0ULL, offsets, K, N, rows, F, err,
+                                                                      ShardRows{});
     return BHMM_OK;
 }
 
@@ -380,8 +430,8 @@ int launch_sample_table_philox(const double* alpha, const double* A, unsigned lo
 {
     if (N > 256) return BHMM_ERR_UNSUPPORTED;
     if (rows <= 0) return BHMM_OK;
-    k_sample_table<true><<<nblk(rows * N, 256), 256, 0, st>>>(alpha, A, nullptr, seed, ctr, offsets, K, N, rows, F,
-                                                                err);
+    k_sample_table<true, false><<<nblk(rows * N, 256), 256, 0, st>>>(alpha, A, nullptr, seed, ctr, offsets, K, N, rows, F,
+                                                                       err, ShardRows{});
     return BHMM_OK;
 }
 
@@ -399,8 +449,8 @@ static int chase_tiled_threshold()
 
 static void link_segments(const Chains& seg, int N, const unsigned char* seg_map, int* seg_enter, cudaStream_t st)
 {
-    if (seg.n >= chase_tiled_threshold() && N <= 256) k_chase_link_tiled<<<nblk(seg.n, 32), 32, 0, st>>>(seg, N, seg_map, seg_enter);
-    else k_chase_link<<<nblk(seg.n, 128), 128, 0, st>>>(seg, N, seg_map, seg_enter);
+    if (seg.n >= chase_tiled_threshold() && N <= 256) k_chase_link_tiled<false><<<nblk(seg.n, 32), 32, 0, st>>>(seg, N, seg_map, seg_enter, ShardRows{});
+    else k_chase_link<false><<<nblk(seg.n, 128), 128, 0, st>>>(seg, N, seg_map, seg_enter, ShardRows{});
 }
 
 int launch_chase(const unsigned char* F, const Chains& seg, int N, unsigned char* seg_map, int* seg_enter, int* path,
@@ -420,18 +470,70 @@ int launch_chase_link(const Chains& seg, int N, const unsigned char* seg_map, in
     return BHMM_OK;
 }
 
-int launch_path_stats(const int* path, const double* obs, const long long* offsets, int K, int N, long long rows,
-                      long long* Cint, long long* n0, long long* cnt, double* so, double* soo, cudaStream_t st)
+template <bool SHARD>
+static int path_stats(const int* path, const double* obs, const long long* offsets, int K, int N, long long rows,
+                      long long* Cint, long long* n0, long long* cnt, double* so, double* soo, const ShardRows& sh,
+                      cudaStream_t st)
 {
     if (rows <= 0) return BHMM_OK;
     const int use_smem = (N <= 64) ? 1 : 0;
     const size_t smem = use_smem ? sizeof(unsigned long long) * ((size_t)N * N + 2 * N) + sizeof(double) * 2 * N : 0;
     const int blocks = (int)min((long long)148 * 8, (rows + 255) / 256);
-    k_path_stats<<<blocks, 256, smem, st>>>(path, obs, offsets, K, N, rows,
-                                            reinterpret_cast<unsigned long long*>(Cint),
-                                            reinterpret_cast<unsigned long long*>(n0),
-                                            reinterpret_cast<unsigned long long*>(cnt), so, soo, use_smem);
+    k_path_stats<SHARD><<<blocks, 256, smem, st>>>(path, obs, offsets, K, N, rows,
+                                                   reinterpret_cast<unsigned long long*>(Cint),
+                                                   reinterpret_cast<unsigned long long*>(n0),
+                                                   reinterpret_cast<unsigned long long*>(cnt), so, soo, use_smem, sh);
     return BHMM_OK;
+}
+
+int launch_path_stats(const int* path, const double* obs, const long long* offsets, int K, int N, long long rows,
+                      long long* Cint, long long* n0, long long* cnt, double* so, double* soo, cudaStream_t st)
+{
+    return path_stats<false>(path, obs, offsets, K, N, rows, Cint, n0, cnt, so, soo, ShardRows{}, st);
+}
+
+// ---- Gibbs sweep on a time shard (engine.cu: gibbs_shard)
+int launch_sample_table_shard(const double* alpha, const double* A, const double* u, unsigned long long seed,
+                              unsigned long long ctr, const long long* offsets, int K, int N, long long rows,
+                              unsigned char* F, int* err, const ShardRows& sh, cudaStream_t st)
+{
+    if (N > 256) return BHMM_ERR_UNSUPPORTED;
+    if (rows <= 0) return BHMM_OK;
+    if (u) k_sample_table<false, true><<<nblk(rows * N, 256), 256, 0, st>>>(alpha, A, u, 0ULL, 0ULL, offsets, K, N, rows, F, err, sh);
+    else k_sample_table<true, true><<<nblk(rows * N, 256), 256, 0, st>>>(alpha, A, nullptr, seed, ctr, offsets, K, N, rows, F, err, sh);
+    return BHMM_OK;
+}
+
+int launch_chase_maps(const unsigned char* F, const Chains& seg, int N, unsigned char* seg_map, cudaStream_t st)
+{
+    if (seg.n <= 0) return BHMM_OK;
+    k_chase_map<<<nblk((long long)seg.n * N, 128), 128, 0, st>>>(F, seg, N, seg_map);
+    return BHMM_OK;
+}
+
+int launch_compose_maps(const unsigned char* src, const long long* beg, const int* len, int n, int N, unsigned char* dst,
+                        cudaStream_t st)
+{
+    if (n <= 0) return BHMM_OK;
+    k_compose_maps<<<nblk((long long)n * N, 128), 128, 0, st>>>(src, beg, len, n, N, dst);
+    return BHMM_OK;
+}
+
+int launch_chase_resolve_shard(const unsigned char* F, const Chains& seg, int N, const unsigned char* seg_map, int* seg_enter,
+                               int* path, const ShardRows& sh, cudaStream_t st)
+{
+    if (seg.n <= 0) return BHMM_OK;
+    if (seg.n >= chase_tiled_threshold()) k_chase_link_tiled<true><<<nblk(seg.n, 32), 32, 0, st>>>(seg, N, seg_map, seg_enter, sh);
+    else k_chase_link<true><<<nblk(seg.n, 128), 128, 0, st>>>(seg, N, seg_map, seg_enter, sh);
+    k_chase_path<<<nblk(seg.n, 128), 128, 0, st>>>(F, seg, N, seg_enter, path);
+    return BHMM_OK;
+}
+
+int launch_path_stats_shard(const int* path, const double* obs, const long long* offsets, int K, int N, long long rows,
+                            long long* Cint, long long* n0, long long* cnt, double* so, double* soo, const ShardRows& sh,
+                            cudaStream_t st)
+{
+    return path_stats<true>(path, obs, offsets, K, N, rows, Cint, n0, cnt, so, soo, sh, st);
 }
 
 int launch_symbol_histogram(const int* path, const int* sym, long long rows, int N, int M, long long* hist,

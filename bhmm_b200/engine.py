@@ -830,6 +830,25 @@ def _rel_mismatch(a, b):
     return float(d.max())
 
 
+def compose_shard_maps(maps_by_rank, owns_by_rank):
+    """Entering states of a Gibbs sweep on time shards, from the shards' whole-shard maps (a host function; no device).
+
+    ``maps_by_rank[r][k]``: N states; shard r's map of trajectory k sends the state at the frame after its owned range to the
+    state at its first owned frame.  ``owns_by_rank[r][k]``: whether shard r owns frames of trajectory k.  The maps are
+    composed from the last shard to the first: the entering state of shard r is the state at the first owned frame of the
+    next shard that owns frames of the trajectory, -1 where none does (shard r holds the trajectory's end; its map ignores
+    the entering state).  A shard that owns nothing passes the state through.  Returns a (world, K) int64 array."""
+    world, K = len(maps_by_rank), len(owns_by_rank[0])
+    enter = np.full((world, K), -1, dtype=np.int64)
+    for k in range(K):
+        s = -1
+        for r in range(world - 1, -1, -1):
+            enter[r, k] = s
+            if owns_by_rank[r][k]:
+                s = int(maps_by_rank[r][k][max(s, 0)])
+    return enter
+
+
 class TimeShardedTrajectories(object):
     """E-step over trajectories that are cut in TIME across shards (SURVEY 8e, C5: one trajectory too long for one GPU).
 
@@ -850,7 +869,18 @@ class TimeShardedTrajectories(object):
     component-wise relative test as for the E-step); then the paths are resolved from the last shard to the first, each
     shard handing the state at its neighbour's last frame -- one integer per trajectory -- to the left.  A path that goes
     through a decision whose margin is below the certified tolerance raises (run that trajectory on one device).
-    Hidden-path sampling needs whole trajectories and is not available on shards.
+
+    Gibbs sweeps work across shards too (``gibbs_gaussian`` / ``gibbs_discrete``, ``BayesianHMMSampler(shard='time')``).
+    Given the uniforms, the draw at frame t is a function s_t = F_t(s_{t+1}) of the next state only, so every shard runs the
+    forward filter over its owned frames (warming up on the halo before them, borders certified as for Viterbi), builds the
+    table of its owned rows and composes it into one map per trajectory: from the state at the frame after its range to the
+    state at its first owned frame (``gibbs_map``).  One ``all_gather`` exchanges those maps (N bytes per trajectory) and the
+    border vectors; every shard composes the maps from the last shard to the first, which gives its entering state
+    (``compose_shard_maps``), and all shards replay their frames and count their statistics at the same time
+    (``gibbs_resolve``).  Frame t of a trajectory draws the uniform of the row it has in the UNSHARDED batch, so for the same
+    (seed, sweep) the paths are those of ``TrajectoryBatch.gibbs_*`` on the team / panel kernels, bit for bit, and the
+    statistics summed over shards are that batch's (integer counts exactly).  The forward variables of the two agree to the
+    certified tolerance only: a uniform within that tolerance of a cumulative boundary may be drawn differently.
     """
 
     def __init__(self, observations, nstates, rank, world, halo=None, device=None, chunk=0, warm=0, tol=1e-11):
@@ -862,6 +892,7 @@ class TimeShardedTrajectories(object):
         self.halo = int(halo)
         pieces, lengths, own = [], [], []
         self.global_ranges = []
+        self._starts = []                                # global frame of every local trajectory's frame 0
         for o in observations:
             o = np.asarray(o)
             T = len(o)
@@ -873,6 +904,7 @@ class TimeShardedTrajectories(object):
             lengths.append(b - a)
             own.append((lo - a, max(lo, hi) - a))
             self.global_ranges.append((lo, hi, T))
+            self._starts.append(a)
         host_dtype = np.int32 if np.issubdtype(np.asarray(observations[0]).dtype, np.integer) else np.float64
         cat = np.concatenate([np.asarray(p, dtype=host_dtype) for p in pieces])
         self.batch = TrajectoryBatch.from_concatenated(cat, lengths, self.N, device=device, chunk=chunk, warm=warm,
@@ -899,6 +931,7 @@ class TimeShardedTrajectories(object):
             raise ValueError('the piece [%d, %d) does not cover the owned range [%d, %d)' % (start, start + n, lo, hi))
         self.halo = max(lo - start, start + n - hi)
         self.global_ranges = [(lo, hi, T)]
+        self._starts = [int(start)]
         self.batch = TrajectoryBatch.from_concatenated(piece, [n], self.N, device=device, chunk=chunk, warm=warm,
                                                        own_ranges=[(lo - start, hi - start)])
         self.K = 1
@@ -909,6 +942,9 @@ class TimeShardedTrajectories(object):
         if getattr(self, '_vbatch', None) is not None:
             self._vbatch.close()
             self._vbatch = None
+        if getattr(self, '_gbatch', None) is not None:
+            self._gbatch.close()
+            self._gbatch = None
 
     def info(self):
         return self.batch.info()
@@ -976,16 +1012,17 @@ class TimeShardedTrajectories(object):
         return paths
 
     @staticmethod
-    def certify_viterbi(borders_by_rank, ranges_by_rank, tol):
-        """Worst relative mismatch of the max-product hand-overs at the shard borders; raises above ``tol``."""
+    def certify_viterbi(borders_by_rank, ranges_by_rank, tol, what='Viterbi'):
+        """Worst relative mismatch of the max-product (or, for the Gibbs sweep, forward) hand-overs at the shard borders:
+        the vector each shard started from against the one its left neighbour computed; raises above ``tol``."""
         world, worst = len(borders_by_rank), 0.0
         for k in range(len(ranges_by_rank[0])):
             owners = [r for r in range(world) if ranges_by_rank[r][k][1] > ranges_by_rank[r][k][0]]
             for left, right in zip(owners, owners[1:]):
                 worst = max(worst, _rel_mismatch(borders_by_rank[right][k][0], borders_by_rank[left][k][1]))
         if worst > tol:
-            raise RuntimeError('time-sharded Viterbi: a shard border disagrees by %.3g (tolerance %.3g); the halo is too '
-                               'short for this model -- increase halo=' % (worst, tol))
+            raise RuntimeError('time-sharded %s: a shard border disagrees by %.3g (tolerance %.3g); the halo is too '
+                               'short for this model -- increase halo=' % (what, worst, tol))
         return worst
 
     @classmethod
@@ -1034,6 +1071,191 @@ class TimeShardedTrajectories(object):
 
     def viterbi_discrete(self, A, pi, B, ignore_outliers=False):
         return self.viterbi((A, pi, B, ignore_outliers), 'discrete')
+
+    # ------------------------------------------------------------------------------------------ Gibbs sweeps across shards
+    def _gibbs_batch(self):
+        """The shard's sampling batch: frames [a, hi) of every trajectory (left halo + owned range, no right halo: the forward
+        filter only looks back, and the draws look forward only through the handed-in state), with forward variables, on
+        the team / panel family, drawing the Philox rows of the unsharded batch."""
+        if getattr(self, '_gbatch', None) is None:
+            b = self.batch
+            pieces, lengths, own = [], [], []
+            for k in range(self.K):
+                lo_l, hi_l = b._own_ranges[k]
+                r0 = int(b.offsets[k])
+                n = max(hi_l, 1)                         # a trajectory with no owned frames keeps one halo frame
+                pieces.append(b.obs[r0:r0 + n])
+                lengths.append(n)
+                own.append((lo_l, hi_l))
+            cat = b.torch.cat(pieces) if len(pieces) > 1 else pieces[0]
+            gb = TrajectoryBatch.from_concatenated(cat, lengths, self.N, device=b.device, own_ranges=own)
+            check(lib.bhmm_b200_batch_set_family(gb._handle, 0))
+            check(lib.bhmm_b200_batch_set_gibbs_phase(gb._handle, 1))
+            gb._workspace = None                         # the segment table changed: lay the workspace out again
+            gb._attach()
+            T = np.asarray([g[2] for g in self.global_ranges], dtype=np.int64)
+            goff = np.concatenate([[0], np.cumsum(T)[:-1]]).astype(np.int64)
+            base = np.ascontiguousarray(goff + np.asarray(self._starts, dtype=np.int64))
+            flags = np.zeros(self.K, dtype=np.int32)
+            for k, (lo, hi, Tk) in enumerate(self.global_ranges):
+                if hi > lo and hi < Tk:
+                    flags[k] |= 1                        # the trajectory continues after this shard
+                if self._starts[k] == 0:
+                    flags[k] |= 2                        # local frame 0 is the trajectory's frame 0
+            check(lib.bhmm_b200_batch_set_philox_rows(gb._handle, base.ctypes.data_as(C.POINTER(C.c_longlong))))
+            check(lib.bhmm_b200_batch_set_gibbs_borders(gb._handle, flags.ctypes.data_as(C.POINTER(C.c_int))))
+            self._gbatch, self._grow0 = gb, base
+        return self._gbatch
+
+    def _local_uniforms(self, uniforms):
+        """The rows of ``uniforms`` (one per row of the UNSHARDED batch) that the sampling batch's frames have there."""
+        if uniforms is None:
+            return None
+        gb = self._gibbs_batch()
+        torch = gb.torch
+        u = uniforms if torch.is_tensor(uniforms) else torch.from_numpy(np.ascontiguousarray(uniforms, dtype=np.float64))
+        parts = [u[int(self._grow0[k]):int(self._grow0[k]) + int(gb.lengths[k])] for k in range(self.K)]
+        return torch.cat(parts).to(device=gb.device, dtype=torch.float64).contiguous()
+
+    def _gibbs_call(self, phase, seed=0, sweep=0, uniforms=None):
+        gb = self._gibbs_batch()
+        model, kind = self._gibbs_model
+        check(lib.bhmm_b200_batch_set_gibbs_phase(gb._handle, int(phase)))
+        path = gb._path_buffer()
+        counts, sums = gb._gibbs_buffers()
+        ll = C.c_double(0.0)
+        u_dev = self._local_uniforms(uniforms) if phase == 1 else None
+        u = C.c_void_p(u_dev.data_ptr()) if u_dev is not None else None
+        with gb.torch.cuda.device(gb.device):
+            if kind == 'gaussian':
+                A, pi, means, sigmas, io = model
+                if gb.discrete:
+                    raise TypeError('this batch holds integer symbols; a Gaussian output model needs float observations')
+                A_, pi_, m_, s_ = f64(A), f64(pi), f64(means), f64(sigmas)
+                rc = lib.bhmm_b200_gibbs_gaussian(gb._handle, C.c_void_p(gb.obs.data_ptr()), dptr(A_), dptr(pi_), dptr(m_),
+                                                  dptr(s_), int(bool(io)), u, C.c_ulonglong(int(seed)), C.c_ulonglong(int(sweep)),
+                                                  C.c_void_p(path.data_ptr()), C.c_void_p(counts.data_ptr()),
+                                                  C.c_void_p(sums.data_ptr()), C.byref(ll), gb._stream())
+            else:
+                A, pi, B, io = model
+                A_, pi_, B_ = f64(A), f64(pi), f64(B)
+                gb._require_discrete(B_.shape[1])
+                rc = lib.bhmm_b200_gibbs_discrete(gb._handle, C.c_void_p(gb.obs.data_ptr()), dptr(A_), dptr(pi_), dptr(B_),
+                                                  B_.shape[1], int(bool(io)), u, C.c_ulonglong(int(seed)),
+                                                  C.c_ulonglong(int(sweep)), C.c_void_p(path.data_ptr()),
+                                                  C.c_void_p(counts.data_ptr()), C.byref(ll), gb._stream())
+        check(rc)
+        return ll.value
+
+    def gibbs_map(self, model, kind='gaussian', seed=0, sweep=0, uniforms=None):
+        """Phase 1 of a Gibbs sweep: forward filter, table of the owned rows and the whole-shard maps.  ``model``:
+        (A, pi, means, sigmas, ignore_outliers) or (A, pi, B, ignore_outliers); ``uniforms``: optional uniforms of the
+        UNSHARDED batch's rows (reference parity), default Philox keyed by (seed, sweep).  Returns the (K, N) uint8 maps
+        (map k sends the state at the frame after the owned range to the state at its first owned frame; the identity where
+        the shard owns nothing of trajectory k) and the (K, 2, N) forward border vectors [used at lo - 1, end at hi - 1]."""
+        self._gibbs_model = (model, kind)
+        self._gibbs_call(1, seed, sweep, uniforms)
+        gb = self._gibbs_batch()
+        maps = np.zeros((self.K, self.N), dtype=np.uint8)
+        for k in range(self.K):
+            check(lib.bhmm_b200_batch_gibbs_shard_map(gb._handle, k, C.c_void_p(maps[k].ctypes.data)))
+        return maps, np.array([gb.border_handovers(k)[:2] for k in range(self.K)])
+
+    def gibbs_resolve(self, enter_states):
+        """Phase 2: replay the owned frames from the state of every trajectory at the frame after this shard's range (-1
+        where the shard holds the trajectory's end) and count their statistics.  Returns (paths, counts, sums or histogram,
+        loglik): the owned-range paths as int32 DEVICE views (one per trajectory), int64 [C | n0 | frames per state],
+        float64 [sum o | sum o^2] (Gaussian) or the (N, M) int64 symbol histogram (discrete), and the log-likelihood of the
+        owned frames.  All statistics cover the owned frames and add over shards."""
+        gb = self._gibbs_batch()
+        for k in range(self.K):
+            lo, hi, T = self.global_ranges[k]
+            e = int(enter_states[k]) if (hi > lo and hi < T) else -1
+            check(lib.bhmm_b200_batch_set_gibbs_enter_state(gb._handle, k, e))
+        ll = self._gibbs_call(2)
+        path = gb._path
+        counts, sums = gb._counts, gb._sums
+        paths = [path[int(gb.offsets[k]) + gb._own_ranges[k][0]:int(gb.offsets[k]) + gb._own_ranges[k][1]]
+                 for k in range(self.K)]
+        model, kind = self._gibbs_model
+        if kind == 'gaussian':
+            return paths, counts, sums, ll
+        B = f64(model[2])
+        N, M = B.shape
+        hist = gb.torch.zeros((N, M), dtype=gb.torch.int64, device=gb.device)
+        with gb.torch.cuda.device(gb.device):
+            for k, p in enumerate(paths):
+                if p.numel() == 0:
+                    continue
+                r = int(gb.offsets[k]) + gb._own_ranges[k][0]
+                check(lib.bhmm_b200_path_symbol_histogram(C.c_void_p(p.data_ptr()), C.c_void_p(gb.obs.data_ptr() + 4 * r),
+                                                          C.c_longlong(p.numel()), N, M, C.c_void_p(hist.data_ptr()),
+                                                          gb._stream()))
+        return paths, counts, hist, ll
+
+    @classmethod
+    def gibbs_combine(cls, shards, model, kind='gaussian', seed=0, sweep=0, uniforms=None):
+        """Single-process use (tests): one Gibbs sweep over all shards in this process.  Returns (list over trajectories of
+        the full int32 paths, summed counts, summed sums or histogram, summed loglik, worst border mismatch) -- the
+        statistics as host tensors."""
+        results = [s.gibbs_map(model, kind, seed, sweep, uniforms) for s in shards]
+        worst = cls.certify_viterbi([b for _, b in results], [s.global_ranges for s in shards], shards[0].tol, 'Gibbs sweep')
+        owns = [[g[1] > g[0] for g in s.global_ranges] for s in shards]
+        enter = compose_shard_maps([m for m, _ in results], owns)
+        K = shards[0].K
+        parts = [[] for _ in range(K)]
+        counts = extra = None
+        ll = 0.0
+        for r, s in enumerate(shards):
+            paths, c, e, l = s.gibbs_resolve(enter[r])
+            for k, p in enumerate(s.split_owned(paths)):
+                parts[k].append(p)
+            counts = c.cpu().clone() if counts is None else counts + c.cpu()
+            extra = e.cpu().clone() if extra is None else extra + e.cpu()
+            ll += l
+        return [np.concatenate(p) for p in parts], counts, extra, ll, worst
+
+    def gibbs(self, model, kind='gaussian', seed=0, sweep=0, uniforms=None):
+        """Distributed use (one process per shard, torch.distributed initialised when world > 1): ONE all_gather of the
+        whole-shard maps and border vectors, then every shard replays its own frames.  Returns what ``gibbs_resolve``
+        does, for this shard's owned frames; the worst border mismatch is kept in ``last_gibbs_worst``."""
+        maps, borders = self.gibbs_map(model, kind, seed, sweep, uniforms)
+        enter, self.last_gibbs_worst = self.gibbs_exchange(maps, borders, [T for (_, _, T) in self.global_ranges], self.rank,
+                                                           self.world, self.tol, self.batch.device)
+        return self.gibbs_resolve(enter)
+
+    @classmethod
+    def gibbs_exchange(cls, maps, borders, lengths, rank, world, tol, device):
+        """The exchange of a distributed Gibbs sweep: ONE all_gather of this shard's (K, N) maps and (K, 2, N) border vectors
+        (as one float64 tensor on ``device``), certification of the borders, and the composition of all shards' maps.
+        ``lengths``: the K trajectory lengths.  Returns (entering states of this shard, worst border mismatch)."""
+        K, N = np.shape(maps)
+        pack = np.concatenate([np.asarray(borders, dtype=np.float64).reshape(-1), np.asarray(maps).reshape(-1).astype(np.float64)])
+        if world > 1:
+            import torch
+            import torch.distributed as td
+            mine = torch.from_numpy(pack).to(device)
+            gathered = [torch.empty_like(mine) for _ in range(world)]
+            td.all_gather(gathered, mine)
+            got = [g.cpu().numpy() for g in gathered]
+        else:
+            got = [pack]
+        ranges = [[((T * r) // world, (T * (r + 1)) // world, T) for T in lengths] for r in range(world)]
+        worst = cls.certify_viterbi([g[:K * 2 * N].reshape(K, 2, N) for g in got], ranges, tol, 'Gibbs sweep')
+        owns = [[rg[1] > rg[0] for rg in ranges[r]] for r in range(world)]
+        enter = compose_shard_maps([g[K * 2 * N:].reshape(K, N).astype(np.int64) for g in got], owns)
+        return enter[rank], worst
+
+    def gibbs_gaussian(self, A, pi, means, sigmas, seed=0, sweep=0, uniforms=None, ignore_outliers=True):
+        return self.gibbs((A, pi, means, sigmas, ignore_outliers), 'gaussian', seed, sweep, uniforms)
+
+    def gibbs_discrete(self, A, pi, B, seed=0, sweep=0, uniforms=None, ignore_outliers=False):
+        return self.gibbs((A, pi, B, ignore_outliers), 'discrete', seed, sweep, uniforms)
+
+    @staticmethod
+    def split_owned(paths):
+        """Host copies of the owned-range paths returned by ``gibbs_*`` (one device-to-host copy each)."""
+        return [download_array(p) if p.numel() else np.zeros(0, dtype=np.int32) for p in paths]
 
     def estep_gaussian_local(self, A, pi, means, sigmas, ignore_outliers=True):
         """Local statistics (device tensor) and the (K, 4, N) border hand-overs of this shard."""

@@ -17,14 +17,22 @@ import time
 import numpy as np
 
 from .. import dist
-from ..engine import TrajectoryBatch, make_batch, download_array
+from ..engine import TrajectoryBatch, TimeShardedTrajectories, make_batch, download_array
 from ..util import config
 from ..util.logger import logger
 from ..util import tmatrix as _tmatrix
 
 
 class BayesianHMMSampler(object):
-    """Bayesian hidden Markov model sampler (bayesian_sampling.py:33-204)."""
+    """Bayesian hidden Markov model sampler (bayesian_sampling.py:33-204).
+
+    ``shard=True`` (default) gives every rank of a torch.distributed job a contiguous block of whole trajectories;
+    ``shard='time'`` cuts EVERY trajectory in time over the ranks instead (``engine.TimeShardedTrajectories``: one trajectory
+    too long for one GPU), and ``batch=`` may then be a ``TimeShardedTrajectories`` the caller built, e.g. with
+    ``from_local_piece``.  With time shards the hidden paths are the ones one GPU would draw for the same key: the Philox key
+    is the same on every rank and every frame draws the uniform of its row in the unsharded data set.
+    ``save_hidden_state_trajectory`` then keeps, on each rank, the paths of the frames that rank owns.
+    """
 
     def __init__(self, observations, nstates, initial_model=None, reversible=True, stationary=False,
                  transition_matrix_sampling_steps=1000, p0_prior='mixed', transition_matrix_prior='mixed',
@@ -34,6 +42,7 @@ class BayesianHMMSampler(object):
         if initial_model is None:
             raise NotImplementedError('bhmm_b200 needs initial_model= (bhmm.init_hmm is outside the hot path)')
         self.reversible = reversible
+        self._time_sharded = (isinstance(shard, str) and shard == 'time') or isinstance(batch, TimeShardedTrajectories)
         # Host-side parameter draws.  One process: numpy's global RNG, as in the reference (np.random.seed reproduces a
         # run).  Sharded over several ranks: every rank must draw the SAME parameters from the all-reduced statistics, so
         # the ranks agree on one seed (rank 0's next global draw) and use a private stream from it.
@@ -44,7 +53,7 @@ class BayesianHMMSampler(object):
         self.stationary = stationary
         self.nstates = nstates
         dist.tune_for_world()
-        if shard and dist.world_size() > 1:
+        if shard and dist.world_size() > 1 and not self._time_sharded:
             lo, hi = dist.shard_bounds([len(o) for o in observations], dist.rank(), dist.world_size())
         else:
             lo, hi = 0, len(observations)
@@ -81,7 +90,13 @@ class BayesianHMMSampler(object):
         self.transition_matrix_sampling_steps = transition_matrix_sampling_steps
         self.model.output_model.set_implementation(config.kernel)
         # batch=: an engine batch that already holds these trajectories on the GPU (no second upload)
-        self._batch = batch if batch is not None else (make_batch(self.observations, nstates, chunk=chunk, warm=warm) if self.nobs else None)
+        if batch is not None:
+            self._batch = batch
+        elif self._time_sharded:
+            self._batch = TimeShardedTrajectories(self.observations, nstates, dist.rank(), dist.world_size(), chunk=chunk,
+                                                  warm=warm)
+        else:
+            self._batch = make_batch(self.observations, nstates, chunk=chunk, warm=warm) if self.nobs else None
         self._sweep = 0
         # Philox key of the hidden-path draws.  Without an explicit seed= in sample() it comes from the agreed host stream
         # (np.random.seed makes a run reproducible, two samplers do not share their uniforms; the reference continues
@@ -125,8 +140,9 @@ class BayesianHMMSampler(object):
         om = self.model.output_model
         A, pi = self.model.transition_matrix, self.model.initial_distribution
         st = {}
-        # a different Philox key per rank keeps the shards' draws independent
-        seed = self._seed * 1000003 + dist.rank()
+        # a different Philox key per rank keeps the shards' draws independent; time shards draw the rows of ONE data set
+        # under one key
+        seed = self._seed * 1000003 + (0 if self._time_sharded else dist.rank())
         N = self.nstates
         if self._batch is None:
             # empty shard (more ranks than trajectories): zero statistics, so that the collectives below still match
@@ -153,7 +169,9 @@ class BayesianHMMSampler(object):
         st.update(C=c[:N * N].reshape(N, N).copy(), n0=c[N * N:N * N + N].copy(), count=c[N * N + N:].copy())
         self._sweep += 1
         self.last_loglik = ll
-        if keep_paths and self._batch is not None:
+        if keep_paths and self._time_sharded:
+            self.model.hidden_state_trajectories = self._batch.split_owned(path)   # this rank's owned piece of every trajectory
+        elif keep_paths and self._batch is not None:
             self.model.hidden_state_trajectories = list(self._batch.split(download_array(path)))   # views of one fresh host copy
         return st
 

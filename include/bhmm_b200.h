@@ -137,7 +137,8 @@ int bhmm_b200_batch_create(bhmm_b200_batch** out, const long long* offsets, int 
  *   [3] the backward vector at the first owned frame            (beta at own_lo)
  * -- so that the caller compares [0] with the previous shard's [1] and [2] with the next shard's [3]
  * (bhmm_b200.engine.TimeShardedTrajectories does, component-wise and relatively, with the engine's tolerance).
- * Viterbi and hidden-path sampling need whole trajectories and return BHMM_B200_ERR_UNSUPPORTED on such a batch. */
+ * Viterbi and hidden-path sampling return BHMM_B200_ERR_UNSUPPORTED on such a batch unless their time-shard phases are set
+ * (bhmm_b200_batch_set_viterbi_phase, bhmm_b200_batch_set_gibbs_phase). */
 int bhmm_b200_batch_create_ranges(bhmm_b200_batch** out, const long long* offsets, const long long* own_lo,
                                   const long long* own_hi, int K, int N, int chunk, int warm);
 int bhmm_b200_batch_border_handovers(const bhmm_b200_batch* b, int k, double* out);
@@ -225,6 +226,31 @@ int bhmm_b200_gibbs_discrete(bhmm_b200_batch* b, const int* d_obs, const double*
                              const double* B, int M, int ignore_outliers, const double* d_u,
                              unsigned long long seed, unsigned long long sweep, int* d_path, long long* d_counts,
                              double* loglik_host, void* stream);
+/* Gibbs hidden-path sweep of trajectories cut in TIME across devices.  A sampling shard is a batch with owned ranges whose
+ * local trajectories END with their owned range (halo frames before it, none after), on the team / panel family
+ * (bhmm_b200_batch_set_family(b, 0); N <= 256).  Given the uniforms, the draw at frame t is a function s_t = F_t(s_{t+1}) of the
+ * next state only, so the shard's owned frames of trajectory k reduce to one map of N states: from the state at the frame
+ * after the local end to the state at the first owned frame.
+ *   phase 1: bhmm_b200_gibbs_* runs the forward filter (warm-up on the halo), the table of the owned rows and those maps;
+ *            bhmm_b200_batch_gibbs_shard_map copies map k (N bytes) to the host.  The forward border vectors are in
+ *            bhmm_b200_batch_border_handovers, rows 0 and 1, for the caller to compare across shards.
+ *   phase 2: bhmm_b200_gibbs_* links and replays the owned frames from the states set by
+ *            bhmm_b200_batch_set_gibbs_enter_state (state of trajectory k at the frame after its local end; -1 = the shard
+ *            holds the trajectory's end) and returns the statistics of the owned frames: the transition out of the last owned
+ *            frame into the entering state belongs to this shard, n0 is counted only where local frame 0 is the
+ *            trajectory's frame 0, the log-likelihood covers the owned frames.  Summed over shards they are the statistics
+ *            of the whole trajectories.  d_path is filled for the owned rows only.
+ *   phase 0 (default): whole trajectories only; a batch with owned ranges is refused.
+ * bhmm_b200_batch_set_philox_rows: frame t of local trajectory k draws the Philox row base[k] + t (NULL: the batch row), so
+ * that a shard draws the uniforms of the rows its frames have in the unsharded batch.  bhmm_b200_batch_set_gibbs_borders:
+ * per trajectory, flag 1 = the trajectory continues after the local end (its last owned row is an ordinary row), flag 2 =
+ * local frame 0 is the trajectory's frame 0 (NULL: flag 2 for every trajectory).  Bad phases, flags, states, a right halo
+ * and phase 2 before phase 1 are rejected with BHMM_B200_ERR_INVALID. */
+int bhmm_b200_batch_set_gibbs_phase(bhmm_b200_batch* b, int phase);
+int bhmm_b200_batch_set_philox_rows(bhmm_b200_batch* b, const long long* base);
+int bhmm_b200_batch_set_gibbs_borders(bhmm_b200_batch* b, const int* flags);
+int bhmm_b200_batch_set_gibbs_enter_state(bhmm_b200_batch* b, int k, int state);
+int bhmm_b200_batch_gibbs_shard_map(const bhmm_b200_batch* b, int k, unsigned char* out);
 /* Per-state symbol histogram of sampled paths (DiscreteOutputModel.sample's bincount, discrete.py:240-245):
  * d_hist (device int64, N*M) += [path==i][obs==m]. */
 int bhmm_b200_path_symbol_histogram(const int* d_path, const int* d_obs, long long rows, int N, int M,
