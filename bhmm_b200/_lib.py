@@ -95,6 +95,9 @@ _proto('bhmm_b200_batch_set_philox_rows', C.c_int, _vp, _llp)
 _proto('bhmm_b200_batch_set_gibbs_borders', C.c_int, _vp, _ip)
 _proto('bhmm_b200_batch_set_gibbs_enter_state', C.c_int, _vp, C.c_int, C.c_int)
 _proto('bhmm_b200_batch_gibbs_shard_map', C.c_int, _vp, C.c_int, _vp)
+_proto('bhmm_b200_shard_operators_gaussian', C.c_int, _vp, _vp, _dp, _dp, _dp, _dp, C.c_int, _vp, _vp)
+_proto('bhmm_b200_shard_operators_discrete', C.c_int, _vp, _vp, _dp, _dp, _dp, C.c_int, C.c_int, _vp, _vp)
+_proto('bhmm_b200_batch_set_border_starts', C.c_int, _vp, C.c_int, _dp, _dp)
 _proto('bhmm_b200_batch_workspace_bytes', C.c_size_t, _vp)
 _proto('bhmm_b200_batch_attach_workspace', C.c_int, _vp, _vp, C.c_size_t)
 _proto('bhmm_b200_batch_info', None, _vp, _dp)

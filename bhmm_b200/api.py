@@ -187,9 +187,10 @@ def init_hmm(observations, nstates, lag=1, output=None, reversible=True):
 # estimation
 # --------------------------------------------------------------------------------------------------------------------
 def estimate_hmm(observations, nstates, lag=1, initial_model=None, output=None, reversible=True, stationary=False, p=None,
-                 accuracy=1e-3, maxit=1000, maxit_P=100000, mincount_connectivity=1e-2):
+                 accuracy=1e-3, maxit=1000, maxit_P=100000, mincount_connectivity=1e-2, shard=True):
     """Maximum-likelihood HMM by Baum-Welch EM on the GPU engine (api.py:309-372).  `initial_model=None` uses
-    ``init_hmm``."""
+    ``init_hmm``.  ``shard`` goes to ``MaximumLikelihoodEstimator``: True (default) spreads whole trajectories over the ranks
+    of a torch.distributed job, 'time' cuts every trajectory in time over them."""
     if output is None:
         output = _guess_output_type(observations)
     if lag > 1:
@@ -201,7 +202,7 @@ def estimate_hmm(observations, nstates, lag=1, initial_model=None, output=None, 
     from .estimators.maximum_likelihood import MaximumLikelihoodEstimator
     est = MaximumLikelihoodEstimator(observations, nstates, initial_model=initial_model, output=output,
                                      reversible=reversible, stationary=stationary, p=p, accuracy=accuracy, maxit=maxit,
-                                     maxit_P=maxit_P)
+                                     maxit_P=maxit_P, shard=shard)
     est.fit()
     est.hmm._lag = lag
     return est.hmm

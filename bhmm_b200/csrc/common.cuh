@@ -51,7 +51,33 @@ struct Chains {
     int warm;               // warm-up frames (used when warmv is NULL)
     const int* warmv;       // optional per-chain warm-up lengths, adapted by the certification (certify.cu)
     int exact;              // 1: fix-up pass, start from the recorded exact hand-over vector instead of warming up
+    // optional per-chain starts of a time shard's E-step (engine.cu: border_setup), NULL elsewhere: chain c with gidx[c] >= 0
+    // starts from the given border vector gvec + gidx[c] * N (forward: alpha at t0 - 1, backward: beta at t0 + len) instead
+    // of a warm-up; gidx[c] == CHAIN_WARMS_UP marks a chain at the border of the owned range whose neighbour in the table is
+    // not its neighbour in time, so that it keeps its warm-up in an exact pass too
+    const int* gidx;
+    const double* gvec;
 };
+constexpr int CHAIN_WARMS_UP = -2;
+
+__device__ __forceinline__ bool chain_start_given(const Chains& ch, int c) { return ch.gidx != nullptr && ch.gidx[c] >= 0; }
+
+// whether chain c starts from an exact vector (mode 2 of the chain kernels) rather than from pi or a warm-up
+__device__ __forceinline__ bool chain_exact_start(const Chains& ch, int c)
+{
+    if (ch.gidx) {
+        const int g = ch.gidx[c];
+        return g >= 0 || (ch.exact && g != CHAIN_WARMS_UP);
+    }
+    return ch.exact != 0;
+}
+
+// Where an exact start of chain c is read: its given border start, else the end vector of its neighbour nb in hand_end
+// (nb = c - 1 forward, c + 1 backward); rows of `stride` doubles.
+__device__ __forceinline__ const double* chain_start_vec(const Chains& ch, const double* hand_end, int c, int nb, int stride)
+{
+    return chain_start_given(ch, c) ? ch.gvec + (long long)ch.gidx[c] * stride : hand_end + (long long)nb * stride;
+}
 
 __device__ __forceinline__ double gauss_pdf(double o, double mu, double sigma)
 {

@@ -5,6 +5,7 @@
 // of MaximumLikelihoodEstimator.fit (maximum_likelihood.py:383-385), compute_viterbi_paths (:332-352) and
 // BayesianHMMSampler._updateHiddenStateTrajectories (bayesian_sampling.py:283-291).
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -64,6 +65,14 @@ struct bhmm_b200_batch {
     unsigned* d_vflag = nullptr;   // chunked Viterbi: near-tie flags per row of the back-pointer map
     Arena disc;                 // B staging + Bt for the discrete model (sized on first use)
     Arena scan;                 // transfer operators of the exact-scan fallback (scan_kernels.cu; allocated when first needed)
+    // border starts of a time shard (bhmm_b200_batch_set_border_starts): per trajectory an exact alpha at own_lo - 1 and / or
+    // beta at own_hi (host, K x N each), and their device tables for the E-step (chain -> row, rows)
+    std::vector<double> bs_f, bs_b;
+    std::vector<char> has_f, has_b;
+    bool bst_ok = false;        // the device tables match the plan and the starts
+    Arena bst;
+    int *d_gidx_f = nullptr, *d_gidx_b = nullptr;
+    double *d_gvec_f = nullptr, *d_gvec_b = nullptr;
     RunInfo info;
     // optional per-kernel timing (CUDA events on the launching stream)
     bool profile = false;
@@ -213,6 +222,7 @@ void batch_plan(bhmm_b200_batch* b, int chunk, int warm)
     b->carved = false;
     b->gsh_ready = false;
     b->gibbs_mapped = false;
+    b->bst_ok = false;
 }
 
 int upload_small(double* dst, const double* src, size_t n, cudaStream_t st)
@@ -276,6 +286,64 @@ int prepare_discrete(bhmm_b200_batch* b, const double* B, int M, Emission& em, c
     return BHMM_OK;
 }
 
+bool border_starts_set(const bhmm_b200_batch* b)
+{
+    for (int k = 0; k < (int)b->has_f.size(); ++k)
+        if (b->has_f[k] || b->has_b[k]) return true;
+    return false;
+}
+
+// Per-chain start tables of a time shard's E-step (Chains.gidx / gvec).  The first owned chain of trajectory k starts its
+// forward recursion from row k of gvec_f where a border start is set, the last owned chain its backward recursion from row k
+// of gvec_b; without one, a chain whose owned range does not begin at the trajectory's start (forward) or end at its end
+// (backward) is marked CHAIN_WARMS_UP: its neighbour in the chain table belongs to another trajectory, so it keeps its halo
+// warm-up in the exact passes after the transfer-operator scan as well.  Every other chain: -1.
+int border_setup(bhmm_b200_batch* b, cudaStream_t st)
+{
+    if (b->bst_ok) return BHMM_OK;
+    const int K = b->K, N = b->N, n = b->w.n_total;
+    const bool given = (int)b->has_f.size() == K;
+    if (!given) {
+        b->bs_f.assign((size_t)K * N, 0.0); b->bs_b.assign((size_t)K * N, 0.0);
+    }
+    std::vector<int> gf(std::max(n, 1), -1), gb(std::max(n, 1), -1);
+    for (int k = 0; k < K; ++k) {
+        const int cf = b->plan.first_chain[k], cl = b->plan.last_chain[k];
+        if (cf < 0) continue;
+        if (given && b->has_f[k]) gf[cf] = k;
+        else if (b->plan.t0[cf] > 0) gf[cf] = CHAIN_WARMS_UP;
+        if (given && b->has_b[k]) gb[cl] = k;
+        else if (b->plan.t0[cl] + b->plan.len[cl] < b->plan.T[cl]) gb[cl] = CHAIN_WARMS_UP;
+    }
+    Carver cv;
+    const size_t o_if = cv.add<int>(gf.size()), o_ib = cv.add<int>(gb.size());
+    const size_t o_vf = cv.add<double>((size_t)K * N), o_vb = cv.add<double>((size_t)K * N);
+    RC_TRY(b->bst.ensure(cv.off + 256));
+    char* base = b->bst.base;
+    b->d_gidx_f = (int*)(base + o_if); b->d_gidx_b = (int*)(base + o_ib);
+    b->d_gvec_f = (double*)(base + o_vf); b->d_gvec_b = (double*)(base + o_vb);
+    CUDA_TRY(cudaMemcpyAsync(b->d_gidx_f, gf.data(), sizeof(int) * gf.size(), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b->d_gidx_b, gb.data(), sizeof(int) * gb.size(), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b->d_gvec_f, b->bs_f.data(), sizeof(double) * K * N, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b->d_gvec_b, b->bs_b.data(), sizeof(double) * K * N, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaStreamSynchronize(st));     // the host tables go out of scope
+    b->bst_ok = true;
+    return BHMM_OK;
+}
+
+// Hands the per-chain start tables of one direction to the chain launches of a pass; removed again at the end.
+struct BorderGuard {
+    ChainWork& w;
+    bool on;
+    explicit BorderGuard(ChainWork& w_, bool on_) : w(w_), on(on_) {}
+    void use(const bhmm_b200_batch* b, int dir)
+    {
+        w.ch.gidx = (on && dir != 0) ? (dir > 0 ? b->d_gidx_f : b->d_gidx_b) : nullptr;
+        w.ch.gvec = (on && dir != 0) ? (dir > 0 ? b->d_gvec_f : b->d_gvec_b) : nullptr;
+    }
+    ~BorderGuard() { w.ch.gidx = nullptr; w.ch.gvec = nullptr; }
+};
+
 // forward + (backward & statistics with whole-pass retry) + finalize
 int estep_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, const double* pi, const double* mu,
                  const double* sigma, double* d_gamma, double* d_stats, double* d_Bnum, cudaStream_t st)
@@ -287,6 +355,9 @@ int estep_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, 
     b->w.ch.warm = b->warm_f;
     ScanGuard scan_guard(b, em, emkind);
     RepairTolGuard repair_guard(b->w);
+    const bool borders = !b->own_lo.empty();
+    if (borders) RC_TRY(border_setup(b, st));
+    BorderGuard border_guard(b->w, borders);
     LaneArgs la{};
     LaneHostParams hp{A, pi, mu, sigma};
     if (b->lane) {
@@ -336,7 +407,7 @@ int estep_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, 
         }
         return BHMM_OK;
     };
-    if (optimistic && b->w.chunked) {
+    if (optimistic && b->w.chunked && !border_starts_set(b)) {
         Chains all = b->w.ch;
         all.list = nullptr; all.n = b->w.n_total; all.exact = 0; all.warmv = nullptr;
         b->w.need_f = b->w.need_b = 0.0;
@@ -368,7 +439,9 @@ int estep_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, 
     }
 
     if (b->profile) cudaEventRecord(b->ev[0], st);
+    border_guard.use(b, +1);
     RC_TRY(run_chains_certified(b->w, N, +1, launch_fwd, b->info, st));
+    border_guard.use(b, -1);
     if (b->profile) cudaEventRecord(b->ev[1], st);
     if (b->w.chunked) b->warm_f = adapt_warm(b->warm_f, b->w.need_f, b->info.worst_f, b->info.fix_f > 0, b->warm_min, b->plan.maxT, b->edge_f);
 
@@ -388,7 +461,10 @@ int estep_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, 
         if (nfail == 0) { b->warm_b = adapt_warm(b->warm_b, b->w.need_b, b->info.worst_b, false, b->warm_min, b->plan.maxT, b->edge_b); break; }
         // statistics of a failed pass cannot be patched chain by chain: lengthen the warm-up (at least +32 frames, up to
         // the longest trajectory, which is an exact start) and redo the pass.
-        if (exact_bwd || b->warm_b >= b->plan.maxT) {
+        // a warm-up as long as the longest trajectory starts every chain from an exact end -- except on a time shard, whose
+        // local trajectories end in a halo: there the scan takes over
+        const bool capped = b->warm_b >= b->plan.maxT;
+        if (exact_bwd || (capped && (b->own_lo.empty() || !b->w.scan))) {
             char msg[160];
             snprintf(msg, sizeof(msg), "backward hand-overs not certified (%lld chains, worst mismatch %.3g%s)", nfail, b->info.worst_b,
                      exact_bwd ? ", after the exact scan" : "");
@@ -397,7 +473,7 @@ int estep_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, 
         }
         b->info.fix_b += 1;
         b->info.rerun += (double)b->w.n_total;
-        if (attempt >= 1 && b->w.scan) {
+        if ((attempt >= 1 || capped) && b->w.scan) {
             // a longer warm-up did not help either: the model does not forget.  Exact starts from the transfer-operator
             // scan (the hand-over vectors the failed pass left behind are exact at the trajectory ends), then the pass once more
             RC_TRY(b->w.scan(-1, st));
@@ -699,6 +775,7 @@ extern "C" void bhmm_b200_batch_destroy(bhmm_b200_batch* b)
     b->arena.release();
     b->disc.release();
     b->scan.release();
+    b->bst.release();
     b->gsh.release();
     for (int k = 0; k < 4; ++k) if (b->ev[k]) cudaEventDestroy(b->ev[k]);
     delete b;
@@ -720,6 +797,37 @@ extern "C" int bhmm_b200_batch_border_handovers(const bhmm_b200_batch* b, int k,
                             b->w.he_b + (size_t)cf * N};
     for (int q = 0; q < 4; ++q)
         CUDA_TRY(cudaMemcpy(out + q * N, src[q], sizeof(double) * N, cudaMemcpyDeviceToHost));
+    return BHMM_OK;
+}
+
+extern "C" int bhmm_b200_batch_set_border_starts(bhmm_b200_batch* b, int k, const double* fwd, const double* bwd)
+{
+    bhmm_set_error(BHMM_OK, "");
+    if (!b || b->own_lo.empty()) { bhmm_set_error(BHMM_ERR_INVALID, "border starts are for time shards (batches with owned ranges)"); return BHMM_ERR_INVALID; }
+    if (k < 0 || k >= b->K) { bhmm_set_error(BHMM_ERR_INVALID, "border starts: trajectory out of range"); return BHMM_ERR_INVALID; }
+    const int N = b->N;
+    const long long T = b->offsets[k + 1] - b->offsets[k];
+    auto bad = [N](const double* v) {
+        double s = 0.0;
+        for (int i = 0; i < N; ++i) {
+            if (!(v[i] >= 0.0) || !std::isfinite(v[i])) return true;         // NaN, negative, infinite
+            s += v[i];
+        }
+        return !(s > 0.0);
+    };
+    if ((fwd || bwd) && b->own_lo[k] >= b->own_hi[k]) { bhmm_set_error(BHMM_ERR_INVALID, "border starts: the shard owns no frame of this trajectory"); return BHMM_ERR_INVALID; }
+    if (fwd && b->own_lo[k] == 0) { bhmm_set_error(BHMM_ERR_INVALID, "forward border start: the owned range starts at local frame 0 (the trajectory's start)"); return BHMM_ERR_INVALID; }
+    if (bwd && b->own_hi[k] >= T) { bhmm_set_error(BHMM_ERR_INVALID, "backward border start: the owned range ends with the local trajectory (the trajectory's end)"); return BHMM_ERR_INVALID; }
+    if ((fwd && bad(fwd)) || (bwd && bad(bwd))) { bhmm_set_error(BHMM_ERR_INVALID, "border starts must be finite, non-negative and not all zero"); return BHMM_ERR_INVALID; }
+    if ((int)b->has_f.size() != b->K) {
+        b->has_f.assign(b->K, 0); b->has_b.assign(b->K, 0);
+        b->bs_f.assign((size_t)b->K * N, 0.0); b->bs_b.assign((size_t)b->K * N, 0.0);
+    }
+    b->has_f[k] = fwd != nullptr;
+    b->has_b[k] = bwd != nullptr;
+    b->bst_ok = false;
+    if (fwd) std::copy(fwd, fwd + N, b->bs_f.begin() + (size_t)k * N);
+    if (bwd) std::copy(bwd, bwd + N, b->bs_b.begin() + (size_t)k * N);
     return BHMM_OK;
 }
 
@@ -848,6 +956,88 @@ extern "C" int bhmm_b200_estep_discrete(bhmm_b200_batch* b, const int* d_obs, co
     RC_TRY(finish_stream(st));
     collect_times(b);
     return BHMM_OK;
+}
+
+// Operators of the owned frames of every trajectory (bhmm_b200.h): k_chain_operator[_wide] over the batch's chains, then the
+// per-trajectory tree reduction (k_compose_operators), forward and backward, into d_out (K, 2, N, N + 1).
+static int shard_operators(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, const double* pi, double* d_out,
+                           cudaStream_t st)
+{
+    const int N = b->N, K = b->K;
+    const int n = b->w.n_total;
+    std::vector<int> pairs, lev_n;
+    std::vector<long long> lev_off;
+    // level L pairs every chain at offset 2^(L+1) m from its run's first chain with the one 2^L after it (if still in the run)
+    for (int s = 1;; s *= 2) {
+        const size_t before = pairs.size();
+        for (int k = 0; k < K; ++k) {
+            const int cf = b->plan.first_chain[k], cl = b->plan.last_chain[k];
+            if (cf < 0) continue;
+            for (int c = cf; c + s <= cl; c += 2 * s) { pairs.push_back(c); pairs.push_back(c + s); }
+        }
+        if (pairs.size() == before) break;
+        lev_off.push_back((long long)before / 2);
+        lev_n.push_back((int)((pairs.size() - before) / 2));
+    }
+    std::vector<int> first(b->plan.first_chain.begin(), b->plan.first_chain.end());
+    const size_t ops_bytes = (exact_scan_bytes(std::max(n, 1), N) + 255) & ~(size_t)255;
+    const size_t pair_bytes = ((sizeof(int) * std::max<size_t>(pairs.size(), 2)) + 255) & ~(size_t)255;
+    if (b->scan.ensure(ops_bytes + pair_bytes + sizeof(int) * K) != BHMM_OK) {
+        bhmm_set_error(BHMM_ERR_NO_MEM, "shard operators: device memory for the chain operators");
+        return BHMM_ERR_NO_MEM;
+    }
+    double* ops = reinterpret_cast<double*>(b->scan.base);
+    int* d_pairs = reinterpret_cast<int*>(b->scan.base + ops_bytes);
+    int* d_first = reinterpret_cast<int*>(b->scan.base + ops_bytes + pair_bytes);
+    RC_TRY(upload_small(b->d_A, A, (size_t)N * N, st));
+    RC_TRY(upload_small(b->d_pi, pi, N, st));
+    if (!pairs.empty()) CUDA_TRY(cudaMemcpyAsync(d_pairs, pairs.data(), sizeof(int) * pairs.size(), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_first, first.data(), sizeof(int) * K, cudaMemcpyHostToDevice, st));
+    const long long kstride = 2LL * N * (N + 1);
+    for (int d = 0; d < 2; ++d) {
+        RC_TRY(launch_shard_operators(b->w.ch, n, em, emkind, b->d_A, N, d == 0 ? +1 : -1, d_pairs, lev_n, lev_off, d_first,
+                                      K, ops, d_out + (size_t)d * N * (N + 1), kstride, st));
+        LAUNCHED((n > 0 ? 1 + lev_n.size() : 0) + 1);
+    }
+    return finish_stream(st);                 // (the host tables above are in use until the copies have run)
+}
+
+static int shard_operators_check(bhmm_b200_batch* b, double* d_out)
+{
+    if (!b || !d_out) { bhmm_set_error(BHMM_ERR_INVALID, "shard operators: null batch or output"); return BHMM_ERR_INVALID; }
+    if (b->own_lo.empty()) { bhmm_set_error(BHMM_ERR_INVALID, "shard operators are for time shards (batches with owned ranges)"); return BHMM_ERR_INVALID; }
+    if (!exact_scan_ok(b->N)) { bhmm_set_error(BHMM_ERR_UNSUPPORTED, "shard operators support N <= 128"); return BHMM_ERR_UNSUPPORTED; }
+    return BHMM_OK;
+}
+
+extern "C" int bhmm_b200_shard_operators_gaussian(bhmm_b200_batch* b, const double* d_obs, const double* A, const double* pi,
+                                                  const double* means, const double* sigmas, int ignore_outliers,
+                                                  double* d_out, void* stream)
+{
+    bhmm_set_error(BHMM_OK, "");
+    RC_TRY(shard_operators_check(b, d_out));
+    if (!d_obs || !A || !pi || !means || !sigmas) { bhmm_set_error(BHMM_ERR_INVALID, "shard operators: null argument"); return BHMM_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    RC_TRY(batch_carve(b, st));
+    RC_TRY(upload_small(b->d_mu, means, b->N, st));
+    RC_TRY(upload_small(b->d_sigma, sigmas, b->N, st));
+    Emission em{};
+    em.obs = d_obs; em.mu = b->d_mu; em.sigma = b->d_sigma; em.ignore_outliers = ignore_outliers;
+    return shard_operators(b, em, EM_GAUSS, A, pi, d_out, st);
+}
+
+extern "C" int bhmm_b200_shard_operators_discrete(bhmm_b200_batch* b, const int* d_obs, const double* A, const double* pi,
+                                                  const double* B, int M, int ignore_outliers, double* d_out, void* stream)
+{
+    bhmm_set_error(BHMM_OK, "");
+    RC_TRY(shard_operators_check(b, d_out));
+    if (!d_obs || !A || !pi || !B || M < 1) { bhmm_set_error(BHMM_ERR_INVALID, "shard operators: null argument or M < 1"); return BHMM_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    RC_TRY(batch_carve(b, st));
+    Emission em{};
+    em.sym = d_obs; em.ignore_outliers = ignore_outliers;
+    RC_TRY(prepare_discrete(b, B, M, em, st));
+    return shard_operators(b, em, EM_DISC, A, pi, d_out, st);
 }
 
 static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, const double* pi,

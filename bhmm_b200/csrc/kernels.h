@@ -1,5 +1,7 @@
 // bhmm_b200/csrc/kernels.h -- internal launch interface between the C ABI (capi.cu) and the kernels.
 #pragma once
+#include <vector>
+
 #include "common.cuh"
 
 struct FwdArgs {
@@ -137,6 +139,12 @@ bool exact_scan_ok(int N);
 size_t exact_scan_bytes(int n_chains, int N);
 int launch_exact_scan(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
                       double* he, double* ops, cudaStream_t st);
+// operators of the owned frames of every trajectory of a time shard: the chains' operators reduced level by level (lev_n[L]
+// (dst, src) chain pairs at d_pairs + 2 lev_off[L]) to the chain d_first[k]; out row i of trajectory k (stride kstride
+// doubles) = [operator row i | log-scale i], the identity where d_first[k] < 0.  ops: exact_scan_bytes(n_total, N).
+int launch_shard_operators(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
+                           const int* d_pairs, const std::vector<int>& lev_n, const std::vector<long long>& lev_off,
+                           const int* d_first, int K, double* ops, double* out, long long kstride, cudaStream_t st);
 bool lane_viterbi_ok(int N);                 // N <= 16: the chunked Viterbi runs one thread per chain (lane_viterbi.cu)
 int launch_viterbi_chain_lane(const VitChainArgs& a, int em, cudaStream_t st);
 bool panel_viterbi_chain_ok(int N);          // N <= 32: time-chunked Viterbi for trajectories cut into chains

@@ -423,7 +423,7 @@ k_forward_lane(const __grid_constant__ LaneParams<N> Pk, const LaneArgs a)
         t0 = a.ch.t0[c];
         trow = a.ch.row0[c] - t0;
         if (t0 == 0) { tstart = 0; mode = 0; }
-        else if (a.ch.exact) { tstart = t0 - 1; mode = 2; }
+        else if (chain_exact_start(a.ch, c)) { tstart = t0 - 1; mode = 2; }
         else { tstart = max(0, t0 - (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm)); mode = (tstart == 0) ? 0 : 1; }
     }
     const int maxpre = __reduce_max_sync(FULL, have ? (t0 - tstart) : 0);
@@ -434,8 +434,9 @@ k_forward_lane(const __grid_constant__ LaneParams<N> Pk, const LaneArgs a)
 #pragma unroll
     for (int j = 0; j < N; ++j) al[j] = 0.0;
     if (have && mode == 2) {
+        const double* hv = chain_start_vec(a.ch, a.hand_end, c, c - 1, N);
 #pragma unroll
-        for (int j = 0; j < N; ++j) al[j] = a.hand_end[(long long)(c - 1) * N + j];
+        for (int j = 0; j < N; ++j) al[j] = hv[j];
     }
     long long esum = 0;             // sum of the power-of-two shifts applied to the chain's own frames
     double slow = 0.0, log_start = 0.0, log_end = 0.0;
@@ -630,7 +631,7 @@ k_backward_stats_lane(const __grid_constant__ LaneParams<N> Pk, const LaneArgs a
         trow = a.ch.row0[c] - t0;
         e = t0 + len;
         if (e >= T) fs = T - 1;
-        else if (a.ch.exact) { fs = e; mode = 2; }
+        else if (chain_exact_start(a.ch, c)) { fs = e; mode = 2; }
         else fs = min(T - 1, e + (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm) - 1);
     }
     const int maxpre = __reduce_max_sync(FULL, have ? (fs - (e - 1)) : 0);
@@ -794,8 +795,9 @@ k_backward_stats_lane(const __grid_constant__ LaneParams<N> Pk, const LaneArgs a
             double b[N];
             if (init) {
                 if (mode == 2) {
+                    const double* hv = chain_start_vec(a.ch, a.hand_end, c, c + 1, N);
 #pragma unroll
-                    for (int j = 0; j < N; ++j) b[j] = a.hand_end[(long long)(c + 1) * N + j];
+                    for (int j = 0; j < N; ++j) b[j] = hv[j];
                 } else {
 #pragma unroll
                     for (int j = 0; j < N; ++j) b[j] = 1.0;

@@ -282,7 +282,7 @@ __global__ void __launch_bounds__(PW * 32) k_forward_panel32(const FwdArgs a)
             t0 = a.ch.t0[c];
             trow = a.ch.row0[c] - t0;
             if (t0 == 0) { tstart = 0; mode = 0; }
-            else if (a.ch.exact) { tstart = t0 - 1; mode = 2; }
+            else if (chain_exact_start(a.ch, c)) { tstart = t0 - 1; mode = 2; }
             else { tstart = max(0, t0 - (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm)); mode = (tstart == 0) ? 0 : 1; }
         }
         const int npre = have ? (t0 - tstart) : 0;
@@ -293,7 +293,7 @@ __global__ void __launch_bounds__(PW * 32) k_forward_panel32(const FwdArgs a)
         double av[8];                                      // normalised alpha of the previous frame, the lane's states
 #pragma unroll
         for (int k = 0; k < 8; ++k) av[k] = 0.0;
-        if (have && mode == 2) load8(a.hand_end + (long long)(c - 1) * PN, q, av);
+        if (have && mode == 2) load8(chain_start_vec(a.ch, a.hand_end, c, c - 1, PN), q, av);
         LogAcc acc;
 
         auto fetch = [&](int s, Raw<EM>& r) {
@@ -421,7 +421,7 @@ __global__ void __launch_bounds__(PW * 32) k_backward_stats_panel32(const BwdArg
             trow = a.ch.row0[c] - t0;
             e = t0 + len;
             if (e >= T) { virt = true; fstart = T; }
-            else if (a.ch.exact) { fstart = e; mode = 2; }
+            else if (chain_exact_start(a.ch, c)) { fstart = e; mode = 2; }
             else { fstart = min(T - 1, e + (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm) - 1); }
         }
         const int flast = t0 + 1;                           // step f emits frame f-1
@@ -432,7 +432,7 @@ __global__ void __launch_bounds__(PW * 32) k_backward_stats_panel32(const BwdArg
         double bn[8];
 #pragma unroll
         for (int k = 0; k < 8; ++k) bn[k] = 1.0 / PN;      // beta_{T-1} = 1/N (_hidden.c:76-77), also the warm-up start
-        if (have && mode == 2) load8(a.hand_end + (long long)(c + 1) * PN, q, bn);
+        if (have && mode == 2) load8(chain_start_vec(a.ch, a.hand_end, c, c + 1, PN), q, bn);
 
         auto frame_of = [&](int s) -> int { return (e - 1) + maxpre - s; };
         auto fetch = [&](int s, Raw<EM>& r) {
@@ -681,7 +681,7 @@ __global__ void WIDE_KERNEL_ATTR(NT) k_forward_wide(const FwdArgs a)
             t0 = a.ch.t0[c];
             trow = a.ch.row0[c] - t0;
             if (t0 == 0) { tstart = 0; mode = 0; }
-            else if (a.ch.exact) { tstart = t0 - 1; mode = 2; }
+            else if (chain_exact_start(a.ch, c)) { tstart = t0 - 1; mode = 2; }
             else { tstart = max(0, t0 - (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm)); mode = (tstart == 0) ? 0 : 1; }
         }
         const int npre = have ? (t0 - tstart) : 0;
@@ -694,8 +694,9 @@ __global__ void WIDE_KERNEL_ATTR(NT) k_forward_wide(const FwdArgs a)
 
         double vec[2] = {0.0, 0.0};
         if (have && mode == 2) {
-            if (ok0) vec[0] = a.hand_end[(long long)(c - 1) * N + s0];
-            if (ok1) vec[1] = a.hand_end[(long long)(c - 1) * N + s0 + 1];
+            const double* hv = chain_start_vec(a.ch, a.hand_end, c, c - 1, N);
+            if (ok0) vec[0] = hv[s0];
+            if (ok1) vec[1] = hv[s0 + 1];
         }
         double v[2] = {0.0, 0.0}, dd[2] = {0.0, 0.0};       // the lane's values of the frame in flight: with densities / with ones
         LogAcc acc;
@@ -875,7 +876,7 @@ __global__ void WIDE_KERNEL_ATTR(NT) k_backward_stats_wide(const BwdArgs a)
             trow = a.ch.row0[c] - t0;
             e = t0 + len;
             if (e >= T) { virt = true; fstart = T; }
-            else if (a.ch.exact) { fstart = e; mode = 2; }
+            else if (chain_exact_start(a.ch, c)) { fstart = e; mode = 2; }
             else { fstart = min(T - 1, e + (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm) - 1); }
         }
         const int flast = t0 + 1;
@@ -888,8 +889,9 @@ __global__ void WIDE_KERNEL_ATTR(NT) k_backward_stats_wide(const BwdArgs a)
 
         double bn[2] = {ok0 ? 1.0 / N : 0.0, ok1 ? 1.0 / N : 0.0};   // beta_{T-1} = 1/N (_hidden.c:76-77); warm-up start
         if (have && mode == 2) {
-            if (ok0) bn[0] = a.hand_end[(long long)(c + 1) * N + s0];
-            if (ok1) bn[1] = a.hand_end[(long long)(c + 1) * N + s0 + 1];
+            const double* hv = chain_start_vec(a.ch, a.hand_end, c, c + 1, N);
+            if (ok0) bn[0] = hv[s0];
+            if (ok1) bn[1] = hv[s0 + 1];
         }
         auto frame_of = [&](int s) -> int { return (e - 1) + maxpre - s; };
         auto em_row = [&](int s) -> long long { return trow + min(max(frame_of(s), t0), T - 1); };
@@ -1119,7 +1121,7 @@ __global__ void WIDE_KERNEL_ATTR(NT) k_forward_wide2(const FwdArgs a)
                 t0[z] = a.ch.t0[c[z]];
                 trow[z] = a.ch.row0[c[z]] - t0[z];
                 if (t0[z] == 0) { tstart[z] = 0; mode[z] = 0; }
-                else if (a.ch.exact) { tstart[z] = t0[z] - 1; mode[z] = 2; }
+                else if (chain_exact_start(a.ch, c[z])) { tstart[z] = t0[z] - 1; mode[z] = 2; }
                 else { tstart[z] = max(0, t0[z] - (a.ch.warmv ? a.ch.warmv[c[z]] : a.ch.warm)); mode[z] = (tstart[z] == 0) ? 0 : 1; }
             }
             tend[z] = t0[z] + len;
@@ -1143,8 +1145,9 @@ __global__ void WIDE_KERNEL_ATTR(NT) k_forward_wide2(const FwdArgs a)
             vec[z][0] = vec[z][1] = v[z][0] = v[z][1] = dd[z][0] = dd[z][1] = 0.0;
             o_next[z] = 0.0; pn[z][0] = pn[z][1] = 0.0; symA[z] = 0;
             if (have[z] && mode[z] == 2) {
-                if (ok0) vec[z][0] = a.hand_end[(long long)(c[z] - 1) * N + s0];
-                if (ok1) vec[z][1] = a.hand_end[(long long)(c[z] - 1) * N + s0 + 1];
+                const double* hv = chain_start_vec(a.ch, a.hand_end, c[z], c[z] - 1, N);
+                if (ok0) vec[z][0] = hv[s0];
+                if (ok1) vec[z][1] = hv[s0 + 1];
             }
             if (have[z]) {
                 if (EM == EM_GAUSS) o_next[z] = a.em.obs[frame_row(z, 0)];
@@ -1352,7 +1355,7 @@ __global__ void WIDE_KERNEL_ATTR(NT) k_backward_stats_wide2(const BwdArgs a)
                 trow[z] = a.ch.row0[c[z]] - t0[z];
                 e[z] = t0[z] + len;
                 if (e[z] >= T[z]) { virt[z] = true; fstart[z] = T[z]; }
-                else if (a.ch.exact) { fstart[z] = e[z]; mode[z] = 2; }
+                else if (chain_exact_start(a.ch, c[z])) { fstart[z] = e[z]; mode[z] = 2; }
                 else { fstart[z] = min(T[z] - 1, e[z] + (a.ch.warmv ? a.ch.warmv[c[z]] : a.ch.warm) - 1); }
             }
             maxpre[z] = __reduce_max_sync(FULL, have[z] ? (fstart[z] - (e[z] - 1)) : 0);
@@ -1373,8 +1376,9 @@ __global__ void WIDE_KERNEL_ATTR(NT) k_backward_stats_wide2(const BwdArgs a)
             bn[z][1] = ok1 ? 1.0 / N : 0.0;
             o_next[z] = 0.0; al_next[z][0] = al_next[z][1] = 0.0; pn[z][0] = pn[z][1] = 0.0; symA[z] = 0;
             if (have[z] && mode[z] == 2) {
-                if (ok0) bn[z][0] = a.hand_end[(long long)(c[z] + 1) * N + s0];
-                if (ok1) bn[z][1] = a.hand_end[(long long)(c[z] + 1) * N + s0 + 1];
+                const double* hv = chain_start_vec(a.ch, a.hand_end, c[z], c[z] + 1, N);
+                if (ok0) bn[z][0] = hv[s0];
+                if (ok1) bn[z][1] = hv[s0 + 1];
             }
             if (have[z]) {
                 if (EM == EM_GAUSS) o_next[z] = a.em.obs[em_row(z, 0)];

@@ -307,7 +307,141 @@ int launch_exact_scan_wide(const Chains& ch, int n_total, const Emission& em, in
     return BHMM_OK;
 }
 
+// ---- operators of a whole shard (time-sharded trajectories) --------------------------------------------------------
+// One block per pair of one level of a tree reduction: X <- X . Y with X = operator of chain pairs[2b], Y = operator of chain
+// pairs[2b + 1] (the chain right after X's range in time), both in the representation k_chain_operator writes (row i of the
+// true operator = exp(L_i) m_i, m_i summing to one).  Warp w takes the rows i = w, w + 32, ...; component k of a row lives in
+// lane k & 31, slot k >> 5 (NT = 1: lane per column, N <= 32).  A warp reads row i of X and writes it back itself, so the
+// product is formed in place; Y is read through the cache.  Plain FP64 FMAs: this serves the fallback, not the fast path.
+template <int NT>
+__global__ void __launch_bounds__(1024) k_compose_operators(const int* __restrict__ pairs, int N, double* ops, double* lscale)
+{
+    const int dst = pairs[2 * blockIdx.x], src = pairs[2 * blockIdx.x + 1];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const double* Y = ops + (long long)src * N * N;
+    double* X = ops + (long long)dst * N * N;
+    bool jv[NT];
+    double ly[NT];
+#pragma unroll
+    for (int q = 0; q < NT; ++q) {
+        jv[q] = lane + 32 * q < N;
+        ly[q] = jv[q] ? lscale[(long long)src * N + lane + 32 * q] : -INFINITY;
+    }
+    for (int i = w; i < N; i += 32) {
+        double x[NT];
+        double Lmax = -INFINITY;
+#pragma unroll
+        for (int q = 0; q < NT; ++q) {
+            x[q] = jv[q] ? X[(long long)i * N + lane + 32 * q] : 0.0;
+            if (x[q] > 0.0) Lmax = fmax(Lmax, ly[q]);
+        }
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) Lmax = fmax(Lmax, __shfl_xor_sync(FULLM, Lmax, off));
+        // weights of Y's rows: x_ik exp(L_k - max L)
+#pragma unroll
+        for (int q = 0; q < NT; ++q) x[q] = (x[q] > 0.0 && ly[q] > -INFINITY) ? x[q] * exp(ly[q] - Lmax) : 0.0;
+        double r[NT];
+#pragma unroll
+        for (int q = 0; q < NT; ++q) r[q] = 0.0;
+        for (int k = 0; k < N; ++k) {
+            double s = x[0];
+#pragma unroll
+            for (int q = 1; q < NT; ++q) s = ((k >> 5) == q) ? x[q] : s;      // k is uniform over the warp
+            const double wk = __shfl_sync(FULLM, s, k & 31);
+            const double* Yk = Y + (long long)k * N + lane;
+#pragma unroll
+            for (int q = 0; q < NT; ++q)
+                if (jv[q]) r[q] = fma(wk, Yk[32 * q], r[q]);
+        }
+        double tot = 0.0;
+#pragma unroll
+        for (int q = 0; q < NT; ++q) tot += r[q];
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) tot += __shfl_xor_sync(FULLM, tot, off);
+        const double Lx = lscale[(long long)dst * N + i];
+        const bool live = tot > 0.0 && Lx > -INFINITY;
+#pragma unroll
+        for (int q = 0; q < NT; ++q)
+            if (jv[q]) X[(long long)i * N + lane + 32 * q] = live ? r[q] / tot : 0.0;
+        if (lane == 0) lscale[(long long)dst * N + i] = live ? Lx + Lmax + log(tot) : -INFINITY;
+    }
+}
+
+// out (K, N, N + 1) for one direction: row i = [operator row i | log-scale i] of the chain first[k], the identity with zero
+// log-scales where the shard owns no frame of trajectory k (first[k] < 0).
+__global__ void k_operator_out(const int* __restrict__ first, int N, const double* __restrict__ ops,
+                               const double* __restrict__ lscale, double* __restrict__ out, long long kstride)
+{
+    const int k = blockIdx.x, c = first[k];
+    double* o = out + (long long)k * kstride;
+    for (int e = threadIdx.x; e < N * (N + 1); e += blockDim.x) {
+        const int i = e / (N + 1), j = e - i * (N + 1);
+        double v;
+        if (c < 0) v = (j == N) ? 0.0 : (i == j ? 1.0 : 0.0);
+        else v = (j == N) ? lscale[(long long)c * N + i] : ops[((long long)c * N + i) * N + j];
+        o[e] = v;
+    }
+}
+
+template <int NT>
+void launch_chain_operator_wide(const Chains& ch, int n_total, const Emission& em, int emkind, const double* dA, int N,
+                                int dir, double* ops, double* lscale, cudaStream_t st)
+{
+    switch (emkind) {
+        case EM_POBS: k_chain_operator_wide<EM_POBS, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        case EM_GAUSS: k_chain_operator_wide<EM_GAUSS, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        default: k_chain_operator_wide<EM_DISC, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+    }
+}
+
+template <int NT>
+void launch_compose_level(const int* pairs, int n, int N, double* ops, double* lscale, cudaStream_t st)
+{
+    k_compose_operators<NT><<<n, 32 * std::min(N, 32), 0, st>>>(pairs, N, ops, lscale);
+}
+
 }  // namespace
+
+// Operators of the owned frames of every trajectory of a time shard (bhmm_b200_shard_operators_*): the chains' operators,
+// then level after level of the reduction (lev_n[L] pairs at d_pairs + 2 lev_off[L]), then one (N, N + 1) block per
+// trajectory written to out (trajectory stride kstride doubles).
+int launch_shard_operators(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
+                           const int* d_pairs, const std::vector<int>& lev_n, const std::vector<long long>& lev_off,
+                           const int* d_first, int K, double* ops, double* out, long long kstride, cudaStream_t st)
+{
+    if (!exact_scan_ok(N)) return BHMM_ERR_UNSUPPORTED;
+    if (emkind != EM_POBS && emkind != EM_GAUSS && emkind != EM_DISC) return BHMM_ERR_INVALID;
+    double* lscale = ops + (size_t)n_total * N * N;
+    if (n_total > 0) {
+        Chains ch = all;
+        ch.list = nullptr; ch.n = n_total;
+        if (N > 32) {
+            switch ((N + 31) / 32) {
+                case 2: launch_chain_operator_wide<2>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
+                case 3: launch_chain_operator_wide<3>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
+                default: launch_chain_operator_wide<4>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
+            }
+        } else {
+            const size_t smem = sizeof(double) * (size_t)N * N;
+            switch (emkind) {
+                case EM_POBS: k_chain_operator<EM_POBS><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+                case EM_GAUSS: k_chain_operator<EM_GAUSS><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+                default: k_chain_operator<EM_DISC><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+            }
+        }
+        for (size_t L = 0; L < lev_n.size(); ++L) {
+            const int* pairs = d_pairs + 2 * lev_off[L];
+            switch ((N + 31) / 32) {
+                case 1: launch_compose_level<1>(pairs, lev_n[L], N, ops, lscale, st); break;
+                case 2: launch_compose_level<2>(pairs, lev_n[L], N, ops, lscale, st); break;
+                case 3: launch_compose_level<3>(pairs, lev_n[L], N, ops, lscale, st); break;
+                default: launch_compose_level<4>(pairs, lev_n[L], N, ops, lscale, st); break;
+            }
+        }
+    }
+    k_operator_out<<<K, 256, 0, st>>>(d_first, N, ops, lscale, out, kstride);
+    return BHMM_OK;
+}
 
 bool exact_scan_ok(int N) { return N >= 1 && N <= 128; }
 

@@ -186,7 +186,7 @@ __global__ void k_forward_team(const FwdArgs a)
             t0 = a.ch.t0[c];
             trow = a.ch.row0[c] - t0;
             if (t0 == 0) { tstart = 0; mode = 0; }
-            else if (a.ch.exact) { tstart = t0 - 1; mode = 2; }
+            else if (chain_exact_start(a.ch, c)) { tstart = t0 - 1; mode = 2; }
             else { tstart = max(0, t0 - (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm)); mode = (tstart == 0) ? 0 : 1; }
         }
         const int npre = have ? (t0 - tstart) : 0;
@@ -196,7 +196,7 @@ __global__ void k_forward_team(const FwdArgs a)
 
         double ll = 0.0, cprev = 1.0;
         double vec_j = 0.0;
-        if (have && mode == 2 && jv) vec_j = a.hand_end[(long long)(c - 1) * N + j];
+        if (have && mode == 2 && jv) vec_j = chain_start_vec(a.ch, a.hand_end, c, c - 1, N)[j];
 
         // depth-1 software prefetch of the emission input
         auto fetch = [&](int s) -> double {
@@ -317,7 +317,7 @@ __global__ void k_backward_team(const BwdArgs a)
             trow = a.ch.row0[c] - t0;
             e = t0 + len;
             if (e >= T) { virt = true; fstart = STATS ? T : T - 1; }
-            else if (a.ch.exact) { fstart = e; mode = 2; }
+            else if (chain_exact_start(a.ch, c)) { fstart = e; mode = 2; }
             else { fstart = min(T - 1, e + (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm) - 1); }
         }
         // literal backward emits frame f at step f; STATS emits frame f-1 at step f.
@@ -327,7 +327,7 @@ __global__ void k_backward_team(const BwdArgs a)
         const int total = maxpre + block_max(have ? (e - flast) : 0);
 
         double b_own = 0.0;
-        if (have && jv) b_own = (mode == 2) ? a.hand_end[(long long)(c + 1) * N + j] : 1.0;
+        if (have && jv) b_own = (mode == 2) ? chain_start_vec(a.ch, a.hand_end, c, c + 1, N)[j] : 1.0;
 
         auto frame_of = [&](int s) -> int { return (e - 1) + maxpre - s; };
         auto fetch_em = [&](int s) -> double {

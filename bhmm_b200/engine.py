@@ -815,9 +815,9 @@ def generate_trajectories(A, pi, lengths, seed, means=None, sigmas=None, B=None,
         return obs, states, torch.as_tensor(offsets, device=dev)
 
 
-def _rel_mismatch(a, b):
+def _rel_mismatch(a, b, floor=0.0):
     """Largest component-wise relative difference of two hand-over vectors; NaN counts as a full mismatch
-    (csrc/common.cuh:rel_mismatch)."""
+    (csrc/common.cuh:rel_mismatch).  Components below ``floor`` in both vectors are not compared."""
     a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
     if a.size == 0:
         return 0.0
@@ -825,7 +825,7 @@ def _rel_mismatch(a, b):
         return 1.0
     m = np.maximum(np.abs(a), np.abs(b))
     d = np.zeros_like(m)
-    nz = m > 0
+    nz = m > floor
     d[nz] = np.abs(a - b)[nz] / m[nz]
     return float(d.max())
 
@@ -849,6 +849,57 @@ def compose_shard_maps(maps_by_rank, owns_by_rank):
     return enter
 
 
+def _apply_operator(v, op, forward):
+    """One shard's operator on a border vector (a host function): ``op`` (N, N + 1) = [row-normalised operator | log-scale of
+    every row] as bhmm_b200_shard_operators_* write it.  forward: the row vector v . M, backward: the column vector M . v.
+    The log-scales only weigh the rows against each other; the result is normalised to sum one."""
+    M, L = op[:, :-1], op[:, -1]
+    if forward:
+        live = (v > 0) & np.isfinite(L)
+        if not live.any():
+            raise RuntimeError('time-sharded E-step: the exact border vector vanished (the model gives the data zero probability)')
+        w = np.where(live, v * np.exp(np.where(live, L - L[live].max(), -np.inf)), 0.0)
+        x = w @ M
+    else:
+        x = M @ v
+        live = (x > 0) & np.isfinite(L)
+        if not live.any():
+            raise RuntimeError('time-sharded E-step: the exact border vector vanished (the model gives the data zero probability)')
+        x = np.where(live, x * np.exp(np.where(live, L - L[live].max(), -np.inf)), 0.0)
+    return x / x.sum()
+
+
+def compose_shard_operators(ops_by_rank, borders_by_rank, owns_by_rank):
+    """Exact border vectors of an E-step on time shards, from all shards' operators (a host function; no device).
+
+    ``ops_by_rank[r]``: (K, 2, N, N + 1), shard r's forward and backward operators of its owned frames
+    (``TimeShardedTrajectories.shard_operators``); ``borders_by_rank[r]``: (K, 4, N), its border vectors
+    (``bhmm_b200_batch_border_handovers``); ``owns_by_rank[r][k]``: whether shard r owns frames of trajectory k.  Forward: the
+    first owner's alpha at its last owned frame ([1], exact: that shard holds the trajectory's start) is carried left to right
+    through the operators of the following owners; backward: the last owner's beta at its first owned frame ([3]) right to
+    left.  Shards that own nothing of a trajectory pass the vector through.  Returns (fwd, bwd), each (world, K, N): the exact
+    alpha at lo - 1 and beta at hi of every shard, normalised to sum one; zero rows where a shard owns nothing of the
+    trajectory, holds its start (fwd) or holds its end (bwd)."""
+    world = len(ops_by_rank)
+    K, _, N, _ = np.shape(ops_by_rank[0])
+    fwd, bwd = np.zeros((world, K, N)), np.zeros((world, K, N))
+    for k in range(K):
+        owners = [r for r in range(world) if owns_by_rank[r][k]]
+        if not owners:
+            continue
+        v = np.asarray(borders_by_rank[owners[0]][k][1], dtype=np.float64)
+        v = v / v.sum()
+        for r in owners[1:]:
+            fwd[r, k] = v
+            v = _apply_operator(v, np.asarray(ops_by_rank[r][k][0], dtype=np.float64), True)
+        v = np.asarray(borders_by_rank[owners[-1]][k][3], dtype=np.float64)
+        v = v / v.sum()
+        for r in owners[-2::-1]:
+            bwd[r, k] = v
+            v = _apply_operator(v, np.asarray(ops_by_rank[r][k][1], dtype=np.float64), False)
+    return fwd, bwd
+
+
 class TimeShardedTrajectories(object):
     """E-step over trajectories that are cut in TIME across shards (SURVEY 8e, C5: one trajectory too long for one GPU).
 
@@ -862,6 +913,14 @@ class TimeShardedTrajectories(object):
 
     One process per shard (``torch.distributed``), or several shards in one process for tests (``combine``,
     ``viterbi_combine``).
+
+    ``estep`` (distributed) and ``estep_combine`` (all shards in one process) add an exact fallback for models whose filter
+    does not forget its start within the halo, which can happen in the middle of an EM run as the model changes.  When a
+    border fails the certification and N <= 128, every shard reduces its owned frames to a forward and a backward transfer
+    operator (``shard_operators``: N times the work of a forward pass), one ``all_gather`` exchanges them, every shard
+    composes its exact border vectors (``compose_shard_operators``), and the E-step runs once more from those starts
+    (``set_border_starts``) instead of the halo warm-up; its borders are certified again.  ``combine``, ``certify`` and
+    ``estep_gaussian`` keep raising on a halo that is too short.
 
     Viterbi works across shards as well (``viterbi_gaussian`` / ``viterbi_discrete``): every shard builds the back-pointer
     map of its owned frames with the chain-parallel Viterbi kernels, warming its max-product vector up on the halo BEFORE
@@ -1270,15 +1329,7 @@ class TimeShardedTrajectories(object):
     def certify(borders_by_rank, ranges_by_rank, tol):
         """Worst relative mismatch over all shard borders; raises when it exceeds ``tol``.
         borders_by_rank[r]: (K, 4, N); ranges_by_rank[r]: [(lo, hi, T)] per trajectory."""
-        world = len(borders_by_rank)
-        worst = 0.0
-        K = len(ranges_by_rank[0])
-        for k in range(K):
-            owners = [r for r in range(world) if ranges_by_rank[r][k][1] > ranges_by_rank[r][k][0]]
-            for left, right in zip(owners, owners[1:]):
-                fwd = _rel_mismatch(borders_by_rank[right][k][0], borders_by_rank[left][k][1])
-                bwd = _rel_mismatch(borders_by_rank[left][k][2], borders_by_rank[right][k][3])
-                worst = max(worst, fwd, bwd)
+        worst = TimeShardedTrajectories.border_mismatch(borders_by_rank, ranges_by_rank)
         if worst > tol:
             raise RuntimeError('time-sharded E-step: a shard border disagrees by %.3g (tolerance %.3g); the halo is too '
                                'short for this model -- increase halo=' % (worst, tol))
@@ -1292,6 +1343,220 @@ class TimeShardedTrajectories(object):
             stats = st.clone() if stats is None else stats.add_(st.to(stats.device))
         worst = cls.certify([b for _, b in local_results], [s.global_ranges for s in shards], shards[0].tol)
         return stats, worst
+
+    # ------------------------------------------------------------------------------------------ E-step with exact borders
+    # Exact border vectors are composed through operator products, the border vectors they are compared with by the vector
+    # recursion: the same numbers in a different order.  Components in the subnormal range (below 2.2e-308; 1e-300 leaves
+    # headroom for subnormal intermediates) carry too few significant bits for a relative comparison -- at 1e-318 the spacing
+    # of doubles is 1.6e-6 of the value -- so the certification after the fallback leaves them out.
+    EXACT_BORDER_FLOOR = 1e-300
+
+    @staticmethod
+    def border_mismatch(borders_by_rank, ranges_by_rank, floor=0.0):
+        """Worst relative mismatch over all shard borders (what ``certify`` compares with its tolerance), without raising;
+        components below ``floor`` in both vectors are not compared."""
+        world, worst = len(borders_by_rank), 0.0
+        for k in range(len(ranges_by_rank[0])):
+            owners = [r for r in range(world) if ranges_by_rank[r][k][1] > ranges_by_rank[r][k][0]]
+            for left, right in zip(owners, owners[1:]):
+                worst = max(worst, _rel_mismatch(borders_by_rank[right][k][0], borders_by_rank[left][k][1], floor),
+                            _rel_mismatch(borders_by_rank[left][k][2], borders_by_rank[right][k][3], floor))
+        return worst
+
+    @classmethod
+    def _certify_exact(cls, borders_by_rank, ranges_by_rank, tol):
+        """Certification of the E-step after the fallback; raises when a border still disagrees."""
+        worst = cls.border_mismatch(borders_by_rank, ranges_by_rank, cls.EXACT_BORDER_FLOOR)
+        if worst > tol:
+            raise RuntimeError('time-sharded E-step: a shard border disagrees by %.3g (tolerance %.3g) after the exact '
+                               'border exchange' % (worst, tol))
+        return worst
+
+    def _ranges(self, world=None):
+        """[(lo, hi, T)] of every trajectory for every shard of the job."""
+        world = self.world if world is None else world
+        return [[((T * r) // world, (T * (r + 1)) // world, T) for (_, _, T) in self.global_ranges] for r in range(world)]
+
+    def estep_local(self, model, kind='gaussian'):
+        """Local E-step.  ``model``: (A, pi, means, sigmas, ignore_outliers) or (A, pi, B, ignore_outliers).  Returns the
+        statistics (a device copy), the B numerators (discrete; else None) and the (K, 4, N) border vectors."""
+        if kind == 'gaussian':
+            A, pi, means, sigmas, io = model
+            stats, Bnum = self.batch.estep_gaussian(A, pi, means, sigmas, ignore_outliers=io), None
+        else:
+            A, pi, B, io = model
+            stats, Bnum = self.batch.estep_discrete(A, pi, B, ignore_outliers=io)
+            Bnum = Bnum.clone()
+        return stats.clone(), Bnum, np.array([self.batch.border_handovers(k) for k in range(self.K)])
+
+    def _missing_right_halo(self):
+        """The first trajectory that continues after this shard while its piece ends with the owned range (the backward
+        operator reads the frame after the range), or None."""
+        b = self.batch
+        for k, (lo, hi, T) in enumerate(self.global_ranges):
+            if lo < hi < T and b._own_ranges[k][1] >= int(b.lengths[k]):
+                return k
+        return None
+
+    def shard_operators(self, model, kind='gaussian'):
+        """Forward and backward transfer operators of this shard's owned frames: a (K, 2, N, N + 1) float64 device tensor,
+        row i = [operator row i normalised to sum one | log of its scale] (bhmm_b200_shard_operators_*).  N <= 128.  A
+        trajectory that continues after the shard needs at least one halo frame after the owned range (ValueError)."""
+        b = self.batch
+        k = self._missing_right_halo()
+        if k is not None:
+            raise ValueError('time-sharded E-step: trajectory %d continues after this shard, whose piece has no halo frame '
+                             'after its owned range (the backward operator needs one)' % k)
+        out = b.torch.empty((self.K, 2, self.N, self.N + 1), dtype=b.torch.float64, device=b.device)
+        with b.torch.cuda.device(b.device):
+            if kind == 'gaussian':
+                A, pi, means, sigmas, io = model
+                if b.discrete:
+                    raise TypeError('this batch holds integer symbols; a Gaussian output model needs float observations')
+                A_, pi_, m_, s_ = f64(A), f64(pi), f64(means), f64(sigmas)
+                rc = lib.bhmm_b200_shard_operators_gaussian(b._handle, C.c_void_p(b.obs.data_ptr()), dptr(A_), dptr(pi_),
+                                                            dptr(m_), dptr(s_), int(bool(io)), C.c_void_p(out.data_ptr()),
+                                                            b._stream())
+            else:
+                A, pi, B, io = model
+                A_, pi_, B_ = f64(A), f64(pi), f64(B)
+                b._require_discrete(B_.shape[1])
+                rc = lib.bhmm_b200_shard_operators_discrete(b._handle, C.c_void_p(b.obs.data_ptr()), dptr(A_), dptr(pi_),
+                                                            dptr(B_), B_.shape[1], int(bool(io)), C.c_void_p(out.data_ptr()),
+                                                            b._stream())
+        check(rc)
+        return out
+
+    def set_border_starts(self, fwd, bwd):
+        """Start the next E-steps from exact border vectors (rows of ``compose_shard_operators``' result for this shard): the
+        forward recursion of trajectory k at lo - 1 where this shard owns frames of it but not its start, the backward one at
+        hi where it owns frames but not its end.  ``clear_border_starts`` returns to the halo warm-up."""
+        for k, (lo, hi, T) in enumerate(self.global_ranges):
+            f = np.ascontiguousarray(fwd[k], dtype=np.float64) if 0 < lo < hi else None
+            g = np.ascontiguousarray(bwd[k], dtype=np.float64) if lo < hi < T else None
+            check(lib.bhmm_b200_batch_set_border_starts(self.batch._handle, k, dptr(f) if f is not None else None,
+                                                        dptr(g) if g is not None else None))
+
+    def clear_border_starts(self):
+        for k in range(self.K):
+            check(lib.bhmm_b200_batch_set_border_starts(self.batch._handle, k, None, None))
+
+    @classmethod
+    def _fallback_starts(cls, ops_by_rank, borders_by_rank, ranges_by_rank):
+        owns = [[g[1] > g[0] for g in ranges] for ranges in ranges_by_rank]
+        return compose_shard_operators(ops_by_rank, borders_by_rank, owns)
+
+    def _exact_borders_unsupported(self, worst):
+        return RuntimeError('time-sharded E-step: a shard border disagrees by %.3g (tolerance %.3g) and the exact fallback '
+                            'supports N <= 128 -- increase halo=' % (worst, self.tol))
+
+    @classmethod
+    def estep_combine(cls, shards, model, kind='gaussian'):
+        """Single-process use (tests): the E-step of ``estep`` with all shards in this process.  Returns (stats, Bnum or None,
+        report) with the summed statistics and ``report`` = {'worst': worst border mismatch of the pass whose statistics are
+        returned, 'fallback': whether the exact borders were needed}."""
+        ranges = [s.global_ranges for s in shards]
+        res = [s.estep_local(model, kind) for s in shards]
+        worst = cls.border_mismatch([r[2] for r in res], ranges)
+        fallback = worst > shards[0].tol
+        if fallback:
+            if shards[0].N > 128:
+                raise shards[0]._exact_borders_unsupported(worst)
+            ops = [s.shard_operators(model, kind).cpu().numpy() for s in shards]
+            fwd, bwd = cls._fallback_starts(ops, [r[2] for r in res], ranges)
+            try:
+                for r, s in enumerate(shards):
+                    s.set_border_starts(fwd[r], bwd[r])
+                res = [s.estep_local(model, kind) for s in shards]
+            finally:
+                for s in shards:
+                    s.clear_border_starts()
+            worst = cls._certify_exact([r[2] for r in res], ranges, shards[0].tol)
+        stats = Bnum = None
+        for st, bn, _ in res:
+            stats = st.clone() if stats is None else stats.add_(st.to(stats.device))
+            if bn is not None:
+                Bnum = bn.clone() if Bnum is None else Bnum.add_(bn.to(Bnum.device))
+        return stats, Bnum, {'worst': worst, 'fallback': bool(fallback)}
+
+    @staticmethod
+    def all_gather_host(array, world, device):
+        """Every shard's copy of a float64 host array: one all_gather through ``device`` (no collective at world 1)."""
+        if world == 1:
+            return [np.asarray(array, dtype=np.float64)]
+        import torch
+        import torch.distributed as td
+        if td.get_backend() != 'nccl':
+            device = 'cpu'                     # gloo and mpi groups gather host tensors
+        mine = torch.from_numpy(np.ascontiguousarray(array, dtype=np.float64)).to(device)
+        gathered = [torch.empty_like(mine) for _ in range(world)]
+        td.all_gather(gathered, mine)
+        return [g.cpu().numpy() for g in gathered]
+
+    @classmethod
+    def operator_exchange(cls, ops, borders_by_rank, lengths, rank, world, device):
+        """The exchange of the exact fallback: ONE all_gather of this shard's (K, 2, N, N + 1) operators, then the composition
+        of all shards' operators with the border vectors gathered before (``borders_by_rank``, (K, 4, N) per shard).
+        ``lengths``: the K trajectory lengths.  Returns this shard's exact (fwd, bwd) border vectors, (K, N) each."""
+        got = cls.all_gather_host(ops, world, device)
+        ranges = [[((T * r) // world, (T * (r + 1)) // world, T) for T in lengths] for r in range(world)]
+        fwd, bwd = cls._fallback_starts(got, borders_by_rank, ranges)
+        return fwd[rank], bwd[rank]
+
+    def _all_gather(self, array):
+        return self.all_gather_host(array, self.world, self.batch.device)
+
+    def estep(self, model, kind='gaussian'):
+        """Distributed E-step (one process per shard; torch.distributed initialised when world > 1): local E-step, one
+        all_gather of the border vectors and their certification; if a border fails and N <= 128, the shards' operators are
+        exchanged (one all_gather of K * 2 * N * (N + 1) doubles per shard), every shard composes its exact border vectors,
+        runs the E-step again from them and certifies again (a second failure raises); then the statistics are all-reduced.
+        ``model``: (A, pi, means, sigmas, ignore_outliers) or (A, pi, B, ignore_outliers).  Returns (stats, Bnum or None,
+        report) like ``estep_combine``, for the whole job."""
+        ranges = self._ranges()
+        stats, Bnum, borders = self.estep_local(model, kind)
+        # every rank learns with the border vectors whether each shard could take the fallback (a right halo frame wherever
+        # a trajectory continues), so that all ranks raise together instead of one rank leaving the others in a collective
+        K, N = self.K, self.N
+        no_halo = self._missing_right_halo()
+        pack = np.concatenate([np.asarray(borders, dtype=np.float64).reshape(-1), [-1.0 if no_halo is None else no_halo]])
+        got = self._all_gather(pack)
+        gathered = [g[:-1].reshape(K, 4, N) for g in got]
+        worst = self.border_mismatch(gathered, ranges)
+        fallback = worst > self.tol
+        if fallback:
+            if self.N > 128:
+                raise self._exact_borders_unsupported(worst)
+            lacking = [(r, int(g[-1])) for r, g in enumerate(got) if g[-1] >= 0]
+            if lacking:
+                raise ValueError('time-sharded E-step: a shard border disagrees by %.3g (tolerance %.3g), and the exact fallback '
+                                 'needs a halo frame after the owned range of every trajectory that continues; rank %d has none '
+                                 'for trajectory %d' % (worst, self.tol, lacking[0][0], lacking[0][1]))
+            fwd, bwd = self.operator_exchange(self.shard_operators(model, kind).cpu().numpy(), gathered,
+                                              [T for (_, _, T) in self.global_ranges], self.rank, self.world, self.batch.device)
+            try:
+                self.set_border_starts(fwd, bwd)
+                stats, Bnum, borders = self.estep_local(model, kind)
+            finally:
+                self.clear_border_starts()
+            worst = self._certify_exact(self._all_gather(borders), ranges, self.tol)
+        if self.world > 1:
+            stats = self._all_reduce(stats)
+            if Bnum is not None:
+                Bnum = self._all_reduce(Bnum)
+        return stats, Bnum, {'worst': worst, 'fallback': bool(fallback)}
+
+    @staticmethod
+    def _all_reduce(t):
+        """In-place sum over the ranks of a device tensor; through a host copy on groups that are not NCCL (gloo)."""
+        import torch.distributed as td
+        if td.get_backend() == 'nccl':
+            td.all_reduce(t, op=td.ReduceOp.SUM)
+            return t
+        h = t.cpu()
+        td.all_reduce(h, op=td.ReduceOp.SUM)
+        t.copy_(h)
+        return t
 
     def estep_gaussian(self, A, pi, means, sigmas, ignore_outliers=True):
         """Distributed use (one process per shard, torch.distributed initialised): all-reduced statistics and the worst

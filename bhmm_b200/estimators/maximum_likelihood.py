@@ -16,7 +16,7 @@ import time
 import numpy as np
 
 from .. import dist
-from ..engine import (TrajectoryBatch, make_batch, unpack_stats, mstep_device, mstep_discrete_device, unpack_mstep, download_array,
+from ..engine import (TrajectoryBatch, TimeShardedTrajectories, make_batch, unpack_stats, mstep_device, mstep_discrete_device, unpack_mstep, download_array,
                       HostBufferInBackground)
 from ..util import config
 from ..util.logger import logger
@@ -30,6 +30,14 @@ class MaximumLikelihoodEstimator(object):
     here: the reference's heuristics in bhmm/init need msmtools / a vendored GMM and are out of scope),
     ``reversible``, ``stationary``, ``p``, ``accuracy``, ``maxit``, ``maxit_P``.  Extra: ``chunk`` / ``warm`` (time
     chunking of the kernels, 0 = automatic) and ``shard`` (True: keep only this rank's share of the trajectories).
+
+    ``shard='time'`` cuts EVERY trajectory in time over the ranks instead (``engine.TimeShardedTrajectories``: one trajectory
+    too long for one GPU), and ``batch=`` may then be a ``TimeShardedTrajectories`` the caller built, e.g. with
+    ``from_local_piece`` (the trajectory lengths then come from its ``global_ranges``).  The E-step runs on the shards with
+    certified borders and, where a border does not certify, the exact operator exchange (``TimeShardedTrajectories.estep``);
+    ``border_fallbacks`` counts the iterations that needed it.  The M-step is unchanged.  ``fit()`` ends with Viterbi across
+    the shards, and ``hidden_state_trajectories`` holds this rank's owned pieces of the paths; where time-sharded Viterbi is
+    not available (N > 32) or its borders do not certify, they stay None and a warning is logged.
     """
 
     def __init__(self, observations, nstates, initial_model=None, output='gaussian', reversible=True, stationary=False,
@@ -41,18 +49,26 @@ class MaximumLikelihoodEstimator(object):
         self._stationary = stationary
         self._hmm = copy.deepcopy(initial_model)
         self._output = self._hmm.output_model.model_type
-        self._all_lengths = [len(o) for o in observations]
-        self._nobs_total = len(observations)
+        self._time_sharded = (isinstance(shard, str) and shard == 'time') or isinstance(batch, TimeShardedTrajectories)
+        if isinstance(batch, TimeShardedTrajectories):
+            self._all_lengths = [T for (_, _, T) in batch.global_ranges]
+            observations = observations if observations is not None else []
+        else:
+            self._all_lengths = [len(o) for o in observations]
+        self._nobs_total = len(self._all_lengths)
+        self.border_fallbacks = 0       # E-steps on time shards that needed the exact border exchange
         # trajectories of this rank
         dist.tune_for_world()
-        if shard and dist.world_size() > 1:
+        if self._time_sharded:
+            lo, hi = 0, len(observations)
+        elif shard and dist.world_size() > 1:
             lo, hi = dist.shard_bounds(self._all_lengths, dist.rank(), dist.world_size())
         else:
             lo, hi = 0, len(observations)
         self._shard = (lo, hi)
         self._observations = [np.asarray(o) for o in observations[lo:hi]]
         self._nobs = len(self._observations)
-        self._Ts = [len(o) for o in self._observations]
+        self._Ts = list(self._all_lengths) if self._time_sharded else [len(o) for o in self._observations]
         self._maxT = np.max(self._Ts) if self._Ts else 0
         self._fixed_stationary_distribution = None
         self._fixed_initial_distribution = None
@@ -66,7 +82,13 @@ class MaximumLikelihoodEstimator(object):
         self._maxit_P = maxit_P
         self._likelihoods = None
         # batch=: an engine batch that already holds these trajectories on the GPU (no second upload)
-        self._batch = batch if batch is not None else (make_batch(self._observations, nstates, chunk=chunk, warm=warm) if self._nobs else None)
+        if batch is not None:
+            self._batch = batch
+        elif self._time_sharded:
+            self._batch = TimeShardedTrajectories(self._observations, nstates, dist.rank(), dist.world_size(), chunk=chunk,
+                                                  warm=warm)
+        else:
+            self._batch = make_batch(self._observations, nstates, chunk=chunk, warm=warm) if self._nobs else None
         self._hmm.output_model.set_implementation(config.kernel)
         self.count_matrix = None
         self.initial_count = None
@@ -126,6 +148,14 @@ class MaximumLikelihoodEstimator(object):
         pi = self._hmm.initial_distribution
         om = self._hmm.output_model
         Bnum = None
+        if self._time_sharded:
+            # statistics of the owned frames, borders certified (or made exact) and all-reduced across the shards
+            stats, Bnum, report = self._batch.estep(self._model_tuple(), self._output)
+            self.border_fallbacks += int(report['fallback'])
+            self._dev = (stats, Bnum)
+            if self._device_mstep and self._device_mstep_applies():
+                return None
+            return self._host_stats()
         if self._batch is None:
             # a rank whose shard is empty (more ranks than trajectories) contributes zero statistics: the other ranks are
             # already waiting in the all-reduce, raising here would deadlock the job
@@ -145,6 +175,33 @@ class MaximumLikelihoodEstimator(object):
         if self._device_mstep and self._device_mstep_applies():
             return None                  # the statistics stay on the GPU: _update_model_device reads back parameters only
         return self._host_stats()
+
+    def _model_tuple(self):
+        A = self._hmm.transition_matrix
+        pi = self._hmm.initial_distribution
+        om = self._hmm.output_model
+        if self._output == 'gaussian':
+            return (A, pi, om.means, om.sigmas, om.ignore_outliers)
+        return (A, pi, om.output_probabilities, om.ignore_outliers)
+
+    def _time_sharded_viterbi(self):
+        """Viterbi across the time shards: this rank's owned pieces of the paths, or None (with a warning) where that is not
+        available -- N > 32, or a border or a decision that does not certify -- so that a finished fit is kept."""
+        if self._nstates > 32:
+            logger().warning('time-sharded Viterbi needs N <= 32; hidden_state_trajectories left at None')
+            return None
+        try:
+            if self._batch.world == 1:
+                paths, _ = TimeShardedTrajectories.viterbi_combine([self._batch], self._model_tuple(), self._output)
+            else:
+                paths, _ = self._batch.viterbi(self._model_tuple(), self._output)
+        except RuntimeError as e:
+            logger().warning('time-sharded Viterbi failed (%s); hidden_state_trajectories left at None' % e)
+            return None
+        out = np.empty(len(paths), dtype=object)
+        for k, p in enumerate(paths):
+            out[k] = p
+        return out
 
     def _host_stats(self):
         stats, Bnum = self._dev
@@ -209,6 +266,8 @@ class MaximumLikelihoodEstimator(object):
         om = self._hmm.output_model
         if self._batch is None:
             return np.empty(0, dtype=object)
+        if self._time_sharded:
+            return self._time_sharded_viterbi()
         if self._output == 'gaussian':
             path = self._batch.viterbi_gaussian(A, pi, om.means, om.sigmas, ignore_outliers=om.ignore_outliers)
         else:
@@ -232,7 +291,8 @@ class MaximumLikelihoodEstimator(object):
         converged = False
         st = None
         # the array that will hold the Viterbi paths: its pages are faulted in by a helper thread while the GPU iterates
-        self._path_host = HostBufferInBackground((int(self._batch.rows),), np.int32) if self._batch is not None else None
+        self._path_host = (HostBufferInBackground((int(self._batch.rows),), np.int32)
+                           if self._batch is not None and not self._time_sharded else None)
         while not converged and it < self.maxit:
             t1 = time.time()
             st = self._estep()

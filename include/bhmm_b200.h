@@ -142,6 +142,30 @@ int bhmm_b200_batch_create(bhmm_b200_batch** out, const long long* offsets, int 
 int bhmm_b200_batch_create_ranges(bhmm_b200_batch** out, const long long* offsets, const long long* own_lo,
                                   const long long* own_hi, int K, int N, int chunk, int warm);
 int bhmm_b200_batch_border_handovers(const bhmm_b200_batch* b, int k, double* out);
+/* Exact shard borders, for models whose filter does not forget its start within the halo (the border vectors then disagree).
+ * The recursions are linear maps, so a shard's owned frames of trajectory k reduce to two N x N operators:
+ *   forward  F_k = prod_{t = own_lo}^{own_hi - 1} (A D_t):  alpha_{own_hi - 1} ~ alpha_{own_lo - 1} . F_k
+ *   backward B_k = prod_{f = own_lo + 1}^{own_hi} (A D_f):  beta_{own_lo}     ~ B_k . beta_{own_hi}
+ * with D_t = diag(p(o_t | state)).  bhmm_b200_shard_operators_* write them to d_out, device (K, 2, N, N + 1) doubles: row i of
+ * [0] = [row i of F_k, normalised to sum one | log of its scale], [1] the same for B_k; the identity with zero log-scales where
+ * the shard owns no frame of trajectory k.  B_k reads frame own_hi, so a trajectory that continues after the owned range
+ * needs at least one halo frame after it; an owned range that ends with the local trajectory is taken to end the trajectory
+ * (its backward operator is not used).  N > 128 returns BHMM_B200_ERR_UNSUPPORTED, a batch without owned ranges
+ * BHMM_B200_ERR_INVALID.  About N times the work of a forward pass.
+ * The caller gathers all shards' operators together with their border vectors [1] and [3] (an all_gather of
+ * K * 2 * N * (N + 1) doubles per shard), composes the exact alpha at own_lo - 1 from the first owner's [1] left to right and the
+ * exact beta at own_hi from the last owner's [3] right to left (engine.compose_shard_operators), and hands them to the shard
+ * with bhmm_b200_batch_set_border_starts (host N-vectors; NULL keeps the halo warm-up on that side, both NULL clear the
+ * trajectory's starts).  The next E-steps start the first owned chain's forward recursion and the last owned chain's backward
+ * recursion from them until they are cleared.  Rejected with BHMM_B200_ERR_INVALID: a batch without owned ranges, k out of
+ * range, a shard that owns no frame of trajectory k, vectors with a NaN, negative or infinite component or no positive one, a
+ * forward start where the owned range begins at local frame 0 and a backward start where it ends with the local trajectory. */
+int bhmm_b200_shard_operators_gaussian(bhmm_b200_batch* b, const double* d_obs, const double* A, const double* pi,
+                                       const double* means, const double* sigmas, int ignore_outliers, double* d_out,
+                                       void* stream);
+int bhmm_b200_shard_operators_discrete(bhmm_b200_batch* b, const int* d_obs, const double* A, const double* pi,
+                                       const double* B, int M, int ignore_outliers, double* d_out, void* stream);
+int bhmm_b200_batch_set_border_starts(bhmm_b200_batch* b, int k, const double* fwd, const double* bwd);
 /* The warm-up adaptation policy of the batch engine as a plain host function (no device needed; used by the tests):
  * next warm-up length from the current one, the certification's need estimate (w log tol / log m), the largest
  * hand-over mismatch m of the pass and whether the pass failed; state[2] = {remembered need, passes since confirmed}. */
