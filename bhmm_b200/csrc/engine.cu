@@ -84,6 +84,13 @@ namespace {
 
 constexpr int SEG_FRAMES = 256;   // frames per segment of the path chase
 
+// the chain-parallel Viterbi of a time shard with 32 < N <= 128 (k_viterbi_chain_wide); whole-trajectory batches with N > 32
+// keep the sequential kernels, chunked or not
+bool vit_wide(const bhmm_b200_batch* b) { return !b->own_lo.empty() && panel_viterbi_chain_wide_ok(b->N); }
+
+// words per row of the near-tie flag map: one for N <= 32, ceil(N / 32) for k_viterbi_chain_wide
+int vflag_row_words(int N) { return N <= 32 ? 1 : (N + 31) / 32; }
+
 size_t batch_layout(bhmm_b200_batch* b, char* base)
 {
     const int N = b->N;
@@ -107,7 +114,9 @@ size_t batch_layout(bhmm_b200_batch* b, char* base)
     if (b->no_alpha) alpha_doubles = 32;      // Viterbi needs the observations, the back-pointer map and the path only
     const size_t o_alpha = cv.add<double>(alpha_doubles);
     const size_t o_F = cv.add<unsigned char>((size_t)b->rows * N * (N > 256 ? 2 : 1));
-    const size_t o_vflag = cv.add<unsigned>(panel_viterbi_chain_ok(N) ? (size_t)b->rows : 1);
+    size_t vflag_words = panel_viterbi_chain_ok(N) ? (size_t)b->rows : 1;
+    if (vit_wide(b)) vflag_words = (size_t)b->rows * vflag_row_words(N);   // time shard, 32 < N <= 128: k_viterbi_chain_wide
+    const size_t o_vflag = cv.add<unsigned>(vflag_words);
     if (base) {
         b->d_offsets = (long long*)(base + o_offs);
         b->w = ChainWork();
@@ -165,8 +174,9 @@ void batch_plan(bhmm_b200_batch* b, int chunk, int warm)
         if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         int tthreads = 32, tcpb = 1;
         team_shape(b->N, &tthreads, &tcpb);
-        const long long cap = b->lane ? (long long)sms * lane_blocks_per_sm(b->N, EM_GAUSS) * lane_threads()
-                                      : (long long)backward_stats_grid(b->N, 1 << 28) * tcpb;
+        long long cap = b->lane ? (long long)sms * lane_blocks_per_sm(b->N, EM_GAUSS) * lane_threads()
+                                : (long long)backward_stats_grid(b->N, 1 << 28) * tcpb;
+        if (b->no_alpha && vit_wide(b)) cap = viterbi_chain_wide_wave(b->N);   // a Viterbi-only shard runs that kernel only
         auto count = [&](long long c) {
             long long n = 0;
             for (int k = 0; k < b->K; ++k) {
@@ -881,8 +891,10 @@ extern "C" int bhmm_b200_wave_chains(int N)
 extern "C" int bhmm_b200_batch_set_viterbi_only(bhmm_b200_batch* b, int on)
 {
     if (!b) return BHMM_ERR_INVALID;
+    const bool was = b->no_alpha;
     b->no_alpha = on != 0;
     b->carved = false;          // the workspace is laid out again (query bhmm_b200_batch_workspace_bytes after this call)
+    if (was != b->no_alpha && vit_wide(b)) batch_plan(b, b->req_chunk, b->req_warm);   // its chain plan follows the Viterbi kernel
     return BHMM_OK;
 }
 
@@ -1049,9 +1061,11 @@ static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const do
     // (bhmm_b200_batch_border_handovers), the state at the last owned frame comes from the shard that owns the next frames
     // (bhmm_b200_batch_set_viterbi_end_state), and the local trajectory must END with the owned range (no right halo).
     const bool sharded = !b->own_lo.empty();
+    const bool wide = vit_wide(b);
+    const int NW = wide ? vflag_row_words(N) : 1;            // flag words per row of the map
     const int phase = b->vit_phase;
     if (sharded) {
-        if (!(panel_viterbi_chain_ok(N) && N <= 256)) { bhmm_set_error(BHMM_ERR_UNSUPPORTED, "Viterbi on a time shard needs the chain-parallel Viterbi kernels (N <= 32, BHMM_B200_PANEL != 0)"); return BHMM_ERR_UNSUPPORTED; }
+        if (!panel_viterbi_chain_ok(N) && !wide) { bhmm_set_error(BHMM_ERR_UNSUPPORTED, "Viterbi on a time shard needs the chain-parallel Viterbi kernels (N <= 128, BHMM_B200_PANEL != 0)"); return BHMM_ERR_UNSUPPORTED; }
         for (int k = 0; k < b->K; ++k) {
             if (b->own_hi[k] != b->offsets[k + 1] - b->offsets[k]) { bhmm_set_error(BHMM_ERR_INVALID, "Viterbi on a time shard: the local trajectory must end with its owned range"); return BHMM_ERR_INVALID; }
             if (!b->w.chunked && b->own_lo[k] != 0) { bhmm_set_error(BHMM_ERR_INVALID, "Viterbi on a time shard: plan without chains"); return BHMM_ERR_INVALID; }
@@ -1064,7 +1078,7 @@ static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const do
     // certified only matters if the resolved path goes through it: that is checked after the path chase, and then -- or when
     // the hand-overs cannot be certified -- the sequential kernel recomputes the whole map.
     bool chunked_map = (phase == 2) ? b->vit_map_chunked : false;
-    if (phase != 2 && panel_viterbi_chain_ok(N) && b->w.chunked) {
+    if (phase != 2 && (panel_viterbi_chain_ok(N) || wide) && b->w.chunked) {
         VitChainArgs va{};
         va.em = em; va.N = N; va.A = b->d_A; va.pi = b->d_pi; va.backptr = b->d_F;
         va.hand_used = b->w.hu_f; va.hand_end = b->w.he_f; va.flagmap = b->d_vflag;
@@ -1073,7 +1087,7 @@ static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const do
         const int rc = run_chains_certified(b->w, N, +1, [&](const Chains& ch, cudaStream_t s2) {
             VitChainArgs x = va;
             x.ch = ch;
-            return launch_viterbi_chain(x, emkind, s2);
+            return wide ? launch_viterbi_chain_wide(x, emkind, s2) : launch_viterbi_chain(x, emkind, s2);
         }, b->info, st);
         if (rc == BHMM_OK) {
             chunked_map = true;
@@ -1099,13 +1113,13 @@ static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const do
                 const long long r0 = b->offsets[k], Tk = b->offsets[k + 1] - r0, lo = b->own_lo[k];
                 if (lo > 1) {
                     CUDA_TRY(cudaMemsetAsync(b->d_F + (size_t)r0 * N, 0, (size_t)(lo - 1) * N, st));
-                    if (chunked_map) CUDA_TRY(cudaMemsetAsync(b->d_vflag + r0, 0, sizeof(unsigned) * (size_t)(lo - 1), st));
+                    if (chunked_map) CUDA_TRY(cudaMemsetAsync(b->d_vflag + (size_t)r0 * NW, 0, sizeof(unsigned) * (size_t)(lo - 1) * NW, st));
                 }
                 const int es = k < (int)b->vit_end.size() ? b->vit_end[k] : -1;
                 if (es >= 0) {
                     if (es >= N) { bhmm_set_error(BHMM_ERR_INVALID, "Viterbi end state out of range"); return BHMM_ERR_INVALID; }
                     CUDA_TRY(cudaMemsetAsync(b->d_F + (size_t)(r0 + Tk - 1) * N, es, (size_t)N, st));
-                    if (chunked_map) CUDA_TRY(cudaMemsetAsync(b->d_vflag + r0 + Tk - 1, 0, sizeof(unsigned), st));
+                    if (chunked_map) CUDA_TRY(cudaMemsetAsync(b->d_vflag + (size_t)(r0 + Tk - 1) * NW, 0, sizeof(unsigned) * NW, st));
                 }
             }
         }
@@ -1116,7 +1130,8 @@ static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const do
         if (!chunked_map) break;
         int flagged = 0;
         CUDA_TRY(cudaMemsetAsync(b->d_err + 1, 0, sizeof(int), st));
-        RC_TRY(launch_viterbi_path_flags(b->d_vflag, d_path, b->d_offsets, b->K, b->rows, b->d_err + 1, st));
+        if (wide) RC_TRY(launch_viterbi_path_flags_wide(b->d_vflag, NW, d_path, b->d_offsets, b->K, b->rows, b->d_err + 1, st));
+        else RC_TRY(launch_viterbi_path_flags(b->d_vflag, d_path, b->d_offsets, b->K, b->rows, b->d_err + 1, st));
         LAUNCHED(1);
         CUDA_TRY(cudaMemcpyAsync(&flagged, b->d_err + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));

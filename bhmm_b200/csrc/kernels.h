@@ -58,7 +58,8 @@ struct VitChainArgs {
     double* hand_used;       // (n_chains_total, N): normalised max-product vector at t0-1 the chain was started from
     double* hand_end;        // (n_chains_total, N): the chain's vector at its last frame
     unsigned* flagmap;       // (rows) one word per row of the map: bit j set = the decision stored in F[row][j] had a
-                             // relative margin below margin_min (only decisions ON the resolved path matter)
+                             // relative margin below margin_min (only decisions ON the resolved path matter);
+                             // (rows, ceil(N / 32)) words for k_viterbi_chain_wide
     double margin_min;
 };
 
@@ -152,6 +153,13 @@ int launch_viterbi_chain(const VitChainArgs& a, int em, cudaStream_t st);
 // counter += number of decisions ON the resolved paths whose margin was flagged (0: the paths are certified)
 int launch_viterbi_path_flags(const unsigned* flagmap, const int* path, const long long* offsets, int K, long long rows,
                               int* counter, cudaStream_t st);
+// 32 < N <= 128: the time-chunked Viterbi of a time shard (panel_kernels.cu:k_viterbi_chain_wide), same contract except for
+// the flag map, which holds NW = ceil(N / 32) words per row (word w, bit b: next state 32 w + b)
+bool panel_viterbi_chain_wide_ok(int N);
+int viterbi_chain_wide_wave(int N);          // chains of one full wave of resident k_viterbi_chain_wide groups
+int launch_viterbi_chain_wide(const VitChainArgs& a, int em, cudaStream_t st);
+int launch_viterbi_path_flags_wide(const unsigned* flagmap, int NW, const int* path, const long long* offsets, int K,
+                                   long long rows, int* counter, cudaStream_t st);
 
 // ---- frame-parallel kernels (frame_kernels.cu)
 int launch_gaussian_pobs(const double* obs, const double* mu, const double* sigma, int N, long long rows,

@@ -2011,6 +2011,251 @@ __global__ void k_viterbi_path_flags(const unsigned* __restrict__ flagmap, const
     if (hits) atomicAdd(counter, hits);
 }
 
+// ================================================================================================
+// Time-chunked Viterbi, 32 < N <= 128 (a trajectory cut in time across devices at the model sizes of C4).  The contract is
+// k_viterbi_chain32's -- start modes (pi at frame 0, uniform warm-up, exact hand-over vector), hand_used at t0 - 1 and
+// hand_end at the last frame, back-pointers for t >= t0 only, near-tie flags -- and the layout k_viterbi_multi's: thread j
+// owns state j in groups of `sthr` threads, A sits in shared memory with the padded stride NPS, one copy per block shared by
+// its nsub groups, and every group walks R chains in lock step (the chains of one plan have nearly equal lengths, so the
+// shorter ones idle for at most a warm-up's difference).  Arithmetic per frame is _hidden.c:229-265's, bit for bit: products
+// v_i A_ij, first maximum with strict '>', (p_j v_best) A_best,j, j-sequential sum, true division.  The flag map has
+// NW = ceil(N / 32) words per row, word w bit b standing for the next state 32 w + b (k_viterbi_path_flags_wide); the last
+// row of a trajectory is flagged as a whole.
+// ================================================================================================
+// doubles of shared memory per group of k_viterbi_chain_wide: vb, ub (R x NPS each), ssum (R), anynz (4 R ints), the chains'
+// first rows (R) and descriptions (8 R ints)
+__host__ __device__ constexpr size_t chain_wide_group_doubles(int NPS, int R) { return 2 * (size_t)R * NPS + 8 * (size_t)R; }
+
+template <int EM, int R>
+__global__ void __launch_bounds__(512, 1) k_viterbi_chain_wide(const VitChainArgs a, int NPS, int sthr)
+{
+    PANEL_DYN_SMEM(vsm);
+    const int N = a.N, nsub = blockDim.x / sthr, sub = threadIdx.x / sthr;
+    const int j = threadIdx.x - sub * sthr, nthr = sthr, wid = j >> 5, lane = j & 31, nwarp = sthr >> 5;
+    const int NW = (N + 31) >> 5;
+    double* const As = vsm;                                 // [N][NPS], shared by the groups
+    double* const vb = As + (size_t)N * NPS + sub * chain_wide_group_doubles(NPS, R);   // [R][NPS] normalised rows
+    double* const ub = vb + R * NPS;                        // [R][NPS] unnormalised rows
+    double* const ssum = ub + R * NPS;                      // [R]
+    int* const anynz = reinterpret_cast<int*>(ssum + R);    // [R][4] per warp: any density != 0 (outlier rule)
+    // the R chains' descriptions live in shared memory, not in registers (at 128 registers per thread they would spill):
+    // row of frame 0, and chain, t0, end frame, trajectory length, start frame, first frame walked, start mode
+    long long* const trow = reinterpret_cast<long long*>(anynz + 4 * R);   // [R]
+    int* const cd = reinterpret_cast<int*>(trow + R);       // [R][8]
+    enum { C_C, C_T0, C_TEND, C_T, C_TSTART, C_TFIRST, C_MODE };
+    const bool jv = j < N;
+    for (int k = threadIdx.x; k < N * NPS; k += blockDim.x) {
+        const int i = k / NPS, c = k - i * NPS;
+        As[k] = (c < N) ? a.A[i * N + c] : 0.0;
+    }
+    double mu = 0.0, sigma = 1.0;
+    if (EM == EM_GAUSS && jv) { mu = a.em.mu[j]; sigma = a.em.sigma[j]; }
+    const double pi_j = jv ? a.pi[j] : 0.0;
+    unsigned char* bp = reinterpret_cast<unsigned char*>(a.backptr);
+    const bool outl = (EM != EM_POBS) && a.em.ignore_outliers;
+    __syncthreads();
+
+    for (int idx0 = (blockIdx.x * nsub + sub) * R; idx0 < a.ch.n; idx0 += gridDim.x * nsub * R) {
+        if (j < R) {                                        // thread r describes chain r
+            int* const d = cd + 8 * j;
+            int c = -1, t0 = 0, tend = 0, T = 0, tstart = 0, mode = 0;
+            long long row = 0;
+            if (idx0 + j < a.ch.n) {
+                c = a.ch.list ? a.ch.list[idx0 + j] : idx0 + j;
+                t0 = a.ch.t0[c];
+                T = a.ch.T[c];
+                tend = t0 + a.ch.len[c];
+                row = a.ch.row0[c] - t0;
+                // mode 0: pi at frame 0, 1: uniform warm-up start, 2: exact vector (k_viterbi_chain32)
+                if (t0 == 0) { tstart = 0; mode = 0; }
+                else if (a.ch.exact) { tstart = t0 - 1; mode = 2; }
+                else { tstart = max(0, t0 - (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm)); mode = (tstart == 0) ? 0 : 1; }
+            }
+            d[C_C] = c; d[C_T0] = t0; d[C_TEND] = tend; d[C_T] = T; d[C_TSTART] = tstart;
+            d[C_TFIRST] = (mode == 2) ? t0 : tstart; d[C_MODE] = mode;
+            trow[j] = row;
+        }
+        for (int k = j; k < 2 * R * NPS; k += nthr) vb[k] = 0.0;
+        sub_barrier(sub, sthr, nsub);
+        int steps = 0;
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            const int* const d = cd + 8 * r;
+            steps = max(steps, d[C_TEND] - d[C_TFIRST]);
+            if (d[C_MODE] == 2 && jv) {
+                const double x = a.hand_end[(long long)(d[C_C] - 1) * N + j];
+                vb[r * NPS + j] = x;
+                a.hand_used[(long long)d[C_C] * N + j] = x;
+            }
+        }
+        sub_barrier(sub, sthr, nsub);
+        auto em_raw = [&](int r, int t) -> double {
+            if (!jv || t >= cd[8 * r + C_TEND]) return 0.0;
+            const long long row = trow[r] + t;
+            if (EM == EM_POBS) return a.em.pobs[row * N + j];
+            if (EM == EM_GAUSS) return a.em.obs[row];
+            return a.em.Bt[(long long)a.em.sym[row] * N + j];
+        };
+        double raw_next[R];
+#pragma unroll
+        for (int r = 0; r < R; ++r) raw_next[r] = em_raw(r, cd[8 * r + C_TFIRST]);
+        for (int s = 0; s < steps; ++s) {
+            double p[R], vn[R];
+#pragma unroll
+            for (int r = 0; r < R; ++r) {
+                const int t = cd[8 * r + C_TFIRST] + s;
+                const double raw = raw_next[r];
+                raw_next[r] = em_raw(r, t + 1);
+                p[r] = 0.0;
+                if (jv && t < cd[8 * r + C_TEND]) p[r] = (EM == EM_GAUSS) ? gauss_pdf(raw, mu, sigma) : raw;
+            }
+            if (outl) {                                     // outputmodel.py:126-130, one vote per chain
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    const unsigned nzw = __ballot_sync(FULL, p[r] != 0.0);
+                    if (lane == 0) anynz[r * 4 + wid] = nzw != 0u;
+                }
+                sub_barrier(sub, sthr, nsub);
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    int any = 0;
+                    for (int w2 = 0; w2 < nwarp; ++w2) any |= anynz[r * 4 + w2];
+                    if (!any) p[r] = (jv && cd[8 * r + C_TFIRST] + s < cd[8 * r + C_TEND]) ? 1.0 : 0.0;
+                }
+            }
+            // the scan of every chain, also of one at its start frame (whose result is not used): best and second-best
+            // candidate, the first maximum with strict '>' (_hidden.c:186-200)
+            double m[R], m2[R];
+            int bi[R];
+#pragma unroll
+            for (int r = 0; r < R; ++r) { m[r] = __dmul_rn(vb[r * NPS], As[j]); m2[r] = -1.0; bi[r] = 0; }
+            {   // N > 32: state 1 alone, then two predecessors per step from one 16-byte broadcast load (k_viterbi_multi)
+                const double a1 = As[NPS + j];
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    const double h = __dmul_rn(vb[r * NPS + 1], a1);
+                    if (h > m[r]) { m2[r] = m[r]; m[r] = h; bi[r] = 1; }
+                    else if (h > m2[r]) m2[r] = h;
+                }
+            }
+            int i = 2;
+#pragma unroll 2
+            for (; i + 1 < N; i += 2) {
+                const double a0 = As[i * NPS + j], a1 = As[(i + 1) * NPS + j];
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    const double2 v2 = *reinterpret_cast<const double2*>(vb + r * NPS + i);
+                    const double h0 = __dmul_rn(v2.x, a0), h1 = __dmul_rn(v2.y, a1);
+                    if (h0 > m[r]) { m2[r] = m[r]; m[r] = h0; bi[r] = i; }
+                    else if (h0 > m2[r]) m2[r] = h0;
+                    if (h1 > m[r]) { m2[r] = m[r]; m[r] = h1; bi[r] = i + 1; }
+                    else if (h1 > m2[r]) m2[r] = h1;
+                }
+            }
+            if (i < N) {
+                const double a0 = As[i * NPS + j];
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    const double h = __dmul_rn(vb[r * NPS + i], a0);
+                    if (h > m[r]) { m2[r] = m[r]; m[r] = h; bi[r] = i; }
+                    else if (h > m2[r]) m2[r] = h;
+                }
+            }
+#pragma unroll
+            for (int r = 0; r < R; ++r) {
+                const int t = cd[8 * r + C_TFIRST] + s;
+                const bool act = t < cd[8 * r + C_TEND], first = act && t == cd[8 * r + C_TSTART] && cd[8 * r + C_MODE] != 2;
+                const bool near = jv && m[r] > 0.0 && (m[r] - fmax(m2[r], 0.0)) < a.margin_min * m[r];
+                const unsigned word = __ballot_sync(FULL, near);
+                if (first) {
+                    vn[r] = (cd[8 * r + C_MODE] == 0) ? __dmul_rn(p[r], pi_j) : p[r];
+                } else {
+                    if (act && t >= cd[8 * r + C_T0]) {
+                        if (jv) bp[(trow[r] + t - 1) * N + j] = (unsigned char)bi[r];
+                        if (lane == 0 && wid < NW) a.flagmap[(trow[r] + t - 1) * NW + wid] = word;
+                    }
+                    vn[r] = __dmul_rn(__dmul_rn(p[r], vb[r * NPS + bi[r]]), As[bi[r] * NPS + j]);   // _hidden.c:247-250
+                }
+            }
+            // (ub's readers -- the sums of the previous frame -- finished before that frame's third barrier)
+            if (j < NPS) {
+#pragma unroll
+                for (int r = 0; r < R; ++r) ub[r * NPS + j] = (jv && cd[8 * r + C_TFIRST] + s < cd[8 * r + C_TEND]) ? vn[r] : 0.0;
+            }
+            sub_barrier(sub, sthr, nsub);
+            {   // j-sequential sums (_hidden.c:254-259): warp w adds up the rows w, w + nwarp, ...
+                constexpr int RW = (R + 1) / 2;             // rows per warp at two warps per group (the fewest)
+                double sacc[RW];
+#pragma unroll
+                for (int q = 0; q < RW; ++q) sacc[q] = 0.0;
+                for (int i = 0; i < N; ++i) {
+#pragma unroll
+                    for (int q = 0; q < RW; ++q) {
+                        const int r = wid + q * nwarp;
+                        if (r < R) sacc[q] = __dadd_rn(sacc[q], ub[r * NPS + i]);
+                    }
+                }
+                if (lane == 0) {
+#pragma unroll
+                    for (int q = 0; q < RW; ++q)
+                        if (wid + q * nwarp < R) ssum[wid + q * nwarp] = sacc[q];
+                }
+            }
+            sub_barrier(sub, sthr, nsub);
+            if (j < NPS) {
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    const int t = cd[8 * r + C_TFIRST] + s;
+                    if (t >= cd[8 * r + C_TEND]) continue;
+                    const double x = jv ? __ddiv_rn(vn[r], ssum[r]) : 0.0;
+                    vb[r * NPS + j] = x;
+                    if (jv && t == cd[8 * r + C_T0] - 1) a.hand_used[(long long)cd[8 * r + C_C] * N + j] = x;
+                    if (jv && t == cd[8 * r + C_TEND] - 1) a.hand_end[(long long)cd[8 * r + C_C] * N + j] = x;
+                }
+            }
+            sub_barrier(sub, sthr, nsub);
+        }
+        // path[T-1] = first maximum of the last row (_hidden.c:268): the last row of the map holds it for every s'
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            if (cd[8 * r + C_C] < 0 || cd[8 * r + C_TEND] != cd[8 * r + C_T]) continue;
+            int best = 0;
+            double mm = vb[r * NPS], second = -1.0;
+            for (int i = 1; i < N; ++i) {
+                const double x = vb[r * NPS + i];
+                if (x > mm) { second = mm; mm = x; best = i; }
+                else if (x > second) second = x;
+            }
+            if (jv) bp[(trow[r] + cd[8 * r + C_T] - 1) * N + j] = (unsigned char)best;
+            const bool near = mm > 0.0 && (mm - fmax(second, 0.0)) < a.margin_min * mm;
+            if (j < NW) a.flagmap[(trow[r] + cd[8 * r + C_T] - 1) * NW + j] = near ? 0xffffffffu : 0u;
+        }
+        sub_barrier(sub, sthr, nsub);
+    }
+}
+
+// On-path flags of the wide chunked Viterbi: row r holds NW words, bit b of word w for the decision "state at r given the
+// state 32 w + b at r + 1"; the last row of a trajectory holds the final arg max (any bit).
+__global__ void k_viterbi_path_flags_wide(const unsigned* __restrict__ flagmap, int NW, const int* __restrict__ path,
+                                          const long long* __restrict__ offsets, int K, long long rows, int* counter)
+{
+    int hits = 0;
+    for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (long long)gridDim.x * blockDim.x) {
+        const unsigned* w = flagmap + r * NW;
+        unsigned any = 0u;
+        for (int q = 0; q < NW; ++q) any |= w[q];
+        if (any == 0u) continue;
+        int lo = 0, hi = K;                                 // trajectory of row r: offsets[lo] <= r < offsets[lo + 1]
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (offsets[mid] <= r) lo = mid; else hi = mid;
+        }
+        const bool last = (r == offsets[lo + 1] - 1);
+        if (last || ((w[path[r + 1] >> 5] >> (path[r + 1] & 31)) & 1u)) ++hits;
+    }
+    if (hits) atomicAdd(counter, hits);
+}
+
 #ifndef PANEL_HOST_NO_LAUNCHERS
 int panel_sms()
 {
@@ -2259,6 +2504,91 @@ int launch_viterbi_path_flags(const unsigned* flagmap, const int* path, const lo
     if (rows <= 0) return BHMM_OK;
     const int grid = (int)std::max(1LL, std::min<long long>((rows + 255) / 256, (long long)panel_sms() * 8));
     k_viterbi_path_flags<<<grid, 256, 0, st>>>(flagmap, path, offsets, K, rows, counter);
+    return BHMM_OK;
+}
+
+bool panel_viterbi_chain_wide_ok(int N) { return panel_mode() > 0 && N > 32 && N <= 128; }
+
+#ifndef VITERBI_CHAIN_WIDE_R
+#define VITERBI_CHAIN_WIDE_R 4
+#endif
+
+namespace {
+// k_viterbi_chain_wide's shape for N: threads per group (one per state), padded stride, groups per block, dynamic shared memory
+struct ChainWideShape { int sthr, NPS, nsub; size_t smem; };
+ChainWideShape chain_wide_shape(int N, int nsub)
+{
+    constexpr int R = VITERBI_CHAIN_WIDE_R;
+    ChainWideShape s;
+    s.sthr = N <= 64 ? 64 : 128;
+    s.NPS = (N + 1) & ~1;
+    s.nsub = nsub;
+    s.smem = sizeof(double) * ((size_t)N * s.NPS + (size_t)nsub * chain_wide_group_doubles(s.NPS, R));
+    return s;
+}
+
+template <int EM>
+int chain_wide_blocks_per_sm(const ChainWideShape& s, int* per)
+{
+    constexpr int R = VITERBI_CHAIN_WIDE_R;
+    if (cudaFuncSetAttribute(k_viterbi_chain_wide<EM, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s.smem) != cudaSuccess) {
+        bhmm_set_error(BHMM_ERR_CUDA, "cudaFuncSetAttribute failed for k_viterbi_chain_wide");
+        return BHMM_ERR_CUDA;
+    }
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(per, k_viterbi_chain_wide<EM, R>, s.nsub * s.sthr, s.smem) != cudaSuccess
+        || *per <= 0)
+        *per = 1;
+    return BHMM_OK;
+}
+
+template <int EM>
+int launch_viterbi_chain_wide_em(const VitChainArgs& a, cudaStream_t st)
+{
+    constexpr int R = VITERBI_CHAIN_WIDE_R;
+    const long long groups = ((long long)a.ch.n + R - 1) / R;
+#ifdef PANEL_HOST_EMU
+    const int nsub = 1;                                     // the emulated build runs one group per block
+#else
+    const int sthr = a.N <= 64 ? 64 : 128;
+    const int nsub = (int)std::max<long long>(1, std::min<long long>(512 / sthr, (groups + panel_sms() - 1) / panel_sms()));
+#endif
+    const ChainWideShape s = chain_wide_shape(a.N, nsub);
+    int per = 1;
+    { const int rc_ = chain_wide_blocks_per_sm<EM>(s, &per); if (rc_ != BHMM_OK) return rc_; }
+    const long long blocks = (groups + nsub - 1) / nsub;
+    k_viterbi_chain_wide<EM, R><<<(int)std::min<long long>(blocks, (long long)panel_sms() * per), nsub * s.sthr, s.smem, st>>>(
+        a, s.NPS, s.sthr);
+    return BHMM_OK;
+}
+}  // namespace
+
+int viterbi_chain_wide_wave(int N)
+{
+    if (!panel_viterbi_chain_wide_ok(N)) return 0;
+    const ChainWideShape s = chain_wide_shape(N, N <= 64 ? 8 : 4);
+    int per = 1;
+    if (chain_wide_blocks_per_sm<EM_GAUSS>(s, &per) != BHMM_OK) { bhmm_set_error(BHMM_OK, ""); per = 1; }
+    return panel_sms() * per * s.nsub * VITERBI_CHAIN_WIDE_R;
+}
+
+int launch_viterbi_chain_wide(const VitChainArgs& a, int em, cudaStream_t st)
+{
+    if (a.N <= 32 || a.N > 128) return BHMM_ERR_UNSUPPORTED;
+    if (a.ch.n <= 0) return BHMM_OK;
+    switch (em) {
+        case EM_POBS: return launch_viterbi_chain_wide_em<EM_POBS>(a, st);
+        case EM_GAUSS: return launch_viterbi_chain_wide_em<EM_GAUSS>(a, st);
+        case EM_DISC: return launch_viterbi_chain_wide_em<EM_DISC>(a, st);
+    }
+    return BHMM_ERR_INVALID;
+}
+
+int launch_viterbi_path_flags_wide(const unsigned* flagmap, int NW, const int* path, const long long* offsets, int K,
+                                   long long rows, int* counter, cudaStream_t st)
+{
+    if (rows <= 0) return BHMM_OK;
+    const int grid = (int)std::max(1LL, std::min<long long>((rows + 255) / 256, (long long)panel_sms() * 8));
+    k_viterbi_path_flags_wide<<<grid, 256, 0, st>>>(flagmap, NW, path, offsets, K, rows, counter);
     return BHMM_OK;
 }
 

@@ -922,8 +922,8 @@ class TimeShardedTrajectories(object):
     (``set_border_starts``) instead of the halo warm-up; its borders are certified again.  ``combine``, ``certify`` and
     ``estep_gaussian`` keep raising on a halo that is too short.
 
-    Viterbi works across shards as well (``viterbi_gaussian`` / ``viterbi_discrete``): every shard builds the back-pointer
-    map of its owned frames with the chain-parallel Viterbi kernels, warming its max-product vector up on the halo BEFORE
+    Viterbi works across shards as well (``viterbi_gaussian`` / ``viterbi_discrete``, N <= 128): every shard builds the
+    back-pointer map of its owned frames with the chain-parallel Viterbi kernels, warming its max-product vector up on the halo BEFORE
     its range; the vector each shard started from is certified against the one its left neighbour computed (same
     component-wise relative test as for the E-step); then the paths are resolved from the last shard to the first, each
     shard handing the state at its neighbour's last frame -- one integer per trajectory -- to the left.  A path that goes

@@ -37,7 +37,7 @@ class MaximumLikelihoodEstimator(object):
     certified borders and, where a border does not certify, the exact operator exchange (``TimeShardedTrajectories.estep``);
     ``border_fallbacks`` counts the iterations that needed it.  The M-step is unchanged.  ``fit()`` ends with Viterbi across
     the shards, and ``hidden_state_trajectories`` holds this rank's owned pieces of the paths; where time-sharded Viterbi is
-    not available (N > 32) or its borders do not certify, they stay None and a warning is logged.
+    not available (N > 128) or its borders do not certify, they stay None and a warning is logged.
     """
 
     def __init__(self, observations, nstates, initial_model=None, output='gaussian', reversible=True, stationary=False,
@@ -186,9 +186,9 @@ class MaximumLikelihoodEstimator(object):
 
     def _time_sharded_viterbi(self):
         """Viterbi across the time shards: this rank's owned pieces of the paths, or None (with a warning) where that is not
-        available -- N > 32, or a border or a decision that does not certify -- so that a finished fit is kept."""
-        if self._nstates > 32:
-            logger().warning('time-sharded Viterbi needs N <= 32; hidden_state_trajectories left at None')
+        available -- N > 128, or a border or a decision that does not certify -- so that a finished fit is kept."""
+        if self._nstates > 128:
+            logger().warning('time-sharded Viterbi needs N <= 128; hidden_state_trajectories left at None')
             return None
         try:
             if self._batch.world == 1:

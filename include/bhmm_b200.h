@@ -234,7 +234,9 @@ int bhmm_b200_viterbi_discrete(bhmm_b200_batch* b, const int* d_obs, const doubl
  * compare across shards).  phase 2: only resolves the path, ending in the state set by
  * bhmm_b200_batch_set_viterbi_end_state (the state of trajectory k at its last local frame, i.e. path[own_lo - 1] of the
  * shard that owns the following frames; -1 = this shard holds the trajectory's end).  phase 0 (default) does both.
- * d_path is filled for the local rows; rows before own_lo - 1 are meaningless. */
+ * d_path is filled for the local rows; rows before own_lo - 1 are meaningless.  N <= 128 (BHMM_B200_PANEL=0: none); a path
+ * through a decision whose margin is below the certified tolerance returns BHMM_B200_ERR_NOT_CERTIFIED.  For 32 < N <= 128
+ * the near-tie flags take ceil(N / 32) words per frame, and a Viterbi-only shard sizes its chains to that kernel's wave. */
 int bhmm_b200_batch_set_viterbi_phase(bhmm_b200_batch* b, int phase);
 int bhmm_b200_batch_set_viterbi_end_state(bhmm_b200_batch* b, int k, int state);
 /* One Gibbs hidden-path sweep (bayesian_sampling.py:283-331): emission + forward + backward sampling of every
