@@ -85,6 +85,7 @@ _proto('bhmm_b200_batch_replan', C.c_int, _vp, C.c_int, C.c_int)
 _proto('bhmm_b200_batch_uses_lane_kernels', C.c_int, _vp)
 _proto('bhmm_b200_wave_chains', C.c_int, C.c_int)
 _proto('bhmm_b200_batch_scan_count', C.c_double, _vp)
+_proto('bhmm_b200_batch_viterbi_sequential_count', C.c_double, _vp)
 _proto('bhmm_b200_batch_debug_handovers', C.c_int, _vp, C.c_int, _dp, _dp)
 _proto('bhmm_b200_batch_set_family', C.c_int, _vp, C.c_int)
 _proto('bhmm_b200_batch_set_viterbi_phase', C.c_int, _vp, C.c_int)
@@ -98,6 +99,9 @@ _proto('bhmm_b200_batch_gibbs_shard_map', C.c_int, _vp, C.c_int, _vp)
 _proto('bhmm_b200_shard_operators_gaussian', C.c_int, _vp, _vp, _dp, _dp, _dp, _dp, C.c_int, _vp, _vp)
 _proto('bhmm_b200_shard_operators_discrete', C.c_int, _vp, _vp, _dp, _dp, _dp, C.c_int, C.c_int, _vp, _vp)
 _proto('bhmm_b200_batch_set_border_starts', C.c_int, _vp, C.c_int, _dp, _dp)
+_proto('bhmm_b200_shard_viterbi_operators_gaussian', C.c_int, _vp, _vp, _dp, _dp, _dp, _dp, C.c_int, _vp, _vp)
+_proto('bhmm_b200_shard_viterbi_operators_discrete', C.c_int, _vp, _vp, _dp, _dp, _dp, C.c_int, C.c_int, _vp, _vp)
+_proto('bhmm_b200_batch_set_viterbi_margin', C.c_int, _vp, C.c_double)
 _proto('bhmm_b200_batch_workspace_bytes', C.c_size_t, _vp)
 _proto('bhmm_b200_batch_attach_workspace', C.c_int, _vp, _vp, C.c_size_t)
 _proto('bhmm_b200_batch_info', None, _vp, _dp)

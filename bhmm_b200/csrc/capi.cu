@@ -278,38 +278,47 @@ long long certify_collect(ChainWork& w, int dir, double* worst)
     return (long long)g_pinned_cert[4 * slot];
 }
 
-int run_chains_certified(ChainWork& w, int N, int dir, const ChainLauncher& launch, RunInfo& info, cudaStream_t st)
+int run_chains_certified(ChainWork& w, int N, int dir, const ChainLauncher& launch, RunInfo& info, cudaStream_t st,
+                         bool scan_first)
 {
     Chains all = w.ch;
     all.list = nullptr; all.n = w.n_total; all.exact = 0;
     all.warmv = nullptr;
     (dir > 0 ? w.need_f : w.need_b) = 0.0;
-    RC_TRY(launch(all, st));
-    LAUNCHED(1);
-    if (!w.chunked) return BHMM_OK;
     double& worst = dir > 0 ? info.worst_f : info.worst_b;
     double& sweeps = dir > 0 ? info.fix_f : info.fix_b;
+    auto exact_from_scan = [&]() -> int {
+        RC_TRY(w.scan(dir, st));
+        LAUNCHED(2);
+        w.scans += 1;
+        Chains ex = all;
+        ex.exact = 1;
+        RC_TRY(launch(ex, st));
+        LAUNCHED(1);
+        return BHMM_OK;
+    };
+    if (scan_first && w.chunked && w.scan) {
+        RC_TRY(exact_from_scan());
+    } else {
+        RC_TRY(launch(all, st));
+        LAUNCHED(1);
+    }
+    if (!w.chunked) return BHMM_OK;
     // After the exact scan the starts are exact up to the rounding of two different evaluation orders (operator products vs.
     // the vector recursion); a model that does not forget does not contract that difference either (measured: up to
     // 1.2e-13 over 400-frame chains), so the hand-overs of that pass are accepted at 1e-11 -- non-expansive, i.e. still two
     // orders below the 1e-10 parity bar.
-    double tol_floor = 0.0;
+    double tol_floor = (scan_first && w.scan) ? EXACT_SCAN_TOL : 0.0;
     for (int sweep = 0;; ++sweep) {
         const long long nfail = certify_sync(w, N, dir, &worst, st, tol_floor);
         if (nfail < 0) { bhmm_set_error(BHMM_ERR_CUDA, cudaGetErrorString(cudaGetLastError())); return BHMM_ERR_CUDA; }
         if (nfail == 0) break;
         if (sweep > w.n_total + 2) { bhmm_set_error(BHMM_ERR_NOT_CERTIFIED, "chain hand-overs not certified"); return BHMM_ERR_NOT_CERTIFIED; }
-        if (sweep == 1 && w.scan && nfail > 1) {
+        if (sweep == 1 && w.scan && nfail > 1 && tol_floor == 0.0) {
             // The first repair sweep did not clear the list: the model does not forget its start within the warm-up, and
             // chain-by-chain repairs would walk the trajectory sequentially.  Exact starts for ALL chains from the
             // transfer-operator scan, then one parallel pass from them.
-            RC_TRY(w.scan(dir, st));
-            LAUNCHED(2);
-            w.scans += 1;
-            Chains ex = all;
-            ex.exact = 1;
-            RC_TRY(launch(ex, st));
-            LAUNCHED(1);
+            RC_TRY(exact_from_scan());
             sweeps += 1;
             info.rerun += (double)w.n_total;
             tol_floor = EXACT_SCAN_TOL;

@@ -23,6 +23,8 @@ struct bhmm_b200_batch {
     // vit_end[k] >= 0: the state of trajectory k at its last local frame, handed over by the shard that owns the next frames
     int vit_phase = 0;
     bool vit_map_chunked = false;
+    double vit_margin = 0.0;    // near-tie margin the caller widened for exact shard starts (0: the default)
+    double vit_seq = 0.0;       // chain-parallel Viterbi maps replaced by the sequential kernel since creation
     std::vector<int> vit_end;
     // Gibbs sweep on a time shard (gibbs_shard): phase 1 = forward, table and whole-shard maps, 2 = link, replay and
     // statistics; the segment table then covers the owned frames only (gibbs_seg)
@@ -83,6 +85,25 @@ struct bhmm_b200_batch {
 namespace {
 
 constexpr int SEG_FRAMES = 256;   // frames per segment of the path chase
+
+// Near-tie margin of a Viterbi pass from exact starts: c B, B the accumulated hand-over mismatch.  A relative mismatch eps
+// bounds Hilbert's projective distance by 2 ln(1 / (1 - eps)) ~ 2 eps, distances add along the trajectory (the normalised
+// max-product map is non-expansive), and a first maximum whose relative margin exceeds the distance D cannot move
+// (candidate ratios change by at most e^D, 1 - e^-D <= D): c = 2, with headroom for the second-order terms (DESIGN.md
+// section 3).
+constexpr double VIT_SCAN_C = 2.5;
+
+// The largest hand-over mismatch the exact pass after a max-product scan is flagged for before it is measured (the pass is
+// redone when the measured one is larger); BHMM_B200_VITERBI_SCAN_GUESS overrides it (tests of the redo).
+double vit_scan_guess()
+{
+    static double g = -1.0;
+    if (g < 0.0) {
+        const char* e = getenv("BHMM_B200_VITERBI_SCAN_GUESS");
+        g = e ? std::max(0.0, atof(e)) : 1e-12;
+    }
+    return g;
+}
 
 // the chain-parallel Viterbi of a time shard with 32 < N <= 128 (k_viterbi_chain_wide); whole-trajectory batches with N > 32
 // keep the sequential kernels, chunked or not
@@ -241,21 +262,21 @@ int upload_small(double* dst, const double* src, size_t n, cudaStream_t st)
     return BHMM_OK;
 }
 
-// Installs the exact-scan fallback (scan_kernels.cu) on the batch's chain work for the duration of a pass; the callback
-// captures the caller's emission by reference, hence the guard that removes it again.
+// Installs the exact-scan fallback (scan_kernels.cu) on the batch's chain work for the duration of a pass, in semiring sr
+// (SR_MAX: Viterbi); the callback captures the caller's emission by reference, hence the guard that removes it again.
 struct ScanGuard {
     bhmm_b200_batch* b;
-    ScanGuard(bhmm_b200_batch* b_, const Emission& em, int emkind) : b(b_)
+    ScanGuard(bhmm_b200_batch* b_, const Emission& em, int emkind, int sr = SR_SUM) : b(b_)
     {
         const int N = b->N;
         static int off = -1;                                // BHMM_B200_EXACT_SCAN=0: repair sweeps only (comparison, tests)
         if (off < 0) { const char* e = getenv("BHMM_B200_EXACT_SCAN"); off = (e && e[0] == '0') ? 1 : 0; }
         if (off || !exact_scan_ok(N) || !b->w.chunked) return;
-        b->w.scan = [this, &em, emkind, N](int dir, cudaStream_t st) -> int {
+        b->w.scan = [this, &em, emkind, N, sr](int dir, cudaStream_t st) -> int {
             const size_t need = exact_scan_bytes(b->w.n_total, N);
             if (b->scan.ensure(need) != BHMM_OK) { bhmm_set_error(BHMM_ERR_NO_MEM, "exact scan: device memory for the chain operators"); return BHMM_ERR_NO_MEM; }
             Chains all = b->w.ch;
-            return launch_exact_scan(all, b->w.n_total, em, emkind, b->d_A, N, dir, dir > 0 ? b->w.he_f : b->w.he_b,
+            return launch_exact_scan(all, b->w.n_total, em, emkind, b->d_A, N, dir, sr, dir > 0 ? b->w.he_f : b->w.he_b,
                                      reinterpret_cast<double*>(b->scan.base), st);
         };
     }
@@ -872,6 +893,8 @@ extern "C" int bhmm_b200_batch_debug_handovers(const bhmm_b200_batch* b, int dir
 
 extern "C" double bhmm_b200_batch_scan_count(const bhmm_b200_batch* b) { return b ? b->w.scans : 0.0; }
 
+extern "C" double bhmm_b200_batch_viterbi_sequential_count(const bhmm_b200_batch* b) { return b ? b->vit_seq : 0.0; }
+
 extern "C" int bhmm_b200_wave_chains(int N)
 {
     if (N < 1 || N > 1024) return 0;
@@ -971,9 +994,10 @@ extern "C" int bhmm_b200_estep_discrete(bhmm_b200_batch* b, const int* d_obs, co
 }
 
 // Operators of the owned frames of every trajectory (bhmm_b200.h): k_chain_operator[_wide] over the batch's chains, then the
-// per-trajectory tree reduction (k_compose_operators), forward and backward, into d_out (K, 2, N, N + 1).
+// per-trajectory tree reduction (k_compose_operators).  E-step: sum-product, forward and backward, into d_out (K, 2, N, N + 1);
+// viterbi: max-product, forward only, into d_out (K, N, N + 1).
 static int shard_operators(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, const double* pi, double* d_out,
-                           cudaStream_t st)
+                           cudaStream_t st, bool viterbi = false)
 {
     const int N = b->N, K = b->K;
     const int n = b->w.n_total;
@@ -1005,10 +1029,11 @@ static int shard_operators(bhmm_b200_batch* b, Emission& em, int emkind, const d
     RC_TRY(upload_small(b->d_pi, pi, N, st));
     if (!pairs.empty()) CUDA_TRY(cudaMemcpyAsync(d_pairs, pairs.data(), sizeof(int) * pairs.size(), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(d_first, first.data(), sizeof(int) * K, cudaMemcpyHostToDevice, st));
-    const long long kstride = 2LL * N * (N + 1);
-    for (int d = 0; d < 2; ++d) {
-        RC_TRY(launch_shard_operators(b->w.ch, n, em, emkind, b->d_A, N, d == 0 ? +1 : -1, d_pairs, lev_n, lev_off, d_first,
-                                      K, ops, d_out + (size_t)d * N * (N + 1), kstride, st));
+    const int ndir = viterbi ? 1 : 2;
+    const long long kstride = (long long)ndir * N * (N + 1);
+    for (int d = 0; d < ndir; ++d) {
+        RC_TRY(launch_shard_operators(b->w.ch, n, em, emkind, b->d_A, N, d == 0 ? +1 : -1, viterbi ? SR_MAX : SR_SUM, d_pairs,
+                                      lev_n, lev_off, d_first, K, ops, d_out + (size_t)d * N * (N + 1), kstride, st));
         LAUNCHED((n > 0 ? 1 + lev_n.size() : 0) + 1);
     }
     return finish_stream(st);                 // (the host tables above are in use until the copies have run)
@@ -1052,6 +1077,44 @@ extern "C" int bhmm_b200_shard_operators_discrete(bhmm_b200_batch* b, const int*
     return shard_operators(b, em, EM_DISC, A, pi, d_out, st);
 }
 
+extern "C" int bhmm_b200_shard_viterbi_operators_gaussian(bhmm_b200_batch* b, const double* d_obs, const double* A,
+                                                          const double* pi, const double* means, const double* sigmas,
+                                                          int ignore_outliers, double* d_out, void* stream)
+{
+    bhmm_set_error(BHMM_OK, "");
+    RC_TRY(shard_operators_check(b, d_out));
+    if (!d_obs || !A || !pi || !means || !sigmas) { bhmm_set_error(BHMM_ERR_INVALID, "shard operators: null argument"); return BHMM_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    RC_TRY(batch_carve(b, st));
+    RC_TRY(upload_small(b->d_mu, means, b->N, st));
+    RC_TRY(upload_small(b->d_sigma, sigmas, b->N, st));
+    Emission em{};
+    em.obs = d_obs; em.mu = b->d_mu; em.sigma = b->d_sigma; em.ignore_outliers = ignore_outliers;
+    return shard_operators(b, em, EM_GAUSS, A, pi, d_out, st, true);
+}
+
+extern "C" int bhmm_b200_shard_viterbi_operators_discrete(bhmm_b200_batch* b, const int* d_obs, const double* A,
+                                                          const double* pi, const double* B, int M, int ignore_outliers,
+                                                          double* d_out, void* stream)
+{
+    bhmm_set_error(BHMM_OK, "");
+    RC_TRY(shard_operators_check(b, d_out));
+    if (!d_obs || !A || !pi || !B || M < 1) { bhmm_set_error(BHMM_ERR_INVALID, "shard operators: null argument or M < 1"); return BHMM_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    RC_TRY(batch_carve(b, st));
+    Emission em{};
+    em.sym = d_obs; em.ignore_outliers = ignore_outliers;
+    RC_TRY(prepare_discrete(b, B, M, em, st));
+    return shard_operators(b, em, EM_DISC, A, pi, d_out, st, true);
+}
+
+extern "C" int bhmm_b200_batch_set_viterbi_margin(bhmm_b200_batch* b, double margin)
+{
+    if (!b || !(margin >= 0.0) || !(margin < 1.0)) { bhmm_set_error(BHMM_ERR_INVALID, "Viterbi margin must lie in [0, 1)"); return BHMM_ERR_INVALID; }
+    b->vit_margin = margin;
+    return BHMM_OK;
+}
+
 static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const double* A, const double* pi,
                           int* d_path, cudaStream_t st)
 {
@@ -1082,20 +1145,61 @@ static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const do
         VitChainArgs va{};
         va.em = em; va.N = N; va.A = b->d_A; va.pi = b->d_pi; va.backptr = b->d_F;
         va.hand_used = b->w.hu_f; va.hand_end = b->w.he_f; va.flagmap = b->d_vflag;
-        va.margin_min = std::max(1e-11, 100.0 * g_cert_tol);   // two orders above the certification tolerance (default 1e-13)
+        // two orders above the certification tolerance (default 1e-13), or what the caller widened it to for exact shard starts
+        const double margin0 = std::max(std::max(1e-11, 100.0 * g_cert_tol), b->vit_margin);
+        va.margin_min = margin0;
         b->w.ch.warm = b->warm_f;
-        const int rc = run_chains_certified(b->w, N, +1, [&](const Chains& ch, cudaStream_t s2) {
+        // A shard's first owned chain starts from its given border start (bhmm_b200_batch_set_border_starts) or keeps its
+        // halo warm-up, also in the exact passes
+        BorderGuard border_guard(b->w, sharded);
+        if (sharded) {
+            RC_TRY(border_setup(b, st));
+            border_guard.use(b, +1);
+        }
+        // The max-product scan (model does not forget its start within the warm-up; DESIGN.md section 3).  After it, chain c
+        // starts within the sum of the hand-over mismatches of the chains before it on its trajectory of the sequential
+        // vector (Hilbert's projective metric, in which the normalised max-product map is non-expansive), and a decision is
+        // only provably the sequential one when its relative margin exceeds VIT_SCAN_C times that sum.  The sum is bounded
+        // by runs x worst, runs = the most chains of one trajectory; the exact pass flags at a guess of it, and is redone
+        // below with the measured bound when that is wider.
+        ScanGuard scan_guard(b, em, emkind, SR_MAX);
+        int runs = 1;
+        for (int k = 0; k < b->K; ++k)
+            if (b->plan.first_chain[k] >= 0) runs = std::max(runs, b->plan.last_chain[k] - b->plan.first_chain[k] + 1);
+        double scan_margin = std::max(margin0, b->vit_margin + VIT_SCAN_C * runs * vit_scan_guess());
+        if (b->w.scan) {
+            auto scan = b->w.scan;
+            b->w.scan = [&, scan](int dir, cudaStream_t s2) -> int {
+                RC_TRY(scan(dir, s2));
+                va.margin_min = scan_margin;
+                return BHMM_OK;
+            };
+        }
+        auto launch = [&](const Chains& ch, cudaStream_t s2) {
             VitChainArgs x = va;
             x.ch = ch;
             return wide ? launch_viterbi_chain_wide(x, emkind, s2) : launch_viterbi_chain(x, emkind, s2);
-        }, b->info, st);
+        };
+        const double scans0 = b->w.scans;
+        int rc = run_chains_certified(b->w, N, +1, launch, b->info, st);
+        if (rc == BHMM_OK && b->w.scans > scans0) {
+            const double need = b->vit_margin + VIT_SCAN_C * runs * b->info.worst_f;
+            if (need > va.margin_min) {
+                // the flags of that pass used a narrower margin than the measured bound: the same exact starts again (the
+                // scan is deterministic, so are the mismatches), flagged at the bound
+                scan_margin = need;
+                b->info.fix_f += 1;
+                b->info.rerun += (double)b->w.n_total;
+                rc = run_chains_certified(b->w, N, +1, launch, b->info, st, true);
+            }
+        }
         if (rc == BHMM_OK) {
             chunked_map = true;
             // the warm-up length learns from this pass like the forward filter's (estep_common)
             b->warm_f = adapt_warm(b->warm_f, b->w.need_f, b->info.worst_f, b->info.fix_f > 0, b->warm_min, b->plan.maxT, b->edge_f);
         }
         else if (rc != BHMM_ERR_NOT_CERTIFIED || sharded) return rc;
-        else bhmm_set_error(BHMM_OK, "");
+        else { bhmm_set_error(BHMM_OK, ""); b->vit_seq += 1; }
     }
     for (int pass = 0; pass < 2; ++pass) {
         if (!chunked_map && phase != 2) {
@@ -1141,6 +1245,7 @@ static int viterbi_common(bhmm_b200_batch* b, Emission& em, int emkind, const do
             return BHMM_ERR_NOT_CERTIFIED;
         }
         chunked_map = false;                                // a near-tie on the path: sequential kernel, resolve again
+        b->vit_seq += 1;
     }
     return finish_stream(st);
 }

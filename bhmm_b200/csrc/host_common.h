@@ -72,7 +72,7 @@ struct ChainWork {
     double repair_tol = 0.0;     // hand-overs above max(g_cert_tol, this) are repaired (0: the certification tolerance itself)
     double need_f = 0, need_b = 0;   // certification's estimate of the warm-up the hardest hand-over needs
     // Exact fallback for models whose filter does not forget (scan_kernels.cu): fills he_f (dir > 0) or he_b (dir < 0) with
-    // the exact hand-over vectors of every chain; set by the engine around a pass, empty when unavailable (N > 32)
+    // the exact hand-over vectors of every chain; set by the engine around a pass, empty when unavailable (N > 128)
     std::function<int(int dir, cudaStream_t st)> scan;
     double scans = 0;            // how many times the fallback ran (reported through bhmm_b200_batch_scan_count)
 };
@@ -87,9 +87,12 @@ struct RunInfo {
 };
 
 // Launch `launch(chains)` over all chains, then certify the hand-overs (dir = +1 forward, -1 backward) and re-run the
-// failing chains from the exact neighbour value (Chains.list / Chains.exact) until none fails.
+// failing chains from the exact neighbour value (Chains.list / Chains.exact) until none fails.  scan_first (with w.scan
+// installed): skip the warm-up pass and start every chain from the exact scan (the Viterbi pass that is redone with a wider
+// near-tie margin, engine.cu).
 typedef std::function<int(const Chains& ch, cudaStream_t st)> ChainLauncher;
-int run_chains_certified(ChainWork& w, int N, int dir, const ChainLauncher& launch, RunInfo& info, cudaStream_t st);
+int run_chains_certified(ChainWork& w, int N, int dir, const ChainLauncher& launch, RunInfo& info, cudaStream_t st,
+                         bool scan_first = false);
 int auto_warm_lane(int N);
 int auto_chunk_lane(long long rows, int N, int warm);
 

@@ -135,16 +135,18 @@ int launch_forward_panel(const FwdArgs& a, int em, cudaStream_t st);
 int launch_backward_stats_panel(const BwdArgs& a, int em, cudaStream_t st);
 bool panel_viterbi_ok(int N);                // 32 < N <= 104: Viterbi with the matrix column in registers
 int launch_viterbi_panel(const VitArgs& a, int em, cudaStream_t st);
-// ---- exact time-parallel chain starts (scan_kernels.cu): transfer operators per chain + a scan over them, N <= 32
+// ---- exact time-parallel chain starts (scan_kernels.cu): transfer operators per chain + a scan over them, N <= 128, in the
+// sum-product semiring (E-step, forward and backward) or the max-product one (Viterbi, forward only)
+enum { SR_SUM = 0, SR_MAX = 1 };
 bool exact_scan_ok(int N);
 size_t exact_scan_bytes(int n_chains, int N);
-int launch_exact_scan(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
+int launch_exact_scan(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir, int sr,
                       double* he, double* ops, cudaStream_t st);
 // operators of the owned frames of every trajectory of a time shard: the chains' operators reduced level by level (lev_n[L]
 // (dst, src) chain pairs at d_pairs + 2 lev_off[L]) to the chain d_first[k]; out row i of trajectory k (stride kstride
 // doubles) = [operator row i | log-scale i], the identity where d_first[k] < 0.  ops: exact_scan_bytes(n_total, N).
 int launch_shard_operators(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
-                           const int* d_pairs, const std::vector<int>& lev_n, const std::vector<long long>& lev_off,
+                           int sr, const int* d_pairs, const std::vector<int>& lev_n, const std::vector<long long>& lev_off,
                            const int* d_first, int K, double* ops, double* out, long long kstride, cudaStream_t st);
 bool lane_viterbi_ok(int N);                 // N <= 16: the chunked Viterbi runs one thread per chain (lane_viterbi.cu)
 int launch_viterbi_chain_lane(const VitChainArgs& a, int em, cudaStream_t st);

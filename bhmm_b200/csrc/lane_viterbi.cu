@@ -47,15 +47,16 @@ __global__ void __launch_bounds__(LV_THREADS) k_viterbi_chain_lane(const VitChai
         const int tend = t0 + len;
         int tstart = 0, mode = 0;                           // mode 0: pi at frame 0, 1: uniform warm-up start, 2: exact vector
         if (t0 == 0) { tstart = 0; mode = 0; }
-        else if (a.ch.exact) { tstart = t0 - 1; mode = 2; }
+        else if (chain_exact_start(a.ch, c)) { tstart = t0 - 1; mode = 2; }
         else { tstart = max(0, t0 - (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm)); mode = (tstart == 0) ? 0 : 1; }
         double v[N];
 #pragma unroll
         for (int j = 0; j < N; ++j) v[j] = 0.0;
         if (mode == 2) {
+            const double* hv = chain_start_vec(a.ch, a.hand_end, c, c - 1, N);
 #pragma unroll
             for (int j = 0; j < N; ++j) {
-                v[j] = a.hand_end[(long long)(c - 1) * N + j];
+                v[j] = hv[j];
                 a.hand_used[(long long)c * N + j] = v[j];
             }
         }

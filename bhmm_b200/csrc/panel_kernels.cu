@@ -1900,14 +1900,14 @@ __global__ void __launch_bounds__(PW * 32) k_viterbi_chain32(const VitChainArgs 
         const int tend = t0 + len;
         int tstart = 0, mode = 0;                           // mode 0: pi at frame 0, 1: uniform warm-up start, 2: exact vector
         if (t0 == 0) { tstart = 0; mode = 0; }
-        else if (a.ch.exact) { tstart = t0 - 1; mode = 2; }
+        else if (chain_exact_start(a.ch, c)) { tstart = t0 - 1; mode = 2; }
         else { tstart = max(0, t0 - (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm)); mode = (tstart == 0) ? 0 : 1; }
         u[lane] = 0.0;
         v[lane] = 0.0;
         __syncwarp();
         if (mode == 2) {
             if (jv) {
-                const double x = a.hand_end[(long long)(c - 1) * N + j];
+                const double x = chain_start_vec(a.ch, a.hand_end, c, c - 1, N)[j];
                 v[j] = x;
                 a.hand_used[(long long)c * N + j] = x;
             }
@@ -2068,7 +2068,7 @@ __global__ void __launch_bounds__(512, 1) k_viterbi_chain_wide(const VitChainArg
                 row = a.ch.row0[c] - t0;
                 // mode 0: pi at frame 0, 1: uniform warm-up start, 2: exact vector (k_viterbi_chain32)
                 if (t0 == 0) { tstart = 0; mode = 0; }
-                else if (a.ch.exact) { tstart = t0 - 1; mode = 2; }
+                else if (chain_exact_start(a.ch, c)) { tstart = t0 - 1; mode = 2; }
                 else { tstart = max(0, t0 - (a.ch.warmv ? a.ch.warmv[c] : a.ch.warm)); mode = (tstart == 0) ? 0 : 1; }
             }
             d[C_C] = c; d[C_T0] = t0; d[C_TEND] = tend; d[C_T] = T; d[C_TSTART] = tstart;
@@ -2083,7 +2083,7 @@ __global__ void __launch_bounds__(512, 1) k_viterbi_chain_wide(const VitChainArg
             const int* const d = cd + 8 * r;
             steps = max(steps, d[C_TEND] - d[C_TFIRST]);
             if (d[C_MODE] == 2 && jv) {
-                const double x = a.hand_end[(long long)(d[C_C] - 1) * N + j];
+                const double x = chain_start_vec(a.ch, a.hand_end, d[C_C], d[C_C] - 1, N)[j];
                 vb[r * NPS + j] = x;
                 a.hand_used[(long long)d[C_C] * N + j] = x;
             }

@@ -13,6 +13,13 @@
 // pass, in parallel over chains.  k_scan_starts then walks the chains of each trajectory ONCE, composing the exact hand-over
 // vectors from the one exact end the normal pass produced (the first chain started from pi, the last from beta = 1/N), and
 // writes them where a pass with Chains.exact = 1 reads its starts.  N <= 32 here, 32 < N <= 128 in the wide variants below.
+//
+// Every kernel here is templated on the semiring SR.  SR_SUM is the sum-product of the E-step.  SR_MAX is the max-product of
+// Viterbi (_hidden.c:229-265): the recursion delta_t(j) = p_j max_i delta_{t-1}(i) A_ij, normalised to sum one per frame, is
+// linear in the max-times semiring, so the same operators, scan and composition carry over with the inner sum replaced by a
+// max.  Row normalisation, log-scales, the exp(L - Lmax) weights, rows that drop out and the outlier rule stay as they are
+// (every step is homogeneous in a positive scalar in both semirings).  The operators carry values only: back-pointers and the
+// first-maximum tie rule stay in the Viterbi chain kernels, which re-run from the exact starts.  SR_MAX runs forward only.
 #include <algorithm>
 
 #include "common.cuh"
@@ -22,7 +29,17 @@ namespace {
 
 constexpr unsigned FULLM = 0xffffffffu;
 
-template <int EM>
+// acc (+) a (x) b: a fused multiply-add in the sum-product semiring, max(acc, a b) in the max-product one (a compare and a
+// select: every value here is non-negative, and a NaN product is ignored as fmax would)
+template <int SR>
+__device__ __forceinline__ double sr_acc(double acc, double a, double b)
+{
+    if (SR == SR_SUM) return fma(a, b, acc);
+    const double h = a * b;
+    return h > acc ? h : acc;
+}
+
+template <int EM, int SR>
 __global__ void __launch_bounds__(1024) k_chain_operator(Chains ch, Emission em, const double* __restrict__ A, int N, int dir,
                                                          double* __restrict__ ops, double* __restrict__ lscale)
 {
@@ -56,7 +73,7 @@ __global__ void __launch_bounds__(1024) k_chain_operator(Chains ch, Emission em,
             double x = 0.0;
             for (int k = 0; k < N; ++k) {
                 const double mk = __shfl_sync(FULLM, m, k);
-                if (jv) x = fma(mk, As[k * N + j], x);
+                if (jv) x = sr_acc<SR>(x, mk, As[k * N + j]);
             }
             x *= p;
             double s = x;
@@ -80,6 +97,7 @@ __global__ void __launch_bounds__(1024) k_chain_operator(Chains ch, Emission em,
 // One block per run of contiguous chains (a trajectory, or its owned range on a time shard); thread j = state j.
 // forward : he[c] = normalise(he[c-1] . M_c) for the chains after the run's first;
 // backward: he[c] = normalise(B_c . he[c+1]) for the chains before the run's last.
+template <int SR>
 __global__ void k_scan_starts(Chains ch, int n_total, int N, int dir, const double* __restrict__ ops,
                               const double* __restrict__ lscale, double* __restrict__ he)
 {
@@ -103,7 +121,7 @@ __global__ void k_scan_starts(Chains ch, int n_total, int N, int dir, const doub
             __syncwarp();
             double x = 0.0;
             if (jv)
-                for (int i = 0; i < N; ++i) x = fma(wgt[i], ops[((long long)c * N + i) * N + j], x);
+                for (int i = 0; i < N; ++i) x = sr_acc<SR>(x, wgt[i], ops[((long long)c * N + i) * N + j]);
             double tot = x;
 #pragma unroll
             for (int off = 16; off > 0; off >>= 1) tot += __shfl_xor_sync(FULLM, tot, off);
@@ -120,7 +138,7 @@ __global__ void k_scan_starts(Chains ch, int n_total, int N, int dir, const doub
         for (int c = c0 - 1; c > 0 && follows(c, c + 1) && follows(c - 1, c); --c) {
             double x = 0.0;
             if (jv)
-                for (int k = 0; k < N; ++k) x = fma(ops[((long long)c * N + j) * N + k], s[k], x);
+                for (int k = 0; k < N; ++k) x = sr_acc<SR>(x, ops[((long long)c * N + j) * N + k], s[k]);
             const double L = jv ? lscale[(long long)c * N + j] : -INFINITY;
             double Lmax = (jv && x > 0.0) ? L : -INFINITY;
 #pragma unroll
@@ -139,14 +157,19 @@ __global__ void k_scan_starts(Chains ch, int n_total, int N, int dir, const doub
 }
 
 // ---- 32 < N <= 128 ------------------------------------------------------------------------------------------------
-// The same two kernels with NT = ceil(N / 32) columns per lane.  Operator: the 32 warps of a block take the rows i = w,
+// The same two kernels with NT = ceil(N / 32) columns per lane.  Operator: the 32 warps of a block (16 for SR_MAX) take the rows i = w,
 // w + 32, ... of the chain's operator one after the other (every row is its own vector recursion through the chain's frames;
 // the emission of a frame is re-evaluated per row: NT exponentials against N * NT multiply-adds); component k of the row
 // vector lives in lane k & 31, slot k >> 5, and is broadcast by one shuffle.  A is read through the cache (80 KB at N = 100:
 // every warp of the block walks the same rows of it).  N times the work of a vector pass, like the narrow kernel; this is
 // the fallback for models that do not forget, not a fast path.
-template <int EM, int NT>
-__global__ void __launch_bounds__(1024) k_chain_operator_wide(Chains ch, Emission em, const double* __restrict__ A, int N,
+// Warps per block of k_chain_operator_wide: the max-product step needs a register more per column than the fused multiply-add,
+// which spills at the 64 registers of a 1024-thread block (N > 64, Gaussian); half the warps give it 128.
+template <int SR>
+constexpr int op_wide_warps() { return SR == SR_SUM ? 32 : 16; }
+
+template <int EM, int NT, int SR>
+__global__ void __launch_bounds__(32 * op_wide_warps<SR>(), SR == SR_SUM ? 0 : 1) k_chain_operator_wide(Chains ch, Emission em, const double* __restrict__ A, int N,
                                                               int dir, double* __restrict__ ops, double* __restrict__ lscale)
 {
     const int c = blockIdx.x;
@@ -165,7 +188,7 @@ __global__ void __launch_bounds__(1024) k_chain_operator_wide(Chains ch, Emissio
         mu[q] = (EM == EM_GAUSS && jv[q]) ? em.mu[j] : 0.0;
         sg[q] = (EM == EM_GAUSS && jv[q]) ? em.sigma[j] : 1.0;
     }
-    for (int i = w; i < N; i += 32) {
+    for (int i = w; i < N; i += op_wide_warps<SR>()) {
         double m[NT];
 #pragma unroll
         for (int q = 0; q < NT; ++q) m[q] = (lane + 32 * q == i) ? 1.0 : 0.0;
@@ -203,7 +226,7 @@ __global__ void __launch_bounds__(1024) k_chain_operator_wide(Chains ch, Emissio
                     const double* Ak = A + (long long)k * N + lane;
 #pragma unroll
                     for (int q = 0; q < NT; ++q)
-                        if (jv[q]) x[q] = fma(mk, Ak[32 * q], x[q]);
+                        if (jv[q]) x[q] = sr_acc<SR>(x[q], mk, Ak[32 * q]);
                 }
                 double s = 0.0;
 #pragma unroll
@@ -248,7 +271,7 @@ __device__ __forceinline__ double scan_block_reduce(double v, double* red)
 }
 
 // One block of 32 NT threads per run of contiguous chains; thread j = state j (see k_scan_starts).
-template <int NT>
+template <int NT, int SR>
 __global__ void k_scan_starts_wide(Chains ch, int n_total, int N, int dir, const double* __restrict__ ops,
                                    const double* __restrict__ lscale, double* __restrict__ he)
 {
@@ -267,7 +290,7 @@ __global__ void k_scan_starts_wide(Chains ch, int n_total, int N, int dir, const
             __syncthreads();
             double x = 0.0;
             if (jv)
-                for (int i = 0; i < N; ++i) x = fma(wgt[i], ops[((long long)c * N + i) * N + j], x);
+                for (int i = 0; i < N; ++i) x = sr_acc<SR>(x, wgt[i], ops[((long long)c * N + i) * N + j]);
             const double tot = scan_block_reduce<NT, false>(x, red);       // (its barriers also fence the reads of wgt)
             if (!(tot > 0.0)) return;                       // degenerate: leave the remaining hand-overs to the fix-up passes
             s[j] = x / tot;
@@ -280,7 +303,7 @@ __global__ void k_scan_starts_wide(Chains ch, int n_total, int N, int dir, const
         for (int c = c0 - 1; c > 0 && follows(c, c + 1) && follows(c - 1, c); --c) {
             double x = 0.0;
             if (jv)
-                for (int k = 0; k < N; ++k) x = fma(ops[((long long)c * N + j) * N + k], s[k], x);
+                for (int k = 0; k < N; ++k) x = sr_acc<SR>(x, ops[((long long)c * N + j) * N + k], s[k]);
             const double L = jv ? lscale[(long long)c * N + j] : -INFINITY;
             const double Lmax = scan_block_reduce<NT, true>((jv && x > 0.0) ? L : -INFINITY, red);
             x = (jv && x > 0.0 && L > -INFINITY) ? x * exp(L - Lmax) : 0.0;
@@ -293,17 +316,17 @@ __global__ void k_scan_starts_wide(Chains ch, int n_total, int N, int dir, const
     }
 }
 
-template <int NT>
+template <int NT, int SR>
 int launch_exact_scan_wide(const Chains& ch, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
                            double* he, double* ops, double* lscale, cudaStream_t st)
 {
     switch (emkind) {
-        case EM_POBS: k_chain_operator_wide<EM_POBS, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-        case EM_GAUSS: k_chain_operator_wide<EM_GAUSS, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-        case EM_DISC: k_chain_operator_wide<EM_DISC, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        case EM_POBS: k_chain_operator_wide<EM_POBS, NT, SR><<<n_total, 32 * op_wide_warps<SR>(), 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        case EM_GAUSS: k_chain_operator_wide<EM_GAUSS, NT, SR><<<n_total, 32 * op_wide_warps<SR>(), 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        case EM_DISC: k_chain_operator_wide<EM_DISC, NT, SR><<<n_total, 32 * op_wide_warps<SR>(), 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
         default: return BHMM_ERR_INVALID;
     }
-    k_scan_starts_wide<NT><<<n_total, 32 * NT, 0, st>>>(ch, n_total, N, dir, ops, lscale, he);
+    k_scan_starts_wide<NT, SR><<<n_total, 32 * NT, 0, st>>>(ch, n_total, N, dir, ops, lscale, he);
     return BHMM_OK;
 }
 
@@ -313,7 +336,7 @@ int launch_exact_scan_wide(const Chains& ch, int n_total, const Emission& em, in
 // true operator = exp(L_i) m_i, m_i summing to one).  Warp w takes the rows i = w, w + 32, ...; component k of a row lives in
 // lane k & 31, slot k >> 5 (NT = 1: lane per column, N <= 32).  A warp reads row i of X and writes it back itself, so the
 // product is formed in place; Y is read through the cache.  Plain FP64 FMAs: this serves the fallback, not the fast path.
-template <int NT>
+template <int NT, int SR>
 __global__ void __launch_bounds__(1024) k_compose_operators(const int* __restrict__ pairs, int N, double* ops, double* lscale)
 {
     const int dst = pairs[2 * blockIdx.x], src = pairs[2 * blockIdx.x + 1];
@@ -351,7 +374,7 @@ __global__ void __launch_bounds__(1024) k_compose_operators(const int* __restric
             const double* Yk = Y + (long long)k * N + lane;
 #pragma unroll
             for (int q = 0; q < NT; ++q)
-                if (jv[q]) r[q] = fma(wk, Yk[32 * q], r[q]);
+                if (jv[q]) r[q] = sr_acc<SR>(r[q], wk, Yk[32 * q]);
         }
         double tot = 0.0;
 #pragma unroll
@@ -383,61 +406,95 @@ __global__ void k_operator_out(const int* __restrict__ first, int N, const doubl
     }
 }
 
-template <int NT>
+template <int NT, int SR>
 void launch_chain_operator_wide(const Chains& ch, int n_total, const Emission& em, int emkind, const double* dA, int N,
                                 int dir, double* ops, double* lscale, cudaStream_t st)
 {
     switch (emkind) {
-        case EM_POBS: k_chain_operator_wide<EM_POBS, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-        case EM_GAUSS: k_chain_operator_wide<EM_GAUSS, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-        default: k_chain_operator_wide<EM_DISC, NT><<<n_total, 1024, 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        case EM_POBS: k_chain_operator_wide<EM_POBS, NT, SR><<<n_total, 32 * op_wide_warps<SR>(), 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        case EM_GAUSS: k_chain_operator_wide<EM_GAUSS, NT, SR><<<n_total, 32 * op_wide_warps<SR>(), 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        default: k_chain_operator_wide<EM_DISC, NT, SR><<<n_total, 32 * op_wide_warps<SR>(), 0, st>>>(ch, em, dA, N, dir, ops, lscale); break;
     }
 }
 
-template <int NT>
+template <int NT, int SR>
 void launch_compose_level(const int* pairs, int n, int N, double* ops, double* lscale, cudaStream_t st)
 {
-    k_compose_operators<NT><<<n, 32 * std::min(N, 32), 0, st>>>(pairs, N, ops, lscale);
+    k_compose_operators<NT, SR><<<n, 32 * std::min(N, 32), 0, st>>>(pairs, N, ops, lscale);
+}
+
+template <int SR>
+void shard_operators_sr(const Chains& ch, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
+                        const int* d_pairs, const std::vector<int>& lev_n, const std::vector<long long>& lev_off, double* ops,
+                        double* lscale, cudaStream_t st)
+{
+    if (N > 32) {
+        switch ((N + 31) / 32) {
+            case 2: launch_chain_operator_wide<2, SR>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
+            case 3: launch_chain_operator_wide<3, SR>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
+            default: launch_chain_operator_wide<4, SR>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
+        }
+    } else {
+        const size_t smem = sizeof(double) * (size_t)N * N;
+        switch (emkind) {
+            case EM_POBS: k_chain_operator<EM_POBS, SR><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+            case EM_GAUSS: k_chain_operator<EM_GAUSS, SR><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+            default: k_chain_operator<EM_DISC, SR><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        }
+    }
+    for (size_t L = 0; L < lev_n.size(); ++L) {
+        const int* pairs = d_pairs + 2 * lev_off[L];
+        switch ((N + 31) / 32) {
+            case 1: launch_compose_level<1, SR>(pairs, lev_n[L], N, ops, lscale, st); break;
+            case 2: launch_compose_level<2, SR>(pairs, lev_n[L], N, ops, lscale, st); break;
+            case 3: launch_compose_level<3, SR>(pairs, lev_n[L], N, ops, lscale, st); break;
+            default: launch_compose_level<4, SR>(pairs, lev_n[L], N, ops, lscale, st); break;
+        }
+    }
+}
+
+template <int SR>
+int exact_scan_sr(const Chains& ch, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir, double* he,
+                  double* ops, double* lscale, cudaStream_t st)
+{
+    if (N > 32) {
+        switch ((N + 31) / 32) {
+            case 2: return launch_exact_scan_wide<2, SR>(ch, n_total, em, emkind, dA, N, dir, he, ops, lscale, st);
+            case 3: return launch_exact_scan_wide<3, SR>(ch, n_total, em, emkind, dA, N, dir, he, ops, lscale, st);
+            default: return launch_exact_scan_wide<4, SR>(ch, n_total, em, emkind, dA, N, dir, he, ops, lscale, st);
+        }
+    }
+    const int threads = 32 * N;
+    const size_t smem = sizeof(double) * (size_t)N * N;
+    switch (emkind) {
+        case EM_POBS: k_chain_operator<EM_POBS, SR><<<n_total, threads, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        case EM_GAUSS: k_chain_operator<EM_GAUSS, SR><<<n_total, threads, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        case EM_DISC: k_chain_operator<EM_DISC, SR><<<n_total, threads, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
+        default: return BHMM_ERR_INVALID;
+    }
+    k_scan_starts<SR><<<n_total, 32, 0, st>>>(ch, n_total, N, dir, ops, lscale, he);
+    return BHMM_OK;
 }
 
 }  // namespace
 
-// Operators of the owned frames of every trajectory of a time shard (bhmm_b200_shard_operators_*): the chains' operators,
-// then level after level of the reduction (lev_n[L] pairs at d_pairs + 2 lev_off[L]), then one (N, N + 1) block per
-// trajectory written to out (trajectory stride kstride doubles).
+// Operators of the owned frames of every trajectory of a time shard (bhmm_b200_shard_operators_*,
+// bhmm_b200_shard_viterbi_operators_*): the chains' operators in semiring sr, then level after level of the reduction
+// (lev_n[L] pairs at d_pairs + 2 lev_off[L]), then one (N, N + 1) block per trajectory written to out (trajectory stride
+// kstride doubles).
 int launch_shard_operators(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
-                           const int* d_pairs, const std::vector<int>& lev_n, const std::vector<long long>& lev_off,
+                           int sr, const int* d_pairs, const std::vector<int>& lev_n, const std::vector<long long>& lev_off,
                            const int* d_first, int K, double* ops, double* out, long long kstride, cudaStream_t st)
 {
     if (!exact_scan_ok(N)) return BHMM_ERR_UNSUPPORTED;
     if (emkind != EM_POBS && emkind != EM_GAUSS && emkind != EM_DISC) return BHMM_ERR_INVALID;
+    if (sr != SR_SUM && !(sr == SR_MAX && dir > 0)) return BHMM_ERR_INVALID;
     double* lscale = ops + (size_t)n_total * N * N;
     if (n_total > 0) {
         Chains ch = all;
         ch.list = nullptr; ch.n = n_total;
-        if (N > 32) {
-            switch ((N + 31) / 32) {
-                case 2: launch_chain_operator_wide<2>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
-                case 3: launch_chain_operator_wide<3>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
-                default: launch_chain_operator_wide<4>(ch, n_total, em, emkind, dA, N, dir, ops, lscale, st); break;
-            }
-        } else {
-            const size_t smem = sizeof(double) * (size_t)N * N;
-            switch (emkind) {
-                case EM_POBS: k_chain_operator<EM_POBS><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-                case EM_GAUSS: k_chain_operator<EM_GAUSS><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-                default: k_chain_operator<EM_DISC><<<n_total, 32 * N, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-            }
-        }
-        for (size_t L = 0; L < lev_n.size(); ++L) {
-            const int* pairs = d_pairs + 2 * lev_off[L];
-            switch ((N + 31) / 32) {
-                case 1: launch_compose_level<1>(pairs, lev_n[L], N, ops, lscale, st); break;
-                case 2: launch_compose_level<2>(pairs, lev_n[L], N, ops, lscale, st); break;
-                case 3: launch_compose_level<3>(pairs, lev_n[L], N, ops, lscale, st); break;
-                default: launch_compose_level<4>(pairs, lev_n[L], N, ops, lscale, st); break;
-            }
-        }
+        if (sr == SR_SUM) shard_operators_sr<SR_SUM>(ch, n_total, em, emkind, dA, N, dir, d_pairs, lev_n, lev_off, ops, lscale, st);
+        else shard_operators_sr<SR_MAX>(ch, n_total, em, emkind, dA, N, dir, d_pairs, lev_n, lev_off, ops, lscale, st);
     }
     k_operator_out<<<K, 256, 0, st>>>(d_first, N, ops, lscale, out, kstride);
     return BHMM_OK;
@@ -448,30 +505,17 @@ bool exact_scan_ok(int N) { return N >= 1 && N <= 128; }
 size_t exact_scan_bytes(int n_chains, int N) { return sizeof(double) * (size_t)n_chains * N * (N + 1); }
 
 // ops: device scratch of exact_scan_bytes(n_total, N).  On return he (= w.he_f or w.he_b) holds exact hand-over vectors for
-// every chain whose run started from an exact end; run the chains with Chains.exact = 1 next.
-int launch_exact_scan(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir,
+// every chain whose run started from an exact end; run the chains with Chains.exact = 1 next.  sr = SR_MAX (Viterbi) runs
+// forward only.
+int launch_exact_scan(const Chains& all, int n_total, const Emission& em, int emkind, const double* dA, int N, int dir, int sr,
                       double* he, double* ops, cudaStream_t st)
 {
     if (!exact_scan_ok(N)) return BHMM_ERR_UNSUPPORTED;
+    if (sr != SR_SUM && !(sr == SR_MAX && dir > 0)) return BHMM_ERR_INVALID;
     if (n_total <= 0) return BHMM_OK;
     double* lscale = ops + (size_t)n_total * N * N;
     Chains ch = all;
     ch.list = nullptr; ch.n = n_total;
-    if (N > 32) {
-        switch ((N + 31) / 32) {
-            case 2: return launch_exact_scan_wide<2>(ch, n_total, em, emkind, dA, N, dir, he, ops, lscale, st);
-            case 3: return launch_exact_scan_wide<3>(ch, n_total, em, emkind, dA, N, dir, he, ops, lscale, st);
-            default: return launch_exact_scan_wide<4>(ch, n_total, em, emkind, dA, N, dir, he, ops, lscale, st);
-        }
-    }
-    const int threads = 32 * N;
-    const size_t smem = sizeof(double) * (size_t)N * N;
-    switch (emkind) {
-        case EM_POBS: k_chain_operator<EM_POBS><<<n_total, threads, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-        case EM_GAUSS: k_chain_operator<EM_GAUSS><<<n_total, threads, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-        case EM_DISC: k_chain_operator<EM_DISC><<<n_total, threads, smem, st>>>(ch, em, dA, N, dir, ops, lscale); break;
-        default: return BHMM_ERR_INVALID;
-    }
-    k_scan_starts<<<n_total, 32, 0, st>>>(ch, n_total, N, dir, ops, lscale, he);
-    return BHMM_OK;
+    return sr == SR_SUM ? exact_scan_sr<SR_SUM>(ch, n_total, em, emkind, dA, N, dir, he, ops, lscale, st)
+                        : exact_scan_sr<SR_MAX>(ch, n_total, em, emkind, dA, N, dir, he, ops, lscale, st);
 }

@@ -299,8 +299,15 @@ class TrajectoryBatch(object):
 
     @property
     def exact_scans(self):
-        """How often the exact transfer-operator scan replaced the warm-up starts (models that do not forget; N <= 32)."""
+        """How often the exact transfer-operator scan replaced the warm-up starts, in the E-step and in Viterbi (models that
+        do not forget; N <= 128)."""
         return int(lib.bhmm_b200_batch_scan_count(self._handle))
+
+    @property
+    def viterbi_sequential_fallbacks(self):
+        """How often a chain-parallel Viterbi map was replaced by the sequential kernel (hand-overs not certified, or a flagged
+        near-tie on the path)."""
+        return int(lib.bhmm_b200_batch_viterbi_sequential_count(self._handle))
 
     @property
     def uses_lane_kernels(self):
@@ -849,28 +856,31 @@ def compose_shard_maps(maps_by_rank, owns_by_rank):
     return enter
 
 
-def _apply_operator(v, op, forward):
+def _apply_operator(v, op, forward, semiring='sum'):
     """One shard's operator on a border vector (a host function): ``op`` (N, N + 1) = [row-normalised operator | log-scale of
-    every row] as bhmm_b200_shard_operators_* write it.  forward: the row vector v . M, backward: the column vector M . v.
-    The log-scales only weigh the rows against each other; the result is normalised to sum one."""
+    every row] as bhmm_b200_shard_operators_* (semiring 'sum') or bhmm_b200_shard_viterbi_operators_* ('max', forward only)
+    write it.  forward: the row vector v . M, backward: the column vector M . v; in the max-times semiring the row vector has
+    x_j = max_i v_i M_ij.  The log-scales only weigh the rows against each other; the result is normalised to sum one."""
     M, L = op[:, :-1], op[:, -1]
+    what = 'Viterbi' if semiring == 'max' else 'E-step'
     if forward:
         live = (v > 0) & np.isfinite(L)
         if not live.any():
-            raise RuntimeError('time-sharded E-step: the exact border vector vanished (the model gives the data zero probability)')
+            raise RuntimeError('time-sharded %s: the exact border vector vanished (the model gives the data zero probability)' % what)
         w = np.where(live, v * np.exp(np.where(live, L - L[live].max(), -np.inf)), 0.0)
-        x = w @ M
+        x = (w[:, None] * M).max(axis=0) if semiring == 'max' else w @ M
     else:
         x = M @ v
         live = (x > 0) & np.isfinite(L)
         if not live.any():
-            raise RuntimeError('time-sharded E-step: the exact border vector vanished (the model gives the data zero probability)')
+            raise RuntimeError('time-sharded %s: the exact border vector vanished (the model gives the data zero probability)' % what)
         x = np.where(live, x * np.exp(np.where(live, L - L[live].max(), -np.inf)), 0.0)
     return x / x.sum()
 
 
-def compose_shard_operators(ops_by_rank, borders_by_rank, owns_by_rank):
-    """Exact border vectors of an E-step on time shards, from all shards' operators (a host function; no device).
+def compose_shard_operators(ops_by_rank, borders_by_rank, owns_by_rank, semiring='sum'):
+    """Exact border vectors of an E-step (or, semiring='max', of Viterbi) on time shards, from all shards' operators (a host
+    function; no device).
 
     ``ops_by_rank[r]``: (K, 2, N, N + 1), shard r's forward and backward operators of its owned frames
     (``TimeShardedTrajectories.shard_operators``); ``borders_by_rank[r]``: (K, 4, N), its border vectors
@@ -879,9 +889,14 @@ def compose_shard_operators(ops_by_rank, borders_by_rank, owns_by_rank):
     through the operators of the following owners; backward: the last owner's beta at its first owned frame ([3]) right to
     left.  Shards that own nothing of a trajectory pass the vector through.  Returns (fwd, bwd), each (world, K, N): the exact
     alpha at lo - 1 and beta at hi of every shard, normalised to sum one; zero rows where a shard owns nothing of the
-    trajectory, holds its start (fwd) or holds its end (bwd)."""
+    trajectory, holds its start (fwd) or holds its end (bwd).
+
+    semiring='max' (Viterbi, forward only): ``ops_by_rank[r]`` is (K, N, N + 1), shard r's max-product operators
+    (``TimeShardedTrajectories.viterbi_operators``), and ``borders_by_rank[r]`` (K, 2, N) the border vectors of its Viterbi
+    batch ([1]: the normalised max-product vector at its last owned frame).  Returns fwd alone: the exact vector at lo - 1."""
     world = len(ops_by_rank)
-    K, _, N, _ = np.shape(ops_by_rank[0])
+    viterbi = semiring == 'max'
+    K, N = np.shape(ops_by_rank[0])[0], np.shape(ops_by_rank[0])[-2]
     fwd, bwd = np.zeros((world, K, N)), np.zeros((world, K, N))
     for k in range(K):
         owners = [r for r in range(world) if owns_by_rank[r][k]]
@@ -891,13 +906,16 @@ def compose_shard_operators(ops_by_rank, borders_by_rank, owns_by_rank):
         v = v / v.sum()
         for r in owners[1:]:
             fwd[r, k] = v
-            v = _apply_operator(v, np.asarray(ops_by_rank[r][k][0], dtype=np.float64), True)
+            op = ops_by_rank[r][k] if viterbi else ops_by_rank[r][k][0]
+            v = _apply_operator(v, np.asarray(op, dtype=np.float64), True, semiring)
+        if viterbi:
+            continue
         v = np.asarray(borders_by_rank[owners[-1]][k][3], dtype=np.float64)
         v = v / v.sum()
         for r in owners[-2::-1]:
             bwd[r, k] = v
             v = _apply_operator(v, np.asarray(ops_by_rank[r][k][1], dtype=np.float64), False)
-    return fwd, bwd
+    return fwd if viterbi else (fwd, bwd)
 
 
 class TimeShardedTrajectories(object):
@@ -927,7 +945,14 @@ class TimeShardedTrajectories(object):
     its range; the vector each shard started from is certified against the one its left neighbour computed (same
     component-wise relative test as for the E-step); then the paths are resolved from the last shard to the first, each
     shard handing the state at its neighbour's last frame -- one integer per trajectory -- to the left.  A path that goes
-    through a decision whose margin is below the certified tolerance raises (run that trajectory on one device).
+    through a decision whose margin is below the certified tolerance raises (run that trajectory on one device).  With
+    ``exact_borders=True`` a border that fails the certification (N <= 128) does not raise: every shard reduces its owned
+    frames to a max-product transfer operator (``viterbi_operators``: about N Viterbi passes), one ``all_gather`` exchanges
+    them with each shard's chain count and worst in-shard mismatch, every shard composes the exact max-product vector at
+    its first owned frame (``compose_shard_operators(..., semiring='max')``) and builds its map again from it, with the
+    near-tie margin widened to the deviation that start can carry (``viterbi_margins``); the borders are certified again (a
+    second failure raises) and the paths resolved as before.  ``viterbi_fallbacks`` counts these.  The default keeps
+    raising on a halo that is too short.
 
     Gibbs sweeps work across shards too (``gibbs_gaussian`` / ``gibbs_discrete``, ``BayesianHMMSampler(shard='time')``).
     Given the uniforms, the draw at frame t is a function s_t = F_t(s_{t+1}) of the next state only, so every shard runs the
@@ -969,6 +994,7 @@ class TimeShardedTrajectories(object):
         self.batch = TrajectoryBatch.from_concatenated(cat, lengths, self.N, device=device, chunk=chunk, warm=warm,
                                                        own_ranges=own)
         self.K = len(lengths)
+        self.viterbi_fallbacks = 0                       # Viterbi calls that needed the exact border exchange
 
     def release_estep_workspace(self):
         """Free the E-step batch's device workspace (forward variables, chain tables); the observations stay resident for
@@ -994,6 +1020,7 @@ class TimeShardedTrajectories(object):
         self.batch = TrajectoryBatch.from_concatenated(piece, [n], self.N, device=device, chunk=chunk, warm=warm,
                                                        own_ranges=[(lo - start, hi - start)])
         self.K = 1
+        self.viterbi_fallbacks = 0
         return self
 
     def close(self):
@@ -1071,25 +1098,190 @@ class TimeShardedTrajectories(object):
         return paths
 
     @staticmethod
-    def certify_viterbi(borders_by_rank, ranges_by_rank, tol, what='Viterbi'):
-        """Worst relative mismatch of the max-product (or, for the Gibbs sweep, forward) hand-overs at the shard borders:
-        the vector each shard started from against the one its left neighbour computed; raises above ``tol``."""
+    def viterbi_mismatch(borders_by_rank, ranges_by_rank, floor=0.0):
+        """Worst relative mismatch of the max-product (or forward) hand-overs at the shard borders, without raising:
+        the vector each shard started from against the one its left neighbour computed."""
         world, worst = len(borders_by_rank), 0.0
         for k in range(len(ranges_by_rank[0])):
             owners = [r for r in range(world) if ranges_by_rank[r][k][1] > ranges_by_rank[r][k][0]]
             for left, right in zip(owners, owners[1:]):
-                worst = max(worst, _rel_mismatch(borders_by_rank[right][k][0], borders_by_rank[left][k][1]))
+                worst = max(worst, _rel_mismatch(borders_by_rank[right][k][0], borders_by_rank[left][k][1], floor))
+        return worst
+
+    @staticmethod
+    def certify_viterbi(borders_by_rank, ranges_by_rank, tol, what='Viterbi'):
+        """Worst relative mismatch of the max-product (or, for the Gibbs sweep, forward) hand-overs at the shard borders:
+        the vector each shard started from against the one its left neighbour computed; raises above ``tol``."""
+        worst = TimeShardedTrajectories.viterbi_mismatch(borders_by_rank, ranges_by_rank)
         if worst > tol:
             raise RuntimeError('time-sharded %s: a shard border disagrees by %.3g (tolerance %.3g); the halo is too '
                                'short for this model -- increase halo=' % (what, worst, tol))
         return worst
 
+    # ------------------------------------------------------------------------------------------ Viterbi with exact borders
+    # Near-tie margin factor of a pass from exact starts, c in c B (csrc/engine.cu: VIT_SCAN_C; DESIGN.md section 3)
+    VITERBI_MARGIN_C = 2.5
+    # mismatch per border assumed for the margin of the pass from exact starts before it is measured
+    VITERBI_BORDER_GUESS = 1e-12
+
+    def viterbi_operators(self, model, kind='gaussian'):
+        """Max-product transfer operators of this shard's owned frames on its Viterbi batch: a (K, N, N + 1) float64 device
+        tensor, row i = [operator row i normalised to sum one | log of its scale] (bhmm_b200_shard_viterbi_operators_*).
+        N <= 128."""
+        vb = self._viterbi_batch()
+        out = vb.torch.empty((self.K, self.N, self.N + 1), dtype=vb.torch.float64, device=vb.device)
+        with vb.torch.cuda.device(vb.device):
+            if kind == 'gaussian':
+                A, pi, means, sigmas, io = model
+                if vb.discrete:
+                    raise TypeError('this batch holds integer symbols; a Gaussian output model needs float observations')
+                A_, pi_, m_, s_ = f64(A), f64(pi), f64(means), f64(sigmas)
+                rc = lib.bhmm_b200_shard_viterbi_operators_gaussian(vb._handle, C.c_void_p(vb.obs.data_ptr()), dptr(A_),
+                                                                    dptr(pi_), dptr(m_), dptr(s_), int(bool(io)),
+                                                                    C.c_void_p(out.data_ptr()), vb._stream())
+            else:
+                A, pi, B, io = model
+                A_, pi_, B_ = f64(A), f64(pi), f64(B)
+                vb._require_discrete(B_.shape[1])
+                rc = lib.bhmm_b200_shard_viterbi_operators_discrete(vb._handle, C.c_void_p(vb.obs.data_ptr()), dptr(A_),
+                                                                    dptr(pi_), dptr(B_), B_.shape[1], int(bool(io)),
+                                                                    C.c_void_p(out.data_ptr()), vb._stream())
+        check(rc)
+        return out
+
+    def set_viterbi_starts(self, fwd, margin=0.0):
+        """Start the next Viterbi maps from exact border vectors (this shard's rows of ``compose_shard_operators(...,
+        semiring='max')``): trajectory k's first owned chain at lo - 1 where this shard owns frames of it but not its start,
+        with the relative near-tie margin widened to at least ``margin`` (0: the default).  ``clear_viterbi_starts`` returns to
+        the halo warm-up.  A margin of 1 or more cannot be honoured (ValueError): ``viterbi_margins``' callers refuse such a
+        bound before they get here."""
+        if not 0.0 <= margin < 1.0:
+            raise ValueError('time-sharded Viterbi: near-tie margin %.3g outside [0, 1)' % margin)
+        vb = self._viterbi_batch()
+        for k, (lo, hi, T) in enumerate(self.global_ranges):
+            f = np.ascontiguousarray(fwd[k], dtype=np.float64) if 0 < lo < hi else None
+            check(lib.bhmm_b200_batch_set_border_starts(vb._handle, k, dptr(f) if f is not None else None, None))
+        check(lib.bhmm_b200_batch_set_viterbi_margin(vb._handle, float(margin)))
+
+    def clear_viterbi_starts(self):
+        vb = self._viterbi_batch()
+        for k in range(self.K):
+            check(lib.bhmm_b200_batch_set_border_starts(vb._handle, k, None, None))
+        check(lib.bhmm_b200_batch_set_viterbi_margin(vb._handle, 0.0))
+
+    def _viterbi_terms(self):
+        """(chains, worst in-shard hand-over mismatch) of this shard's last Viterbi map -- its share of the margin bound --
+        and the first trajectory whose exact start it could not take (-1: none): one that it owns frames of, but not the
+        start of, with no halo frame before its owned range (the start is the vector at the frame before it)."""
+        vb = self._viterbi_batch()
+        info = vb.info()
+        missing = -1
+        for k, (lo, hi, T) in enumerate(self.global_ranges):
+            if 0 < lo < hi and vb._own_ranges[k][0] == 0:
+                missing = k
+                break
+        return np.array([float(info['chains']), float(info['worst_fwd']), float(missing)])
+
+    @staticmethod
+    def _viterbi_check_exchange(terms_by_rank, margins):
+        """Raises (RuntimeError, on every rank alike: the arguments are gathered data) where the exact Viterbi fallback cannot
+        go on: a shard lacks the halo frame before its owned range, or a near-tie margin would reach 1 (every decision would be
+        flagged: the path cannot be certified)."""
+        for r, t in enumerate(terms_by_rank):
+            if t[2] >= 0:
+                raise RuntimeError('time-sharded Viterbi: the exact border fallback starts a shard at the frame before its owned '
+                                   'range; rank %d holds no halo frame there for trajectory %d' % (r, int(t[2])))
+        if np.max(margins) >= 1.0:
+            raise RuntimeError('time-sharded Viterbi: the deviation bound of the exact border starts (near-tie margin %.3g) '
+                               'is too wide to certify any decision' % np.max(margins))
+
     @classmethod
-    def viterbi_combine(cls, shards, model, kind='gaussian'):
+    def viterbi_margins(cls, terms_by_rank, borders_by_rank, ranges_by_rank):
+        """Near-tie margin of every shard's Viterbi map from exact border starts: c B, where B bounds how far the start of the
+        shard's first owned chain lies from the sequential max-product vector (Hilbert's projective metric, DESIGN.md
+        section 3): for every owner of the trajectory before it, its chains x its worst in-shard mismatch (what its own end
+        carries) plus the mismatch at the border it hands over (``borders_by_rank`` None: VITERBI_BORDER_GUESS, before that
+        pass has run); the largest over the trajectories.  ``terms_by_rank[r]`` = (chains, worst mismatch) of shard r."""
+        world = len(terms_by_rank)
+        out = np.zeros(world)
+        for k in range(len(ranges_by_rank[0])):
+            owners = [r for r in range(world) if ranges_by_rank[r][k][1] > ranges_by_rank[r][k][0]]
+            B = 0.0
+            for left, right in zip(owners, owners[1:]):
+                chains, worst = terms_by_rank[left][0], terms_by_rank[left][1]      # (a third term is ignored)
+                m = cls.VITERBI_BORDER_GUESS if borders_by_rank is None else _rel_mismatch(
+                    borders_by_rank[right][k][0], borders_by_rank[left][k][1], cls.EXACT_BORDER_FLOOR)
+                B += chains * worst + m
+                out[right] = max(out[right], cls.VITERBI_MARGIN_C * B)
+        return out
+
+    @classmethod
+    def viterbi_operator_exchange(cls, ops, terms, borders_by_rank, lengths, rank, world, device):
+        """The exchange of the exact Viterbi fallback: ONE all_gather of this shard's (K, N, N + 1) max-product operators and
+        its terms (``_viterbi_terms``), then the composition of all shards' operators with the (K, 2, N) border vectors
+        gathered before.  ``lengths``: the K trajectory lengths.  Returns (this shard's exact (K, N) starts at lo - 1, the
+        near-tie margin of its pass from them); raises on every rank where the fallback cannot go on
+        (``_viterbi_check_exchange``)."""
+        K, N = np.shape(ops)[0], np.shape(ops)[1]
+        nt = len(terms)
+        got = cls.all_gather_host(np.concatenate([np.asarray(ops, dtype=np.float64).reshape(-1), terms]), world, device)
+        ranges = [[((T * r) // world, (T * (r + 1)) // world, T) for T in lengths] for r in range(world)]
+        owns = [[g[1] > g[0] for g in rg] for rg in ranges]
+        terms_all = [g[-nt:] for g in got]
+        margins = cls.viterbi_margins(terms_all, None, ranges)
+        cls._viterbi_check_exchange(terms_all, margins)
+        fwd = compose_shard_operators([g[:-nt].reshape(K, N, N + 1) for g in got], borders_by_rank, owns, semiring='max')
+        return fwd[rank], margins[rank]
+
+    def _viterbi_exact_unsupported(self, worst):
+        if self.N > 128:
+            return RuntimeError('time-sharded Viterbi: a shard border disagrees by %.3g (tolerance %.3g) and the exact '
+                                'fallback supports N <= 128 -- increase halo=' % (worst, self.tol))
+        return None
+
+    def _viterbi_certify_exact(self, borders_by_rank, ranges_by_rank):
+        worst = self.viterbi_mismatch(borders_by_rank, ranges_by_rank, self.EXACT_BORDER_FLOOR)
+        if worst > self.tol:
+            raise RuntimeError('time-sharded Viterbi: a shard border disagrees by %.3g (tolerance %.3g) after the exact '
+                               'border exchange' % (worst, self.tol))
+        return worst
+
+    @classmethod
+    def viterbi_combine(cls, shards, model, kind='gaussian', exact_borders=False):
         """Single-process use (tests): all shards in one process.  Returns (list over trajectories of the full int32 paths,
-        worst border mismatch)."""
+        worst border mismatch).  ``exact_borders``: the exact fallback of ``viterbi`` instead of raising on a border that
+        does not certify."""
         borders = [s.viterbi_map(model, kind) for s in shards]
-        worst = cls.certify_viterbi(borders, [s.global_ranges for s in shards], shards[0].tol)
+        ranges = [s.global_ranges for s in shards]
+        worst = cls.viterbi_mismatch(borders, ranges)
+        if worst > shards[0].tol and exact_borders and shards[0]._viterbi_exact_unsupported(worst) is None:
+            ops = [s.viterbi_operators(model, kind).cpu().numpy() for s in shards]
+            terms = [s._viterbi_terms() for s in shards]
+            owns = [[g[1] > g[0] for g in rg] for rg in ranges]
+            margin0 = cls.viterbi_margins(terms, None, ranges)
+            cls._viterbi_check_exchange(terms, margin0)
+            fwd = compose_shard_operators(ops, borders, owns, semiring='max')
+            try:
+                for r, s in enumerate(shards):
+                    s.set_viterbi_starts(fwd[r], margin0[r])
+                borders = [s.viterbi_map(model, kind) for s in shards]
+                worst = shards[0]._viterbi_certify_exact(borders, ranges)
+                terms = [s._viterbi_terms() for s in shards]
+                margin = cls.viterbi_margins(terms, borders, ranges)
+                cls._viterbi_check_exchange(terms, margin)
+                for r, s in enumerate(shards):
+                    if margin[r] > margin0[r]:          # the same starts again, flagged at the measured bound
+                        s.set_viterbi_starts(fwd[r], margin[r])
+                        s.viterbi_map(model, kind)
+            finally:
+                for s in shards:
+                    s.clear_viterbi_starts()
+            for s in shards:
+                s.viterbi_fallbacks += 1
+        else:
+            if worst > shards[0].tol and exact_borders:
+                raise shards[0]._viterbi_exact_unsupported(worst)
+            worst = cls.certify_viterbi(borders, ranges, shards[0].tol)
         K = shards[0].K
         parts = [[None] * len(shards) for _ in range(K)]
         end = None
@@ -1103,9 +1295,10 @@ class TimeShardedTrajectories(object):
             end = [left[k] if own[k] else (-1 if end is None else end[k]) for k in range(K)]
         return [np.concatenate(parts[k]) for k in range(K)], worst
 
-    def viterbi(self, model, kind='gaussian'):
+    def viterbi(self, model, kind='gaussian', exact_borders=False):
         """Distributed use (one process per shard, torch.distributed initialised).  Returns (owned-range paths of this
-        shard, worst border mismatch)."""
+        shard, worst border mismatch).  ``exact_borders``: where a border does not certify, the exact fallback (class
+        docstring) instead of raising."""
         import torch.distributed as td
         torch = self.batch.torch
         dev = self.batch.device
@@ -1114,7 +1307,35 @@ class TimeShardedTrajectories(object):
         td.all_gather(gathered, mine)
         ranges = [[((T * r) // self.world, (T * (r + 1)) // self.world, T) for (_, _, T) in self.global_ranges]
                   for r in range(self.world)]
-        worst = self.certify_viterbi([g.cpu().numpy() for g in gathered], ranges, self.tol)
+        borders = [g.cpu().numpy() for g in gathered]
+        worst = self.viterbi_mismatch(borders, ranges)
+        if worst > self.tol and exact_borders:
+            err = self._viterbi_exact_unsupported(worst)
+            if err is not None:
+                raise err
+            K, N = self.K, self.N
+            fwd, margin0 = self.viterbi_operator_exchange(self.viterbi_operators(model, kind).cpu().numpy(),
+                                                          self._viterbi_terms(), borders,
+                                                          [T for (_, _, T) in self.global_ranges], self.rank, self.world,
+                                                          self.batch.device)
+            try:
+                self.set_viterbi_starts(fwd, margin0)
+                mine = self.viterbi_map(model, kind)
+                terms = self._viterbi_terms()
+                got = self._all_gather(np.concatenate([mine.reshape(-1), terms]))
+                borders = [g[:-len(terms)].reshape(K, 2, N) for g in got]
+                worst = self._viterbi_certify_exact(borders, ranges)
+                margins = self.viterbi_margins([g[-len(terms):] for g in got], borders, ranges)
+                self._viterbi_check_exchange([g[-len(terms):] for g in got], margins)
+                margin = margins[self.rank]
+                if margin > margin0:                    # the same starts again, flagged at the measured bound
+                    self.set_viterbi_starts(fwd, margin)
+                    self.viterbi_map(model, kind)
+            finally:
+                self.clear_viterbi_starts()
+            self.viterbi_fallbacks += 1
+        else:
+            worst = self.certify_viterbi(borders, ranges, self.tol)
         end = torch.full((self.K,), -1, dtype=torch.int64, device=dev)
         for r in range(self.world - 1, -1, -1):
             if r == self.rank:
@@ -1125,11 +1346,11 @@ class TimeShardedTrajectories(object):
             td.broadcast(end, src=r)
         return self.viterbi_paths(), worst              # all shards copy their paths to the host at the same time
 
-    def viterbi_gaussian(self, A, pi, means, sigmas, ignore_outliers=True):
-        return self.viterbi((A, pi, means, sigmas, ignore_outliers), 'gaussian')
+    def viterbi_gaussian(self, A, pi, means, sigmas, ignore_outliers=True, exact_borders=False):
+        return self.viterbi((A, pi, means, sigmas, ignore_outliers), 'gaussian', exact_borders)
 
-    def viterbi_discrete(self, A, pi, B, ignore_outliers=False):
-        return self.viterbi((A, pi, B, ignore_outliers), 'discrete')
+    def viterbi_discrete(self, A, pi, B, ignore_outliers=False, exact_borders=False):
+        return self.viterbi((A, pi, B, ignore_outliers), 'discrete', exact_borders)
 
     # ------------------------------------------------------------------------------------------ Gibbs sweeps across shards
     def _gibbs_batch(self):

@@ -38,10 +38,13 @@ class MaximumLikelihoodEstimator(object):
     ``border_fallbacks`` counts the iterations that needed it.  The M-step is unchanged.  ``fit()`` ends with Viterbi across
     the shards, and ``hidden_state_trajectories`` holds this rank's owned pieces of the paths; where time-sharded Viterbi is
     not available (N > 128) or its borders do not certify, they stay None and a warning is logged.
+    ``exact_viterbi_borders=True`` gives that Viterbi the exact border fallback (``TimeShardedTrajectories.viterbi``, about N
+    Viterbi passes) where a border does not certify, instead of leaving the paths at None.
     """
 
     def __init__(self, observations, nstates, initial_model=None, output='gaussian', reversible=True, stationary=False,
-                 p=None, accuracy=1e-3, maxit=1000, maxit_P=100000, chunk=0, warm=0, shard=True, device_mstep=True, batch=None):
+                 p=None, accuracy=1e-3, maxit=1000, maxit_P=100000, chunk=0, warm=0, shard=True, device_mstep=True, batch=None,
+                 exact_viterbi_borders=False):
         if initial_model is None:
             raise NotImplementedError('bhmm_b200 needs initial_model= (bhmm.init_hmm is outside the hot path)')
         self._nstates = nstates
@@ -57,6 +60,7 @@ class MaximumLikelihoodEstimator(object):
             self._all_lengths = [len(o) for o in observations]
         self._nobs_total = len(self._all_lengths)
         self.border_fallbacks = 0       # E-steps on time shards that needed the exact border exchange
+        self._exact_viterbi_borders = bool(exact_viterbi_borders)
         # trajectories of this rank
         dist.tune_for_world()
         if self._time_sharded:
@@ -192,9 +196,10 @@ class MaximumLikelihoodEstimator(object):
             return None
         try:
             if self._batch.world == 1:
-                paths, _ = TimeShardedTrajectories.viterbi_combine([self._batch], self._model_tuple(), self._output)
+                paths, _ = TimeShardedTrajectories.viterbi_combine([self._batch], self._model_tuple(), self._output,
+                                                                   exact_borders=self._exact_viterbi_borders)
             else:
-                paths, _ = self._batch.viterbi(self._model_tuple(), self._output)
+                paths, _ = self._batch.viterbi(self._model_tuple(), self._output, exact_borders=self._exact_viterbi_borders)
         except RuntimeError as e:
             logger().warning('time-sharded Viterbi failed (%s); hidden_state_trajectories left at None' % e)
             return None

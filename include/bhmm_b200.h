@@ -180,8 +180,13 @@ int bhmm_b200_batch_uses_lane_kernels(const bhmm_b200_batch* b);
  * of it so that no round of the persistent kernels runs mostly empty. */
 int bhmm_b200_wave_chains(int N);
 /* How many times the exact transfer-operator scan (scan_kernels.cu) replaced the certified warm-up starts of this batch's
- * chains since it was created: the fallback for models whose filter does not forget its start (N <= 32). */
+ * chains since it was created, in the E-step (sum-product) and in Viterbi (max-product): the fallback for models whose
+ * filter does not forget its start (N <= 128; BHMM_B200_EXACT_SCAN=0 turns it off). */
 double bhmm_b200_batch_scan_count(const bhmm_b200_batch* b);
+/* How many times a chain-parallel Viterbi map of this batch was replaced by the sequential kernel since it was created: its
+ * hand-overs did not certify, or its path went through a flagged near-tie.  Batches whose plan has no chains run the
+ * sequential kernel by design and are not counted. */
+double bhmm_b200_batch_viterbi_sequential_count(const bhmm_b200_batch* b);
 /* Diagnostic: the hand-over vectors of the last pass, (chains, N) doubles each (host buffers): the vector every chain was
  * started from and the vector it computed at its own border; dir > 0 forward, dir < 0 backward. */
 int bhmm_b200_batch_debug_handovers(const bhmm_b200_batch* b, int dir, double* used, double* end);
@@ -239,6 +244,30 @@ int bhmm_b200_viterbi_discrete(bhmm_b200_batch* b, const int* d_obs, const doubl
  * the near-tie flags take ceil(N / 32) words per frame, and a Viterbi-only shard sizes its chains to that kernel's wave. */
 int bhmm_b200_batch_set_viterbi_phase(bhmm_b200_batch* b, int phase);
 int bhmm_b200_batch_set_viterbi_end_state(bhmm_b200_batch* b, int k, int state);
+/* Exact Viterbi hand-overs for models whose max-product vector does not forget its start within the warm-up.
+ * Inside a batch: when the chains' warm-up starts fail the certification and the first repair sweep does not clear them, the
+ * chain-parallel pass (N <= 128) takes its starts from a max-product transfer-operator scan, like the E-step, and counts it in
+ * bhmm_b200_batch_scan_count.  A decision is then flagged below the relative margin max(1e-11, c B), c = 2.5 and B = (chains
+ * of the longest trajectory) x (largest hand-over mismatch of the pass); the pass is redone with that margin when it had
+ * flagged at a smaller one.  An on-path flag falls back to the sequential kernel (whole trajectories) or returns
+ * BHMM_B200_ERR_NOT_CERTIFIED (time shard), as before.
+ * Across time shards: bhmm_b200_shard_viterbi_operators_* write to d_out (K, N, N + 1) doubles (device) the max-product
+ * operator of the owned frames of every trajectory, M_k = prod_t (A D_t) in the max-times semiring, as [row i of M_k
+ * normalised to sum one | log of its scale], the identity with zero log-scales where the shard owns no frame of trajectory k.
+ * N > 128 returns BHMM_B200_ERR_UNSUPPORTED, a batch without owned ranges BHMM_B200_ERR_INVALID.  About N times the work of a
+ * Viterbi pass.  The caller gathers all shards' operators with their border vectors (bhmm_b200_batch_border_handovers row 1:
+ * the normalised max-product vector at the last owned frame), composes the exact vector at own_lo - 1 of every shard from the
+ * first owner's row 1 left to right (engine.compose_shard_operators with semiring='max'), and hands it to the shard with
+ * bhmm_b200_batch_set_border_starts(b, k, fwd, NULL): the next phase 1 starts the first owned chain from it instead of the
+ * halo warm-up.  bhmm_b200_batch_set_viterbi_margin sets the relative near-tie margin of the shard's next passes to at least
+ * `margin` (0 = the default; [0, 1), else BHMM_B200_ERR_INVALID): the caller's c B for the deviation that the exact start
+ * carries from the shards before it, which only the caller knows; the in-shard term above is added to it. */
+int bhmm_b200_shard_viterbi_operators_gaussian(bhmm_b200_batch* b, const double* d_obs, const double* A, const double* pi,
+                                               const double* means, const double* sigmas, int ignore_outliers, double* d_out,
+                                               void* stream);
+int bhmm_b200_shard_viterbi_operators_discrete(bhmm_b200_batch* b, const int* d_obs, const double* A, const double* pi,
+                                               const double* B, int M, int ignore_outliers, double* d_out, void* stream);
+int bhmm_b200_batch_set_viterbi_margin(bhmm_b200_batch* b, double margin);
 /* One Gibbs hidden-path sweep (bayesian_sampling.py:283-331): emission + forward + backward sampling of every
  * trajectory, then the path statistics of generic_hmm.py:297-334,398-431.  Uniforms: d_u (device, one per row,
  * u[row] is the draw of that frame) or, when d_u is NULL, device Philox4x32-10 keyed by (seed, sweep).
