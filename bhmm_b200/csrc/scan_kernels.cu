@@ -39,6 +39,17 @@ __device__ __forceinline__ double sr_acc(double acc, double a, double b)
     return h > acc ? h : acc;
 }
 
+// Backward scan, chain c: B_c maps the exact vector after it to zero.  The trajectory then has probability zero (a frame no
+// state can emit, the outlier rule off: the reference's log-likelihood is -inf), and the exact beta is zero on chain c and every
+// chain before it in the run: that is what the exact pass starts them from.  Left as they were, these starts would come from the
+// failed warm-up pass, and the backward pass after the scan has no repair of its own.
+__device__ __forceinline__ void scan_zero_backward(const Chains& ch, int n_total, int N, int c, int j, double* he)
+{
+    auto follows = [&](int a, int b) { return b < n_total && a >= 0 && ch.t0[b] != 0 && ch.row0[a] + ch.len[a] == ch.row0[b]; };
+    for (; c > 0 && follows(c, c + 1) && follows(c - 1, c); --c)
+        if (j < N) he[(long long)c * N + j] = 0.0;
+}
+
 template <int EM, int SR>
 __global__ void __launch_bounds__(1024) k_chain_operator(Chains ch, Emission em, const double* __restrict__ A, int N, int dir,
                                                          double* __restrict__ ops, double* __restrict__ lscale)
@@ -148,7 +159,10 @@ __global__ void k_scan_starts(Chains ch, int n_total, int N, int dir, const doub
 #pragma unroll
             for (int off = 16; off > 0; off >>= 1) tot += __shfl_xor_sync(FULLM, tot, off);
             __syncwarp();
-            if (!(tot > 0.0)) return;
+            if (!(tot > 0.0)) {
+                scan_zero_backward(ch, n_total, N, c, j, he);
+                return;
+            }
             s[j] = x / tot;
             if (jv) he[(long long)c * N + j] = s[j];
             __syncwarp();
@@ -308,7 +322,10 @@ __global__ void k_scan_starts_wide(Chains ch, int n_total, int N, int dir, const
             const double Lmax = scan_block_reduce<NT, true>((jv && x > 0.0) ? L : -INFINITY, red);
             x = (jv && x > 0.0 && L > -INFINITY) ? x * exp(L - Lmax) : 0.0;
             const double tot = scan_block_reduce<NT, false>(x, red);       // (every thread has read s[] before its barriers)
-            if (!(tot > 0.0)) return;
+            if (!(tot > 0.0)) {
+                scan_zero_backward(ch, n_total, N, c, j, he);
+                return;
+            }
             s[j] = x / tot;
             if (jv) he[(long long)c * N + j] = s[j];
             __syncthreads();

@@ -50,3 +50,28 @@ inline double __shfl_sync(unsigned, double v, int src)
 }
 inline void __threadfence_block() {}
 inline void __threadfence() {}
+
+// the lane family (lane_kernels.cuh): constant-bank parameters, cache-hinted loads and stores, and its two warp collectives
+#undef __grid_constant__
+#define __grid_constant__
+inline double __ldg(const double* p) { return *p; }
+inline int __ldg(const int* p) { return *p; }
+inline double2 __ldcs(const double2* p) { return *p; }
+inline void __stcs(double2* p, double2 v) { *p = v; }
+inline double __hiloint2double(int hi, int lo)
+{
+    const long long b = (long long)(((unsigned long long)(unsigned)hi << 32) | (unsigned)lo);
+    double x;
+    memcpy(&x, &b, 8);
+    return x;
+}
+inline int __reduce_min_sync(unsigned, int v)
+{
+    emu::Warp& w = emu::my_warp();
+    w.si[emu::lane_id()] = v;
+    emu::rendezvous(w.g);
+    int r = w.si[0];
+    for (int i = 1; i < w.g.n; ++i) r = std::min(r, w.si[i]);
+    emu::rendezvous(w.g);
+    return r;
+}

@@ -1,5 +1,6 @@
-// tests/emu/lane_stubs.cpp -- the lane family (lane_kernels.cuh, N <= 16) is not part of the CPU emulation: batches are
-// reported as unsupported by it, so the engine takes the general-N path.
+// tests/emu/lane_stubs.cpp -- the default emulator build (engine_emu.so) leaves the lane family (lane_kernels.cuh, N <= 16)
+// out: batches are reported as unsupported by it, so the engine takes the general-N team path, which the other emulated
+// tests rely on.  engine_emu_lane.so (build_engine_emu.sh with LANE=1) links the real lane kernels instead of this file.
 #include "../../bhmm_b200/csrc/kernels.h"
 
 int lane_blocks_per_sm(int, int) { return 1; }

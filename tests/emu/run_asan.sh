@@ -1,7 +1,7 @@
 #!/bin/bash
 # The emulated panel-family tests under AddressSanitizer: any access of a kernel outside the caller's (numpy) buffers aborts.
 # Builds the emulator library with -fsanitize=address into a scratch copy of the test (the repo copy stays untouched).
-#   bash tests/emu/run_asan.sh          # ~5 minutes
+#   bash tests/emu/run_asan.sh          # ~7 minutes
 set -e
 ROOT=$(cd "$(dirname "$0")/../.." && pwd)
 W=$(mktemp -d)
@@ -39,3 +39,22 @@ for mode in 0 1 2; do
         BHMM_B200_PANEL=$mode BHMM_B200_CHASE_TILED=1 python engine_emu_driver.py 32,40,40 21,40,40 s32 l8 v10 w32 w40 | grep -v " ok " || true
 done
 echo "engine under ASan: done (no AddressSanitizer report above = clean)"
+
+# ---- part 3: the library with the lane family (engine_emu_lane.so, build_engine_emu.sh LANE=1) under AddressSanitizer: one
+# E-step and Gibbs sweep for the N whose lane groups pad rows (9, 10, 11, 13, 14, 15) and for N = 1 and 16.  ~2 minutes.
+L="$W/lane"
+mkdir -p "$L"
+python "$ROOT/tests/emu/hostify.py" "$ROOT/bhmm_b200/csrc/lane_kernels.cuh" > "$L/lane_kernels.cuh"
+for f in capi engine certify team_kernels panel_kernels lane_viterbi scan_kernels frame_kernels sample_kernels transfer \
+         lane_dispatch lane_inst_a lane_inst_b lane_inst_c lane_inst_d lane_inst_e lane_inst_f; do
+    python "$ROOT/tests/emu/hostify.py" "$ROOT/bhmm_b200/csrc/$f.cu" > "$L/$f.cpp"
+    g++ -O1 -g -fsanitize=address -fno-omit-frame-pointer -std=c++17 -fPIC -w $INC -DPANEL_HOST_EMU=1 \
+        -include "$ROOT/tests/emu/cuda_fake.h" -c "$L/$f.cpp" -o "$L/$f.o" &
+done
+g++ -O1 -g -fsanitize=address -std=c++17 -fPIC -w $INC -c "$ROOT/tests/emu/cuda_fake.cpp" -o "$L/cuda_fake.o" &
+wait
+g++ -shared -fsanitize=address -o "$L/engine_emu_lane.so" "$L"/*.o
+LD_PRELOAD=$(gcc -print-file-name=libasan.so) ASAN_OPTIONS=detect_leaks=0:detect_stack_use_after_return=0 \
+    BHMM_EMU_LIB="$L/engine_emu_lane.so" BHMM_B200_EXACT_SCAN=0 \
+    python "$ROOT/tests/emu/lane_emu_driver.py" 1,9,10,11,13,14,15,16 estep gibbs | grep -v " ok " || true
+echo "lane family under ASan: done (no AddressSanitizer report above = clean)"

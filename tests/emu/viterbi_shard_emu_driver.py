@@ -19,7 +19,7 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 from oracle.oracle import Oracle   # noqa: E402
 
-lib = C.CDLL(os.path.join(HERE, 'engine_emu.so'))
+lib = C.CDLL(os.environ.get('BHMM_EMU_LIB') or os.path.join(HERE, 'engine_emu.so'))
 lib.bhmm_b200_last_error_string.restype = C.c_char_p
 dp, llp, ip = C.POINTER(C.c_double), C.POINTER(C.c_longlong), C.POINTER(C.c_int)
 ERR_NOT_CERTIFIED = 6
