@@ -119,6 +119,8 @@ _proto('bhmm_b200_gibbs_discrete', C.c_int, _vp, _vp, _dp, _dp, _dp, C.c_int, C.
        C.c_ulonglong, _vp, _vp, _dp, _vp)
 _proto('bhmm_b200_mstep_dev', C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _vp)
 _proto('bhmm_b200_mstep_discrete_dev', C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, _vp)
+_proto('bhmm_b200_mstep_reversible_dev', C.c_int, _vp, _vp, C.c_int, C.c_double, C.c_int, C.c_int, C.c_double, _vp, _vp, _vp)
+_proto('bhmm_b200_sample_tmatrix_reversible_dev', C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_ulonglong, _vp, _vp, _vp, _vp)
 _proto('bhmm_b200_upload_ragged', C.c_int, _vp, C.POINTER(C.c_void_p), _llp, C.c_int, C.c_int, _vp)
 _proto('bhmm_b200_transfer_config', C.c_int, C.c_int, C.c_int)
 _proto('bhmm_b200_prefault', C.c_int, _vp, C.c_longlong, C.c_int)

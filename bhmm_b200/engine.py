@@ -61,6 +61,52 @@ def mstep_device(stats, N, means_old=None, mincount=1e-16, out=None):
     return out
 
 
+def mstep_reversible_device(stats, N, means_old=None, mincount=1e-16, stationary=False, maxiter=100000, maxerr=1e-12,
+                            out=None, iters=None):
+    """Reversible M-step on the GPU, N <= 128 (include/bhmm_b200.h: bhmm_b200_mstep_reversible_dev): ``mstep_device``'s packed
+    result with A the detailed-balance maximum-likelihood estimate (util/tmatrix.py:transition_matrix_reversible's fixed
+    point) and, with ``stationary``, pi its stationary vector.  flags: +1 when the count matrix thresholded at ``mincount`` is
+    not one strongly connected set (the host estimator applies), +1024 per collapsed sigma.  ``iters``: optional device int32
+    tensor that receives the number of fixed-point updates.  Returns the packed DEVICE tensor; nothing is copied to the
+    host."""
+    torch = _torch()
+    if out is None:
+        out = torch.empty(N * N + 3 * N + 2, dtype=torch.float64, device=stats.device)
+    m = None
+    if means_old is not None:
+        m = means_old if torch.is_tensor(means_old) else torch.as_tensor(f64(means_old)).to(stats.device)
+    with torch.cuda.device(stats.device):
+        check(lib.bhmm_b200_mstep_reversible_dev(C.c_void_p(stats.data_ptr()), C.c_void_p(m.data_ptr()) if m is not None else None,
+                                                 int(N), float(mincount), int(bool(stationary)), int(maxiter), float(maxerr),
+                                                 C.c_void_p(out.data_ptr()), C.c_void_p(iters.data_ptr()) if iters is not None else None,
+                                                 C.c_void_p(torch.cuda.current_stream(stats.device).cuda_stream)))
+    return out
+
+
+def sample_tmatrix_reversible_device(counts, prior, N, nsweeps, key):
+    """One draw from the posterior of reversible transition matrices on the GPU, N <= 128
+    (bhmm_b200_sample_tmatrix_reversible_dev; util/tmatrix.py:sample_P_reversible's chain with updates of disjoint rows in
+    parallel).  ``counts``: device int64 tensor whose first N*N entries are the path counts (``gibbs_*``'s counts);
+    ``prior``: device float64 (N, N); ``key``: the 64-bit Philox key of the draw.  Returns device tensors (T (N, N), mu (N),
+    status (1,) int32): status 1 when counts + prior is not strongly connected (T and mu are then undefined)."""
+    torch = _torch()
+    if counts.dtype != torch.int64 or not counts.is_contiguous() or counts.numel() < N * N:
+        raise TypeError('sample_tmatrix_reversible_device: a contiguous int64 tensor of at least N*N counts expected')
+    prior = prior.to(device=counts.device, dtype=torch.float64).contiguous()
+    if prior.numel() != N * N:
+        raise ValueError('sample_tmatrix_reversible_device: prior must hold N*N values')
+    T = torch.empty((N, N), dtype=torch.float64, device=counts.device)
+    mu = torch.empty(N, dtype=torch.float64, device=counts.device)
+    status = torch.empty(1, dtype=torch.int32, device=counts.device)
+    with torch.cuda.device(counts.device):
+        check(lib.bhmm_b200_sample_tmatrix_reversible_dev(C.c_void_p(counts.data_ptr()), C.c_void_p(prior.data_ptr()), int(N),
+                                                          int(nsweeps), C.c_ulonglong(int(key) & 0xFFFFFFFFFFFFFFFF),
+                                                          C.c_void_p(T.data_ptr()), C.c_void_p(mu.data_ptr()),
+                                                          C.c_void_p(status.data_ptr()),
+                                                          C.c_void_p(torch.cuda.current_stream(counts.device).cuda_stream)))
+    return T, mu, status
+
+
 def unpack_mstep(packed, N):
     """Host view of ``mstep_device``'s result: dict(A, pi, means, sigmas, flags, loglik)."""
     p = np.asarray(packed, dtype=np.float64)

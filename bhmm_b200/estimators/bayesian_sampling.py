@@ -9,7 +9,10 @@ need.  The parameter draws are tiny host math with numpy's global RNG, as in the
 Transition-matrix draw: the reference delegates to msmtools.estimation.sample_tmatrix (absent, un-pinned).  The
 non-reversible posterior is row-wise Dirichlet(C_i + prior_i) and is drawn here directly; the reversible posterior is
 sampled by a from-scratch Metropolis sampler on symmetric weights (util/tmatrix.py:sample_P_reversible; the reference
-delegates to msmtools, so this part is PARITY-UNPINNED, SURVEY.md section 8c).
+delegates to msmtools, so this part is PARITY-UNPINNED, SURVEY.md section 8c).  For N <= 128 that chain runs on the GPU from
+the device path counts (engine.sample_tmatrix_reversible_device: the same target, start and sweep count, updates of
+disjoint rows in parallel); path statistics given as host arrays and counts that are not strongly connected take the host
+sampler.
 """
 import copy
 import time
@@ -17,7 +20,7 @@ import time
 import numpy as np
 
 from .. import dist
-from ..engine import TrajectoryBatch, TimeShardedTrajectories, make_batch, download_array
+from ..engine import TrajectoryBatch, TimeShardedTrajectories, make_batch, download_array, sample_tmatrix_reversible_device
 from ..util import config
 from ..util.logger import logger
 from ..util import tmatrix as _tmatrix
@@ -88,6 +91,7 @@ class BayesianHMMSampler(object):
         else:
             raise ValueError('transition matrix prior mode undefined: ' + str(transition_matrix_prior))
         self.transition_matrix_sampling_steps = transition_matrix_sampling_steps
+        self._prior_C_dev = None         # device copy of prior_C for the reversible draw on the GPU
         self.model.output_model.set_implementation(config.kernel)
         # batch=: an engine batch that already holds these trajectories on the GPU (no second upload)
         if batch is not None:
@@ -167,6 +171,7 @@ class BayesianHMMSampler(object):
         counts = dist.allreduce_sum(counts.clone())
         c = counts.cpu().numpy()
         st.update(C=c[:N * N].reshape(N, N).copy(), n0=c[N * N:N * N + N].copy(), count=c[N * N + N:].copy())
+        st['C_dev'] = counts                 # the all-reduced counts stay on the GPU for the reversible draw
         self._sweep += 1
         self.last_loglik = ll
         if keep_paths and self._time_sharded:
@@ -186,12 +191,18 @@ class BayesianHMMSampler(object):
     def _updateTransitionMatrix(self, st):
         """Sample the transition matrix and the initial distribution (:341-373)."""
         Cm = st['C'].astype(float) + self.prior_C
+        mu = None
         if self.reversible:
             # from-scratch reversible sampler (the reference calls msmtools here; parity unpinned, util/tmatrix.py)
             # every draw starts at the reversible maximum-likelihood estimate of the CURRENT counts (their sparsity
-            # pattern may differ from the previous sweep's) and runs transition_matrix_sampling_steps / 50 sweeps
-            Tij = _tmatrix.sample_P_reversible(Cm, nsteps=max(10, self.transition_matrix_sampling_steps // 50),
-                                               rng=self._np_rng)
+            # pattern may differ from the previous sweep's) and runs transition_matrix_sampling_steps / 50 sweeps: on the
+            # GPU from the device counts (N <= 128), else -- and for counts that are not strongly connected -- on the host
+            nsteps = max(10, self.transition_matrix_sampling_steps // 50)
+            Tij = None
+            if st.get('C_dev') is not None and self.nstates <= 128:
+                Tij, mu = self._sample_reversible_device(st['C_dev'], nsteps)
+            if Tij is None:
+                Tij = _tmatrix.sample_P_reversible(Cm, nsteps=nsteps, rng=self._np_rng)
         else:
             Tij = np.zeros_like(Cm)
             for i in range(self.nstates):
@@ -201,7 +212,7 @@ class BayesianHMMSampler(object):
                 else:
                     Tij[i, positive] = self._rng.dirichlet(Cm[i, positive])
         if self.stationary:
-            p0 = _tmatrix.stationary_distribution(Tij, C=Cm)
+            p0 = mu if mu is not None else _tmatrix.stationary_distribution(Tij, C=Cm)
         else:
             n0 = st['n0'].astype(float)
             first_timestep_counts_with_prior = n0 + self.prior_n0
@@ -209,3 +220,18 @@ class BayesianHMMSampler(object):
             p0 = np.zeros_like(n0)
             p0[positive] = self._rng.dirichlet(first_timestep_counts_with_prior[positive])
         self.model.update(p0, Tij)
+
+    def _sample_reversible_device(self, C_dev, nsteps):
+        """The reversible draw on the GPU (engine.sample_tmatrix_reversible_device): (T, stationary vector) as host arrays, or
+        (None, None) when the posterior counts are not strongly connected.  The Philox key is one draw from the stream the
+        host sampler consumes, so np.random.seed reproduces a run and the ranks, which share that stream, draw the same T."""
+        import torch
+        N = self.nstates
+        if getattr(self, '_prior_C_dev', None) is None or self._prior_C_dev.device != C_dev.device:
+            self._prior_C_dev = torch.as_tensor(np.ascontiguousarray(self.prior_C, dtype=np.float64)).to(C_dev.device)
+        key = int(self._np_rng.integers(0, 2 ** 63, dtype=np.int64))
+        T, mu, status = sample_tmatrix_reversible_device(C_dev, self._prior_C_dev, N, nsteps, key)
+        if int(status.item()) != 0:
+            return None, None
+        return T.cpu().numpy(), mu.cpu().numpy()
+

@@ -5,10 +5,12 @@ transition_counts on host arrays (maximum_likelihood.py:221-269), keeps every ga
 in the M-step (:284-330).  Here one fused E-step per iteration runs over all trajectories on the GPU
 (bhmm_b200.engine.TrajectoryBatch) and returns only the sufficient statistics the M-step needs; with several
 ranks (torch.distributed initialised) the trajectories are sharded and the statistics all-reduced
-(bhmm_b200.dist).  On the non-reversible branch the M-step runs on the GPU as well (engine.mstep_device: transition
-matrix, initial distribution, Gaussian means/sigmas or the discrete output matrix from the reduced statistics), and one
-small device-to-host copy per iteration brings back the updated parameters and the log-likelihood; the reversible /
-stationary / fixed-distribution branches and count matrices with empty entries use the host code (util/tmatrix.py).
+(bhmm_b200.dist).  The M-step runs on the GPU as well (engine.mstep_device: transition matrix, initial distribution,
+Gaussian means/sigmas or the discrete output matrix from the reduced statistics; engine.mstep_reversible_device: the
+reversible maximum-likelihood transition matrix for N <= 128, with or without stationary=), and one small device-to-host
+copy per iteration brings back the updated parameters and the log-likelihood.  The non-reversible stationary and the
+fixed-distribution branches, N > 128 on the reversible branch, and the count matrices the kernels flag (empty entries on the
+non-reversible branch, counts that are not strongly connected on the reversible one) use the host code (util/tmatrix.py).
 """
 import copy
 import time
@@ -16,7 +18,7 @@ import time
 import numpy as np
 
 from .. import dist
-from ..engine import (TrajectoryBatch, TimeShardedTrajectories, make_batch, unpack_stats, mstep_device, mstep_discrete_device, unpack_mstep, download_array,
+from ..engine import (TrajectoryBatch, TimeShardedTrajectories, make_batch, unpack_stats, mstep_device, mstep_reversible_device, mstep_discrete_device, unpack_mstep, download_array,
                       HostBufferInBackground)
 from ..util import config
 from ..util.logger import logger
@@ -100,6 +102,7 @@ class MaximumLikelihoodEstimator(object):
         self._device_mstep = bool(device_mstep)
         self.device_msteps = 0          # iterations whose M-step ran on the GPU
         self._dev = None                # device tensors of the last E-step (reduced statistics, B numerators)
+        self._mstep_reversible = False  # the GPU M-step of this iteration is the reversible one
 
     # ---- properties of the reference estimator
     @property
@@ -216,18 +219,30 @@ class MaximumLikelihoodEstimator(object):
         return st
 
     def _device_mstep_applies(self):
-        """The GPU M-step implements the non-reversible estimator C / rowsum with pi = gamma0 / sum: that is what the
-        reference reaches (maximum_likelihood.py:307-320) when the CURRENT matrix is not reversible and nothing is fixed."""
-        return (not self._stationary and self._fixed_initial_distribution is None
-                and self._fixed_stationary_distribution is None and not self._hmm.is_reversible)
+        """Whether the GPU M-step implements the estimator the reference reaches (maximum_likelihood.py:307-320) from the
+        CURRENT matrix with nothing fixed: the non-reversible C / rowsum with pi = gamma0 / sum, or, for a reversible current
+        matrix and N <= 128, the reversible MLE (with or without stationary=).  Remembers which one for
+        _update_model_device."""
+        if self._fixed_initial_distribution is not None or self._fixed_stationary_distribution is not None:
+            return False
+        self._mstep_reversible = self._hmm.is_reversible
+        if self._mstep_reversible:
+            return self._nstates <= 128
+        return not self._stationary
 
     def _update_model_device(self):
         """M-step on the GPU; one device-to-host copy of [A | pi | means | sigmas | flags | loglik].  Returns the
-        log-likelihood, or None when the kernel flagged a case for the host code (an empty count, a collapsed sigma)."""
+        log-likelihood, or None when the kernel flagged a case for the host code (an empty count, counts that are not
+        strongly connected on the reversible branch, a collapsed sigma)."""
         stats, Bnum = self._dev
         N = self._nstates
         om = self._hmm.output_model
-        packed = mstep_device(stats, N, means_old=om.means if self._output == 'gaussian' else None, mincount=1e-16)
+        means_old = om.means if self._output == 'gaussian' else None
+        if self._mstep_reversible:
+            packed = mstep_reversible_device(stats, N, means_old=means_old, mincount=1e-16, stationary=self._stationary,
+                                             maxiter=self._maxit_P, maxerr=1e-12)
+        else:
+            packed = mstep_device(stats, N, means_old=means_old, mincount=1e-16)
         B = mstep_discrete_device(Bnum) if Bnum is not None else None
         res = unpack_mstep(packed.cpu().numpy(), N)
         if res['flags'] != 0:

@@ -322,6 +322,28 @@ int bhmm_b200_mstep_dev(const double* d_stats, const double* d_means_old, int N,
 /* DiscreteOutputModel.estimate's normalisation (discrete.py:214-215): d_B (N,M) = d_Bnum / rowsum; d_Bt (M,N), optional,
  * receives the transposed table. */
 int bhmm_b200_mstep_discrete_dev(const double* d_Bnum, int N, int M, double* d_B, double* d_Bt, void* stream);
+/* Reversible M-step on the device, N <= 128 (util/tmatrix.py:transition_matrix_reversible, the branch estimate_P takes for a
+ * reversible current matrix).  d_out as bhmm_b200_mstep_dev, with A the detailed-balance maximum-likelihood estimate of the
+ * statistics' count matrix C by the fixed point x_ij <- (c_ij + c_ji) / (c_i/x_i + c_j/x_j) from X = (C + C^T) / sum,
+ * normalised to sum 1 after every update, stopped when max |pi_new - pi_old| < maxerr or after maxiter (>= 1) updates,
+ * A = X / rowsum.  stationary != 0: pi = the normalised row sums of X (the stationary vector of A) instead of
+ * gamma0 / sum.  flags: +1 when C thresholded at mincount (entries <= mincount dropped) is not one strongly connected set
+ * (A is then the non-reversible estimate and the caller must use the host estimator), +1024 per collapsed sigma.
+ * d_iters (device int, optional) receives the number of fixed-point updates.  N = 1 gives A = [[1]].  Sums run in a fixed
+ * order: identical statistics give bit-identical results. */
+int bhmm_b200_mstep_reversible_dev(const double* d_stats, const double* d_means_old, int N, double mincount, int stationary,
+                                   int maxiter, double maxerr, double* d_out, int* d_iters, void* stream);
+/* One draw from the posterior of reversible transition matrices (util/tmatrix.py:sample_P_reversible's chain), N <= 128.
+ * C = d_counts (device int64, N*N: the path counts) + d_prior (device float64, N*N).  Start: the reversible MLE of C (maxerr
+ * 1e-12, at most 1e6 updates) as symmetric weights x_ij = pi_i T_ij, scaled so that the weights of the pattern {i <= j :
+ * x_ij > 0} sum to its size; then nsweeps Metropolis sweeps with log-normal proposals (sigma 0.5) and the host's acceptance
+ * rule, in rounds of updates on disjoint rows (the diagonal, then a round-robin matching of the states; DESIGN.md 5.12).
+ * The uniforms come from Philox4x32-10 keyed by `key`: the update in (sweep, round, slot) draws its normal by Box-Muller
+ * from the block with counter (row = round << 32 | slot, sweep) and its acceptance uniform from (row, 1 << 32 | sweep).
+ * d_T (device, N*N) = X / rowsum, d_mu (device, N) = rowsum / sum, *d_status (device int) = 0; status 1 (d_T, d_mu
+ * untouched) when C is not strongly connected.  N = 1 gives [[1]]. */
+int bhmm_b200_sample_tmatrix_reversible_dev(const long long* d_counts, const double* d_prior, int N, int nsweeps,
+                                            unsigned long long key, double* d_T, double* d_mu, int* d_status, void* stream);
 
 /* ---- synthetic trajectories (HMM.generate_synthetic_*, bhmm/hmm/generic_hmm.py:433-589) --------------------------
  * Hidden states of K trajectories (host offsets as in bhmm_b200_batch_create) drawn by exact time-parallel forward
