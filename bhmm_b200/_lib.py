@@ -121,6 +121,15 @@ _proto('bhmm_b200_mstep_dev', C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _vp)
 _proto('bhmm_b200_mstep_discrete_dev', C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, _vp)
 _proto('bhmm_b200_mstep_reversible_dev', C.c_int, _vp, _vp, C.c_int, C.c_double, C.c_int, C.c_int, C.c_double, _vp, _vp, _vp)
 _proto('bhmm_b200_sample_tmatrix_reversible_dev', C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_ulonglong, _vp, _vp, _vp, _vp)
+# initial-model statistics
+_proto('bhmm_b200_init_subsample_dev', C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_longlong, C.c_longlong, _vp, _vp)
+_proto('bhmm_b200_gmm_work_doubles', C.c_longlong, C.c_longlong, C.c_int)
+_proto('bhmm_b200_gmm_em_step_dev', C.c_int, _vp, C.c_longlong, C.c_int, C.c_double, _vp, _vp, _vp, _vp)
+_proto('bhmm_b200_init_counts_gaussian_dev', C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_longlong, C.c_int, C.c_int, _vp,
+       _vp, _vp)
+_proto('bhmm_b200_init_counts_symbols_dev', C.c_int, _vp, _vp, _vp, _vp, C.c_int, C.c_longlong, C.c_int, C.c_int, _vp, _vp)
+_proto('bhmm_b200_init_counts_labels_dev', C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int,
+       _vp, _vp, _vp, _vp)
 _proto('bhmm_b200_upload_ragged', C.c_int, _vp, C.POINTER(C.c_void_p), _llp, C.c_int, C.c_int, _vp)
 _proto('bhmm_b200_transfer_config', C.c_int, C.c_int, C.c_int)
 _proto('bhmm_b200_prefault', C.c_int, _vp, C.c_longlong, C.c_int)

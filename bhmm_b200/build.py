@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, 'csrc')
 OBJ = os.path.join(CSRC, '_obj')
 LIB = os.path.join(HERE, 'libbhmm_b200.so')
 SOURCES = ['lane_inst_a.cu', 'lane_inst_b.cu', 'lane_inst_c.cu', 'lane_inst_d.cu', 'lane_inst_e.cu', 'lane_inst_f.cu',
-           'lane_dispatch.cu', 'team_kernels.cu', 'panel_kernels.cu', 'lane_viterbi.cu', 'scan_kernels.cu', 'frame_kernels.cu', 'tmatrix_kernels.cu', 'certify.cu', 'sample_kernels.cu', 'capi.cu', 'engine.cu', 'transfer.cu']
+           'lane_dispatch.cu', 'team_kernels.cu', 'panel_kernels.cu', 'lane_viterbi.cu', 'scan_kernels.cu', 'frame_kernels.cu', 'tmatrix_kernels.cu', 'init_kernels.cu', 'certify.cu', 'sample_kernels.cu', 'capi.cu', 'engine.cu', 'transfer.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '--expt-relaxed-constexpr', '-Xcompiler', '-fPIC', '-Xptxas', '-v']
 

@@ -76,3 +76,46 @@ def broadcast_int(value, src=0):
     t = torch.tensor([int(value)], dtype=torch.int64, device=dev)
     td.broadcast(t, src=src)
     return int(t.item())
+
+
+def _device():
+    import torch
+    return torch.device('cuda', torch.cuda.current_device()) if _td().get_backend() == 'nccl' else torch.device('cpu')
+
+
+def allreduce_max(tensor):
+    """In-place maximum over ranks of a tensor; identity when torch.distributed is not initialised."""
+    if initialized() and world_size() > 1:
+        _td().all_reduce(tensor, op=_td().ReduceOp.MAX)
+    return tensor
+
+
+def broadcast_array(array, src=0):
+    """Rank `src`'s copy of a numpy array on every rank, bit for bit (identity without torch.distributed).  Every rank passes
+    an array of the same shape and dtype; only `src`'s contents matter.  The initial-model builders send the packed model
+    this way, so that all ranks start from identical parameters."""
+    array = np.ascontiguousarray(array)
+    if not (initialized() and world_size() > 1):
+        return array
+    import torch
+    t = torch.from_numpy(array.copy()).to(_device())
+    _td().broadcast(t, src=src)
+    return t.cpu().numpy()
+
+
+def allgather_varlen(tensor):
+    """Every rank's 1-D tensor, of any length, as a list of host arrays in rank order (the local one alone without
+    torch.distributed): one all_gather of the lengths, one of the pieces padded to the longest."""
+    if not (initialized() and world_size() > 1):
+        return [tensor.cpu().numpy()]
+    import torch
+    td, dev = _td(), _device()
+    n = torch.tensor([tensor.numel()], dtype=torch.int64, device=dev)
+    ns = [torch.empty_like(n) for _ in range(world_size())]
+    td.all_gather(ns, n)
+    ns = [int(x.item()) for x in ns]
+    pad = torch.zeros(max(max(ns), 1), dtype=tensor.dtype, device=dev)
+    pad[:tensor.numel()] = tensor.to(dev)
+    got = [torch.empty_like(pad) for _ in ns]
+    td.all_gather(got, pad)
+    return [g[:m].cpu().numpy() for g, m in zip(got, ns)]

@@ -542,6 +542,140 @@ class TrajectoryBatch(object):
         N = self.N
         return dict(C=c[:N * N].reshape(N, N).copy(), n0=c[N * N:N * N + N].copy(), count=c[N * N + N:].copy())
 
+    # -------------------------------------------------------------------------------------------- initial-model statistics
+    # The per-frame passes of api.init_gaussian_hmm / init_discrete_hmm (batch=) over the owned frames of this batch
+    # (include/bhmm_b200.h, "initial-model statistics").  The integer outputs are ADDED to ``out`` / ``B`` when given, so the
+    # groups of a SubBatchedTrajectories and the shards of one process accumulate into one buffer.
+    _first_is_start = None  # per trajectory: local frame 0 is the trajectory's frame 0 (None: every one; time shards set it)
+
+    def _init_rows(self):
+        """Device (offsets, own_lo, own_hi, flags) of the rows; uploaded on first use, None where the default applies."""
+        if getattr(self, '_init_dev', None) is None:
+            torch = self.torch
+
+            def up(a, dt):
+                return torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).to(self.device)
+            lo = hi = flags = None
+            if self._own_ranges is not None:
+                lo = up([r[0] for r in self._own_ranges], np.int64)
+                hi = up([r[1] for r in self._own_ranges], np.int64)
+            if self._first_is_start is not None:
+                flags = up([2 if s else 0 for s in self._first_is_start], np.int32)
+            self._init_dev = (up(self.offsets, np.int64), lo, hi, flags)
+        return self._init_dev
+
+    def owned_ranges(self):
+        """Host (K, 2) int64 array of the owned local frame range [lo, hi) of every trajectory."""
+        if self._own_ranges is None:
+            return np.stack([np.zeros(self.K, dtype=np.int64), self.lengths]).T.copy()
+        return np.asarray(self._own_ranges, dtype=np.int64).reshape(self.K, 2)
+
+    def owned_frames(self):
+        r = self.owned_ranges()
+        return int(np.maximum(r[:, 1] - r[:, 0], 0).sum())
+
+    @staticmethod
+    def _ptr(t):
+        return C.c_void_p(t.data_ptr()) if t is not None else None
+
+    def init_subsample(self, stride, goff):
+        """The owned frames whose index g in the global concatenation of all trajectories is a multiple of ``stride``, in
+        order (float64 DEVICE tensor).  ``goff``: per trajectory, the global index of its local frame 0."""
+        self._require_gaussian()
+        s = int(stride)
+        goff = np.ascontiguousarray(goff, dtype=np.int64)
+        r = self.owned_ranges()
+        glo, ghi = goff + r[:, 0], goff + np.maximum(r[:, 1], r[:, 0])
+        cnt = (ghi + s - 1) // s - (glo + s - 1) // s
+        outoff = np.zeros(self.K + 1, dtype=np.int64)
+        np.cumsum(cnt, out=outoff[1:])
+        n = int(outoff[-1])
+        torch = self.torch
+        out = torch.empty(n, dtype=torch.float64, device=self.device)
+        if n == 0:
+            return out
+        offs, lo, hi, _ = self._init_rows()
+        d_goff = torch.from_numpy(goff).to(self.device)
+        d_outoff = torch.from_numpy(outoff).to(self.device)
+        with torch.cuda.device(self.device):
+            check(lib.bhmm_b200_init_subsample_dev(self._ptr(self.obs), self._ptr(offs), self._ptr(lo), self._ptr(hi),
+                                                   self._ptr(d_goff), self._ptr(d_outoff), self.K, s, n, self._ptr(out),
+                                                   self._stream()))
+        return out
+
+    def _init_out(self, out, n):
+        if out is None:
+            return self.torch.zeros(n, dtype=self.torch.int64, device=self.device)
+        if out.dtype != self.torch.int64 or not out.is_contiguous() or out.numel() != n or out.device != self.device:
+            raise ValueError('init statistics: a contiguous int64 device tensor of %d entries expected' % n)
+        return out
+
+    @staticmethod
+    def _check_lag(lag):
+        if int(lag) != lag or lag < 1:
+            raise ValueError('lag must be a positive integer, got %r' % (lag,))
+
+    def init_counts_gaussian(self, weights, means, sigmas, lag=1, out=None):
+        """int64 DEVICE [C (N*N) | n0 (N)]: lag-``lag`` pair counts and first-frame histogram of the maximum-responsibility
+        assignment of the mixture (init_gaussian_hmm's arg-max, bit for bit), added to ``out`` when given."""
+        self._require_gaussian()
+        self._check_lag(lag)
+        N = len(means)
+        w, m, sg = f64(weights), f64(means), f64(sigmas)
+        gp = self.torch.from_numpy(np.concatenate([m, sg, np.log(w), np.log(sg)])).to(self.device)
+        out = self._init_out(out, N * N + N)
+        offs, lo, hi, flags = self._init_rows()
+        with self.torch.cuda.device(self.device):
+            check(lib.bhmm_b200_init_counts_gaussian_dev(self._ptr(self.obs), self._ptr(offs), self._ptr(lo), self._ptr(hi),
+                                                         self._ptr(flags), self.K, self.rows, int(lag), N, self._ptr(gp),
+                                                         self._ptr(out), self._stream()))
+        return out
+
+    def symbol_range(self):
+        """(smallest, largest) symbol of an integer batch (one reduction per observation buffer); negative symbols raise
+        IndexError."""
+        if not self.discrete:
+            raise TypeError('this batch holds float observations; a discrete output model needs integer symbols')
+        key = (self.obs.data_ptr(), self.obs._version)
+        if self._sym_range is None or self._sym_range[0] != key:
+            lo, hi = self.torch.aminmax(self.obs)
+            self._sym_range = (key, int(lo.item()), int(hi.item()))
+        _, lo, hi = self._sym_range
+        if lo < 0:
+            raise IndexError('observation symbols must be non-negative, found %d' % lo)
+        return lo, hi
+
+    def init_counts_symbols(self, nsym, lag=1, out=None):
+        """int64 DEVICE (nsym * nsym): lag-``lag`` symbol pair counts of the owned frames (init_discrete_hmm's C), added to
+        ``out`` when given."""
+        self._require_discrete(nsym)
+        self._check_lag(lag)
+        out = self._init_out(out, int(nsym) * int(nsym))
+        offs, lo, hi, _ = self._init_rows()
+        with self.torch.cuda.device(self.device):
+            check(lib.bhmm_b200_init_counts_symbols_dev(self._ptr(self.obs), self._ptr(offs), self._ptr(lo), self._ptr(hi),
+                                                        self.K, self.rows, int(lag), int(nsym), self._ptr(out), self._stream()))
+        return out
+
+    def init_counts_labels(self, label, nstates, lag=1, out=None, B=None):
+        """Hidden statistics of the symbol -> cluster label map ``label`` (host or device int, one entry in [0, nstates) per
+        symbol): int64 DEVICE [Ch (N*N) | n0 (N)] and the (N, M) histogram B[label(o), o] of the owned frames, added to
+        ``out`` / ``B`` when given."""
+        torch = self.torch
+        lab = label if torch.is_tensor(label) else torch.from_numpy(np.ascontiguousarray(label, dtype=np.int32))
+        lab = lab.to(device=self.device, dtype=torch.int32).contiguous()
+        M, N = lab.numel(), int(nstates)
+        self._require_discrete(M)
+        self._check_lag(lag)
+        out = self._init_out(out, N * N + N)
+        B = self._init_out(B, N * M)
+        offs, lo, hi, flags = self._init_rows()
+        with torch.cuda.device(self.device):
+            check(lib.bhmm_b200_init_counts_labels_dev(self._ptr(self.obs), self._ptr(offs), self._ptr(lo), self._ptr(hi),
+                                                       self._ptr(flags), self.K, self.rows, int(lag), N, M, self._ptr(lab),
+                                                       self._ptr(out), self._ptr(B), self._stream()))
+        return out, B
+
 
 class SubBatchedTrajectories(object):
     """The interface of ``TrajectoryBatch`` for data sets whose forward variables do not fit the GPU at once.
@@ -757,6 +891,37 @@ class SubBatchedTrajectories(object):
             hist = h.clone() if hist is None else hist.add_(h)
             ll += l
         return path, counts, hist, ll
+
+    # ---- initial-model statistics: the groups' integer statistics accumulate into one buffer, the subsamples concatenate
+    def owned_frames(self):
+        return self.rows
+
+    def owned_ranges(self):
+        return np.concatenate([sub.owned_ranges() for _, _, sub in self._subs])
+
+    def init_subsample(self, stride, goff):
+        goff = np.asarray(goff, dtype=np.int64)
+        parts = [sub.init_subsample(stride, goff[a:b]) for (a, b), (_, _, sub) in zip(self.groups, self._subs)]
+        return self.torch.cat(parts)
+
+    def init_counts_gaussian(self, weights, means, sigmas, lag=1, out=None):
+        for _, _, sub in self._subs:
+            out = sub.init_counts_gaussian(weights, means, sigmas, lag=lag, out=out)
+        return out
+
+    def symbol_range(self):
+        rng = [sub.symbol_range() for _, _, sub in self._subs]
+        return min(r[0] for r in rng), max(r[1] for r in rng)
+
+    def init_counts_symbols(self, nsym, lag=1, out=None):
+        for _, _, sub in self._subs:
+            out = sub.init_counts_symbols(nsym, lag=lag, out=out)
+        return out
+
+    def init_counts_labels(self, label, nstates, lag=1, out=None, B=None):
+        for _, _, sub in self._subs:
+            out, B = sub.init_counts_labels(label, nstates, lag=lag, out=out, B=B)
+        return out, B
 
 
 def make_batch(observations, nstates, device=None, chunk=0, warm=0, max_workspace_bytes=None):
@@ -1039,6 +1204,7 @@ class TimeShardedTrajectories(object):
         cat = np.concatenate([np.asarray(p, dtype=host_dtype) for p in pieces])
         self.batch = TrajectoryBatch.from_concatenated(cat, lengths, self.N, device=device, chunk=chunk, warm=warm,
                                                        own_ranges=own)
+        self.batch._first_is_start = [a == 0 for a in self._starts]
         self.K = len(lengths)
         self.viterbi_fallbacks = 0                       # Viterbi calls that needed the exact border exchange
 
@@ -1065,6 +1231,7 @@ class TimeShardedTrajectories(object):
         self._starts = [int(start)]
         self.batch = TrajectoryBatch.from_concatenated(piece, [n], self.N, device=device, chunk=chunk, warm=warm,
                                                        own_ranges=[(lo - start, hi - start)])
+        self.batch._first_is_start = [int(start) == 0]
         self.K = 1
         self.viterbi_fallbacks = 0
         return self
@@ -1080,6 +1247,52 @@ class TimeShardedTrajectories(object):
 
     def info(self):
         return self.batch.info()
+
+    # ------------------------------------------------------------------------------------------ initial-model statistics
+    # The owned frames of the shards partition the data set, so their integer statistics add up to the unsharded ones.  A pair
+    # (t, t + lag) whose second frame lies after this shard's piece cannot be counted here: such a lag is refused.
+    def init_lag_error(self, lag):
+        """The message of the ValueError a pair count at ``lag`` raises on this shard, or None: a trajectory that continues
+        past the shard needs a right halo of at least ``lag`` frames."""
+        for k, (lo, hi, T) in enumerate(self.global_ranges):
+            end = self._starts[k] + int(self.batch.lengths[k])
+            if hi > lo and end < T and lag > end - hi:
+                return ('time shard %d: trajectory %d continues after the shard, and its right halo of %d frames is shorter '
+                        'than lag=%d' % (self.rank, k, end - hi, lag))
+        return None
+
+    def _require_lag(self, lag):
+        TrajectoryBatch._check_lag(lag)
+        msg = self.init_lag_error(lag)
+        if msg is not None:
+            raise ValueError(msg)
+
+    def owned_frames(self):
+        return self.batch.owned_frames()
+
+    def owned_ranges(self):
+        return self.batch.owned_ranges()
+
+    def init_subsample(self, stride, goff=None):
+        """As ``TrajectoryBatch.init_subsample``; the global offsets follow from the trajectory lengths (``goff`` unused)."""
+        T = np.asarray([g[2] for g in self.global_ranges], dtype=np.int64)
+        first = np.concatenate([[0], np.cumsum(T)[:-1]]).astype(np.int64)
+        return self.batch.init_subsample(stride, first + np.asarray(self._starts, dtype=np.int64))
+
+    def init_counts_gaussian(self, weights, means, sigmas, lag=1, out=None):
+        self._require_lag(lag)
+        return self.batch.init_counts_gaussian(weights, means, sigmas, lag=lag, out=out)
+
+    def symbol_range(self):
+        return self.batch.symbol_range()
+
+    def init_counts_symbols(self, nsym, lag=1, out=None):
+        self._require_lag(lag)
+        return self.batch.init_counts_symbols(nsym, lag=lag, out=out)
+
+    def init_counts_labels(self, label, nstates, lag=1, out=None, B=None):
+        self._require_lag(lag)
+        return self.batch.init_counts_labels(label, nstates, lag=lag, out=out, B=B)
 
     # ------------------------------------------------------------------------------------------ Viterbi across shards
     def _viterbi_batch(self):

@@ -35,6 +35,9 @@ class BayesianHMMSampler(object):
     ``from_local_piece``.  With time shards the hidden paths are the ones one GPU would draw for the same key: the Philox key
     is the same on every rank and every frame draws the uniform of its row in the unsharded data set.
     ``save_hidden_state_trajectory`` then keeps, on each rank, the paths of the frames that rank owns.
+
+    ``initial_model=None`` starts from a maximum-likelihood fit (``MaximumLikelihoodEstimator`` with ``initial_model=None``
+    and ``output=``) on the sampler's own batch, as the reference's sampler does.
     """
 
     def __init__(self, observations, nstates, initial_model=None, reversible=True, stationary=False,
@@ -42,8 +45,6 @@ class BayesianHMMSampler(object):
                  output='gaussian', chunk=0, warm=0, shard=True, batch=None):
         if len(observations) == 0:
             raise Exception("No observations were provided.")
-        if initial_model is None:
-            raise NotImplementedError('bhmm_b200 needs initial_model= (bhmm.init_hmm is outside the hot path)')
         self.reversible = reversible
         self._time_sharded = (isinstance(shard, str) and shard == 'time') or isinstance(batch, TimeShardedTrajectories)
         # Host-side parameter draws.  One process: numpy's global RNG, as in the reference (np.random.seed reproduces a
@@ -64,6 +65,16 @@ class BayesianHMMSampler(object):
         self.nobs = len(self.observations)
         self.Ts = [len(o) for o in self.observations]
         self.maxT = np.max(self.Ts) if self.Ts else 0
+        # batch=: an engine batch that already holds these trajectories on the GPU (no second upload)
+        if batch is not None:
+            self._batch = batch
+        elif self._time_sharded:
+            self._batch = TimeShardedTrajectories(self.observations, nstates, dist.rank(), dist.world_size(), chunk=chunk,
+                                                  warm=warm)
+        else:
+            self._batch = make_batch(self.observations, nstates, chunk=chunk, warm=warm) if self.nobs else None
+        if initial_model is None:
+            initial_model = self._generate_initial_model(observations, output, shard)
         self.model = copy.deepcopy(initial_model)
         self._output = self.model.output_model.model_type
         # priors (bayesian_sampling.py:146-176)
@@ -93,14 +104,6 @@ class BayesianHMMSampler(object):
         self.transition_matrix_sampling_steps = transition_matrix_sampling_steps
         self._prior_C_dev = None         # device copy of prior_C for the reversible draw on the GPU
         self.model.output_model.set_implementation(config.kernel)
-        # batch=: an engine batch that already holds these trajectories on the GPU (no second upload)
-        if batch is not None:
-            self._batch = batch
-        elif self._time_sharded:
-            self._batch = TimeShardedTrajectories(self.observations, nstates, dist.rank(), dist.world_size(), chunk=chunk,
-                                                  warm=warm)
-        else:
-            self._batch = make_batch(self.observations, nstates, chunk=chunk, warm=warm) if self.nobs else None
         self._sweep = 0
         # Philox key of the hidden-path draws.  Without an explicit seed= in sample() it comes from the agreed host stream
         # (np.random.seed makes a run reproducible, two samplers do not share their uniforms; the reference continues
@@ -108,6 +111,15 @@ class BayesianHMMSampler(object):
         self._seed = int(self._rng.randint(0, 2 ** 31 - 1))
         self.timings = {'hidden': 0.0, 'parameters': 0.0}
         self.last_loglik = None
+
+    def _generate_initial_model(self, observations, output, shard):
+        """The maximum-likelihood fit the sampler starts from when no initial model is given (the reference's
+        _generateInitialModel), run on the sampler's own batch: its initial model comes from ``init_hmm`` on that batch."""
+        from .maximum_likelihood import MaximumLikelihoodEstimator
+        est = MaximumLikelihoodEstimator(observations, self.nstates, initial_model=None, output=output,
+                                         reversible=self.reversible, stationary=self.stationary, shard=shard,
+                                         batch=self._batch)
+        return est.fit()
 
     def sample(self, nsamples, nburn=0, nthin=1, save_hidden_state_trajectory=False, call_back=None, seed=None):
         """Sample from the BHMM posterior (bayesian_sampling.py:206-267)."""

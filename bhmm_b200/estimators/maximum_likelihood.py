@@ -28,9 +28,10 @@ from ..util import tmatrix as _tmatrix
 class MaximumLikelihoodEstimator(object):
     """Maximum likelihood Hidden Markov model (HMM) estimator (maximum_likelihood.py:30-144).
 
-    Parameters follow the reference: ``observations`` (list of 1-D arrays), ``nstates``, ``initial_model`` (required
-    here: the reference's heuristics in bhmm/init need msmtools / a vendored GMM and are out of scope),
-    ``reversible``, ``stationary``, ``p``, ``accuracy``, ``maxit``, ``maxit_P``.  Extra: ``chunk`` / ``warm`` (time
+    Parameters follow the reference: ``observations`` (list of 1-D arrays), ``nstates``, ``initial_model``,
+    ``reversible``, ``stationary``, ``p``, ``accuracy``, ``maxit``, ``maxit_P``.  ``initial_model=None`` builds the initial
+    model of ``api.init_hmm`` for ``output=`` ('gaussian' or 'discrete') from the estimator's own device-resident batch before
+    the first E-step (``init_hmm(batch=...)``: every rank counts its shard, all ranks receive the same model).  Extra: ``chunk`` / ``warm`` (time
     chunking of the kernels, 0 = automatic) and ``shard`` (True: keep only this rank's share of the trajectories).
 
     ``shard='time'`` cuts EVERY trajectory in time over the ranks instead (``engine.TimeShardedTrajectories``: one trajectory
@@ -47,13 +48,11 @@ class MaximumLikelihoodEstimator(object):
     def __init__(self, observations, nstates, initial_model=None, output='gaussian', reversible=True, stationary=False,
                  p=None, accuracy=1e-3, maxit=1000, maxit_P=100000, chunk=0, warm=0, shard=True, device_mstep=True, batch=None,
                  exact_viterbi_borders=False):
-        if initial_model is None:
-            raise NotImplementedError('bhmm_b200 needs initial_model= (bhmm.init_hmm is outside the hot path)')
         self._nstates = nstates
         self._reversible = reversible
         self._stationary = stationary
-        self._hmm = copy.deepcopy(initial_model)
-        self._output = self._hmm.output_model.model_type
+        self._hmm = copy.deepcopy(initial_model) if initial_model is not None else None
+        self._output = self._hmm.output_model.model_type if initial_model is not None else output
         self._time_sharded = (isinstance(shard, str) and shard == 'time') or isinstance(batch, TimeShardedTrajectories)
         if isinstance(batch, TimeShardedTrajectories):
             self._all_lengths = [T for (_, _, T) in batch.global_ranges]
@@ -95,6 +94,12 @@ class MaximumLikelihoodEstimator(object):
                                                   warm=warm)
         else:
             self._batch = make_batch(self._observations, nstates, chunk=chunk, warm=warm) if self._nobs else None
+        if self._hmm is None:
+            # the initial model of init_hmm, its per-frame passes on this rank's batch (an empty shard still joins the
+            # collectives); every rank receives the same model
+            from ..api import init_hmm
+            self._hmm = init_hmm(None, nstates, output=self._output, reversible=reversible,
+                                 batch=self._batch if self._batch is not None else [])
         self._hmm.output_model.set_implementation(config.kernel)
         self.count_matrix = None
         self.initial_count = None

@@ -345,6 +345,46 @@ int bhmm_b200_mstep_reversible_dev(const double* d_stats, const double* d_means_
 int bhmm_b200_sample_tmatrix_reversible_dev(const long long* d_counts, const double* d_prior, int N, int nsweeps,
                                             unsigned long long key, double* d_T, double* d_mu, int* d_status, void* stream);
 
+/* ---- initial-model statistics (api.init_gaussian_hmm / init_discrete_hmm with batch=; csrc/init_kernels.cu) ----------
+ * The per-frame passes of the initial-model heuristics on device-resident trajectories.  Rows as in a batch: d_offsets
+ * (device, K+1) local row offsets; d_own_lo / d_own_hi (device, K; both NULL = whole trajectories): only the frames
+ * [own_lo[k], own_hi[k]) of trajectory k are counted; d_flags (device, K; NULL = 2 everywhere): bit 2 = local frame 0 is
+ * the trajectory's frame 0 (its state is counted in n0).  So the statistics of the shards of a data set -- trajectory blocks
+ * or pieces of trajectories cut in time -- add up to those of the whole.  All pointers are device pointers.
+ *
+ * Subsample of the mixture fit: d_out[j] for j in [outoff[k], outoff[k+1]) are, in order, the owned frames of trajectory k
+ * whose index g in the global concatenation of all trajectories is a multiple of `stride`; d_goff[k] is the global index of
+ * local frame 0, d_outoff (K+1) the caller's prefix of the per-trajectory counts (n_out = outoff[K]).  The union over the
+ * shards is init_gaussian_hmm's pooled[::stride]. */
+int bhmm_b200_init_subsample_dev(const double* d_obs, const long long* d_offsets, const long long* d_own_lo,
+                                 const long long* d_own_hi, const long long* d_goff, const long long* d_outoff, int K,
+                                 long long stride, long long n_out, double* d_out, void* stream);
+/* One EM iteration of the 1-D Gaussian mixture of api._gmm_1d on the n sorted frames d_x: responsibilities in log-sum-exp
+ * form from d_params = [weights | means | sigmas] (N each), then nk = sum r + 1e-300, weights = nk / n, means = sum r x / nk,
+ * sigmas = sqrt(max(sum r (x - means)^2 / nk, floor^2)) written back to d_params, and *d_ll = sum of the log-sum-exps (the
+ * log-likelihood under the parameters the iteration started from).  Sums run in a fixed order that depends on n and N only:
+ * the same input gives the same bits.  d_work holds bhmm_b200_gmm_work_doubles(n, N) doubles. */
+long long bhmm_b200_gmm_work_doubles(long long n, int N);
+int bhmm_b200_gmm_em_step_dev(const double* d_x, long long n, int N, double floor, double* d_params, double* d_work,
+                              double* d_ll, void* stream);
+/* Pair counts at `lag` of a frame -> state map f, over the owned frames t whose frame t + lag is in the local rows, ADDED to
+ * the int64 outputs (zero them first; shards and groups may accumulate into one buffer):
+ *   gaussian  f(t) = the first arg-max over k of (lw_k - (0.5 z) z) - ls_k, z = (x - m_k) / s_k, evaluated without
+ *             contraction like init_gaussian_hmm; d_gauss = [means | sigmas | log weights | log sigmas] (N each);
+ *             d_out = [C (N*N) | n0 (N)];
+ *   symbols   f(t) = the symbol (0 <= symbol < M, checked by the caller); d_out = C (M*M);
+ *   labels    f(t) = d_label[symbol] (M entries in [0, N)); d_out = [C (N*N) | n0 (N)], d_B (N*M) += 1 at (label(o), o) for
+ *             every owned frame. */
+int bhmm_b200_init_counts_gaussian_dev(const double* d_obs, const long long* d_offsets, const long long* d_own_lo,
+                                       const long long* d_own_hi, const int* d_flags, int K, long long rows, int lag, int N,
+                                       const double* d_gauss, long long* d_out, void* stream);
+int bhmm_b200_init_counts_symbols_dev(const int* d_sym, const long long* d_offsets, const long long* d_own_lo,
+                                      const long long* d_own_hi, int K, long long rows, int lag, int M, long long* d_out,
+                                      void* stream);
+int bhmm_b200_init_counts_labels_dev(const int* d_sym, const long long* d_offsets, const long long* d_own_lo,
+                                     const long long* d_own_hi, const int* d_flags, int K, long long rows, int lag, int N,
+                                     int M, const int* d_label, long long* d_out, long long* d_B, void* stream);
+
 /* ---- synthetic trajectories (HMM.generate_synthetic_*, bhmm/hmm/generic_hmm.py:433-589) --------------------------
  * Hidden states of K trajectories (host offsets as in bhmm_b200_batch_create) drawn by exact time-parallel forward
  * simulation of the chain, then one observation per frame.  The stream: with row the frame's index in the call and
