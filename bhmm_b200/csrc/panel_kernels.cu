@@ -1689,6 +1689,9 @@ __device__ __forceinline__ void sub_barrier(int sub, int sthr, int nsub)
 #ifndef VITERBI_MULTI_MINB
 #define VITERBI_MULTI_MINB 1
 #endif
+#ifndef VITERBI_MULTI_R
+#define VITERBI_MULTI_R 4                                   // trajectories per group
+#endif
 template <int EM, int R>
 __global__ void __launch_bounds__(512, VITERBI_MULTI_MINB) k_viterbi_multi(const VitArgs a, int NPS, int sthr)
 {
@@ -2256,6 +2259,19 @@ __global__ void k_viterbi_path_flags_wide(const unsigned* __restrict__ flagmap, 
     if (hits) atomicAdd(counter, hits);
 }
 
+// ---- shapes of the wide kernels, outside the launchers so that the CPU emulation (tests/emu) dispatches like them
+// state tiles (= warps per block) for N, 0 if N is not served (N <= 16 belongs to the lane family)
+int wide_tiles(int N) { return (N <= 16) ? 0 : (N <= 32 ? 4 : (N <= 64 ? 8 : (N <= 104 ? 13 : 0))); }
+// chain sets per block of the backward kernel at NT = 13 (128 registers per thread: two sets spill 200-300 bytes per thread,
+// and with 165 KB of the L1 carved out as shared memory the spills go to L2 -- measured: long-scoreboard stalls, no gain)
+#ifndef BWS13
+#define BWS13 1
+#endif
+// chains per block: the two-set kernels (wide2) serve NT >= 8, the one-set kernels NT = 4
+int wide_cpb(int NT) { return NT >= 8 ? WS * PCH : PCH; }
+// chains per block and round of the backward + statistics kernel (its grid is the number of rows of partial statistics)
+int wide_cpb_bwd(int NT) { return NT > 8 ? BWS13 * PCH : wide_cpb(NT); }
+
 #ifndef PANEL_HOST_NO_LAUNCHERS
 int panel_sms()
 {
@@ -2288,19 +2304,8 @@ int panel_blocks(int n_chains)
     return (int)std::max(1LL, std::min(groups, cap));
 }
 
-// wide kernels: state tiles (= warps per block) for N, 0 if N is not served (N <= 16 belongs to the lane family)
-int wide_tiles(int N) { return (N <= 16) ? 0 : (N <= 32 ? 4 : (N <= 64 ? 8 : (N <= 104 ? 13 : 0))); }
-
 #define WIDE_DISPATCH(NTV, CALL4, CALL8, CALL13) \
     do { if ((NTV) == 4) { CALL4; } else if ((NTV) == 8) { CALL8; } else { CALL13; } } while (0)
-
-// chain sets per block of the backward kernel at NT = 13 (128 registers per thread: two sets spill 200-300 bytes per thread,
-// and with 165 KB of the L1 carved out as shared memory the spills go to L2 -- measured: long-scoreboard stalls, no gain)
-#ifndef BWS13
-#define BWS13 1
-#endif
-// chains per block: the two-set kernels (wide2) serve NT >= 8, the one-set kernels NT = 4
-int wide_cpb(int NT) { return NT >= 8 ? WS * PCH : PCH; }
 
 // dynamic shared memory above 48 KB is an opt-in per kernel; set on every launch (a few microseconds: a cache keyed on the
 // function-pointer TYPE -- the first version -- is shared by all instantiations and left most kernels without the attribute)
@@ -2334,9 +2339,6 @@ int wide_blocks_per_sm(int NT)
     }
     return per[NT];
 }
-
-// chains per block and round of the backward + statistics kernel (its grid is the number of rows of partial statistics)
-int wide_cpb_bwd(int NT) { return NT > 8 ? BWS13 * PCH : wide_cpb(NT); }
 
 int wide_blocks_bwd(int NT, int n_chains)
 {
@@ -2429,10 +2431,6 @@ int panel_stats_rows(int N, int n_chains)
 
 // Viterbi with the matrix column in registers: 32 < N <= 104 (N <= 32 keeps the packed one-warp teams)
 bool panel_viterbi_ok(int N) { return panel_mode() > 0 && N > 32 && N <= 104; }
-
-#ifndef VITERBI_MULTI_R
-#define VITERBI_MULTI_R 4
-#endif
 
 template <int EM>
 static int launch_viterbi_regs_em(const VitArgs& a, cudaStream_t st)

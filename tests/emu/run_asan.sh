@@ -1,12 +1,12 @@
 #!/bin/bash
 # The emulated panel-family tests under AddressSanitizer: any access of a kernel outside the caller's (numpy) buffers aborts.
 # Builds the emulator library with -fsanitize=address into a scratch copy of the test (the repo copy stays untouched).
-#   bash tests/emu/run_asan.sh          # ~7 minutes
+#   bash tests/emu/run_asan.sh          # ~25 minutes
 set -e
 ROOT=$(cd "$(dirname "$0")/../.." && pwd)
 W=$(mktemp -d)
 mkdir -p "$W/emu"
-cp "$ROOT/tests/test_panel_emulated_cpu.py" "$ROOT/tests/conftest.py" "$W/"
+cp "$ROOT/tests/test_panel_emulated_cpu.py" "$ROOT/tests/test_panel_family_emulated_cpu.py" "$ROOT/tests/conftest.py" "$W/"
 cp "$ROOT/tests/emu/panel_emu.cpp" "$ROOT/tests/emu/warp_emu.h" "$W/emu/"
 sed -i "s|ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))|ROOT = '$ROOT'|" "$W/conftest.py"
 sed -i "s|os.path.join(HERE, '..', 'bhmm_b200'|os.path.join('$ROOT', 'bhmm_b200'|g" "$W/test_panel_emulated_cpu.py"
@@ -15,7 +15,7 @@ g++ -O1 -g -fsanitize=address -fno-omit-frame-pointer -std=c++17 -shared -fPIC -
     -o "$W/emu/panel_emu.so" "$W/emu/panel_emu.cpp"
 cd "$W"
 LD_PRELOAD=$(gcc -print-file-name=libasan.so) ASAN_OPTIONS=detect_leaks=0:detect_stack_use_after_return=0 \
-    python -m pytest test_panel_emulated_cpu.py -x -q -p no:cacheprovider
+    python -m pytest test_panel_emulated_cpu.py test_panel_family_emulated_cpu.py -x -q -p no:cacheprovider
 
 # ---- part 2: the whole library (host logic + hostified kernels + fake CUDA runtime) under AddressSanitizer: the library's
 # own "device" allocations (workspace carving, partial-statistics rows, flag maps) are checked too.  ~3 minutes.

@@ -48,15 +48,17 @@ def gauss(o, mu, sigma):
 
 
 def plain_estep(ps, A, pi):
-    """ps: list of (T,N) emission tables.  Per-frame normalised forward-backward, gamma, xi counts."""
+    """ps: list of (T,N) emission tables.  Per-frame normalised forward-backward, gamma, xi counts; lc: the log of every
+    frame's normaliser (row by row, its sum is ll)."""
     N = len(pi)
-    out = dict(alpha=[], beta=[], gamma=[], ll=0.0, C=np.zeros((N, N)), g0=np.zeros(N))
+    out = dict(alpha=[], beta=[], gamma=[], ll=0.0, lc=[], C=np.zeros((N, N)), g0=np.zeros(N))
     for p in ps:
         T = len(p)
         al, be = np.zeros((T, N)), np.zeros((T, N))
         for t in range(T):
             v = pi * p[0] if t == 0 else al[t - 1].dot(A) * p[t]
             out['ll'] += np.log(v.sum())
+            out['lc'].append(np.log(v.sum()))
             al[t] = v / v.sum()
         be[T - 1] = 1.0 / N
         for t in range(T - 2, -1, -1):
@@ -73,6 +75,7 @@ def plain_estep(ps, A, pi):
         out['gamma'].append(gam)
     for k in ('alpha', 'beta', 'gamma'):
         out[k] = np.vstack(out[k])
+    out['lc'] = np.array(out['lc'])
     return out
 
 
@@ -268,9 +271,12 @@ def test_exp8_tail_far_observations(emu):
 # ------------------------------------------------------------------------------------------------ wide kernels, 32 < N <= 104
 @pytest.mark.parametrize('N,grid', [(100, 2), (37, 1), (64, 1), (32, 2), (21, 1)])
 def test_wide_gaussian_estep(emu, N, grid, request_cleanup):
-    """k_forward_wide / k_backward_stats_wide: a block of N/8 warps per 8 chains, state tiles exchanged through shared memory.
-    N = 100 (C4's state count, padded to 104: 13 warps), an odd N with a half-empty last tile, a full 64, and the 4-warp
-    instance at N = 32 (the alternative to the one-warp kernels there) and N = 21."""
+    """The wide kernels as the launchers dispatch them: a block of N/8 warps, state tiles exchanged through shared memory;
+    k_forward_wide2 / k_backward_stats_wide2 (two sets of 8 chains per block, outlier machinery compiled in) at N = 100
+    (C4's state count, padded to 104: 13 warps, B fragments in shared memory, one backward chain set per block), an odd N
+    with a half-empty last tile and a full 64; the one-set k_forward_wide / k_backward_stats_wide (4 warps per 8 chains) at
+    N = 32 (the alternative to the one-warp kernels there) and N = 21.  tests/test_panel_family_emulated_cpu.py covers
+    every tile occupancy."""
     rng, A, pi, mu, sigma = model(100 + N, N=N)
     Ts = [50, 33, 1, 41, 18, 29]
     trajs = [mu[rng.integers(0, N, T)] + 0.7 * rng.standard_normal(T) for T in Ts]
@@ -312,7 +318,8 @@ def test_wide_gaussian_estep(emu, N, grid, request_cleanup):
 
 def test_wide_discrete_c4_shape_and_fix_up(emu):
     """N = 100 states, discrete symbols (the C4 model family) with a symbol no state emits, B-numerators, and an exact
-    fix-up pass over a chain list after a warm-up that is too short."""
+    fix-up pass over a chain list after a warm-up that is too short, on k_forward_wide2 / k_backward_stats_wide2 at 13
+    tiles with the outlier rule on."""
     N, M = 100, 30
     rng, A, pi, mu, sigma = model(77, mixing=25.0, N=N)
     B = rng.random((N, M)) ** 3 + 1e-4
